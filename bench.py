@@ -23,6 +23,8 @@ queue are folded into the kernels that touch them last, so a pass is 2 launches 
             fraction and LD-gather GB/s against the measured HBM bandwidth)
 
 python bench.py --impl reference ... times only the reference CPU implementation and prints the same line.
+python bench.py --dump-outputs DIR ... also writes the result arrays of the last timed pass as DIR/<name>.npy (float64);
+the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -190,12 +192,9 @@ def run_reference_arm(args, L, c, wl):
     if rank != 0:
         return
     cores = os.cpu_count() or 1
-    budget = 240.0
     vals, walls = [], []
     kind = "reference" if os.path.exists(REF_BIN) else "port"
     sample = ""
-    t_all = time.time()
-    steps_done = 0
     for i in range(args.warmup + args.steps):
         timed = i >= args.warmup
         if kind == "reference":
@@ -207,21 +206,9 @@ def run_reference_arm(args, L, c, wl):
             n, secs, cores, what = port_cpu_run(L, c)
             sample = f"oracle OpenMP port, {what}"
         if timed:
-            vals.append(n / secs); walls.append(secs); steps_done += 1
-        elapsed = time.time() - t_all
-        per = elapsed / (i + 1)
-        if elapsed + per > budget:          # keep the whole arm within a few minutes
-            if not timed:
-                continue_from = args.warmup  # skip remaining warm-ups (a fresh process has nothing to warm)
-                if i + 1 < continue_from:
-                    args.warmup = i + 1
-            elif steps_done >= 1:
-                break
-    if not vals:
-        n, secs, wall = reference_cpu_run(L, c - 1, tempfile.mkdtemp()) if kind == "reference" else port_cpu_run(L, c)[:3]
-        vals, walls, steps_done = [n / secs], [secs], 1
+            vals.append(n / secs); walls.append(secs)
     v = float(np.mean(vals))
-    line = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": steps_done,
+    line = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": len(vals),
             "warmup": args.warmup, "ms_per_step": 1e3 * float(np.mean(walls)), "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f64", "data": "synthetic",
             "config": {"workload": wl_desc(wl, L, c), "l2": "n/a (CPU)"},
@@ -256,6 +243,16 @@ def emit(line: dict):
     out.flush()
 
 
+def dump_outputs(res, outdir):
+    """What a caller of the timed pass receives (the pipsort_b200.Results of the last timed step): one float64 array
+    per result member.  Only rank 0 calls it: with several GPUs the root holds the whole job's result."""
+    os.makedirs(outdir, exist_ok=True)
+    arrays = {"total": [res.total], "postValues": res.postValues, "noCausal": res.noCausal, "sharedPips": res.sharedPips,
+              "sharedLL": res.sharedLL, "notSharedLL": res.notSharedLL, "n_configs": [res.n_configs]}
+    for name, a in arrays.items():
+        np.save(os.path.join(outdir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def main():
     claim_stdout()
     ap = argparse.ArgumentParser()
@@ -269,7 +266,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-sat", action="store_true", help="skip the saturating B1500c3 side measurement")
     ap.add_argument("--no-side", action="store_true", help="skip the A300c2 / D5000c5 side measurements (BASELINE.json configs[2], [4])")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the result arrays of the last timed pass as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours: the reference arm only times the CPU implementation")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     from pipsort_b200 import synth
@@ -618,6 +621,8 @@ def main():
                                      "roofline": roofline_of(La, 2, am, peak, "A300c2")}
         side["D5000c5_sss"] = measure_sss(peak)            # BASELINE.json configs[4]
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(main_m["result"], args.dump_outputs)
         cpu = None
         if not args.no_cpu and world == 1:
             cpu = cpu_baseline(L, c)

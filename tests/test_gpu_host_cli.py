@@ -60,17 +60,18 @@ def test_cli_shipped_example_files():
                 assert f.read() == w.read(), suf
 
 
-def test_cli_flag_quirks():
+def test_cli_flag_quirks(tmp_path):
     """-m falls through into -n (pipsort.cpp:128-132): with -n BEFORE -m the sample sizes are overwritten by the map
     path and the run dies with the reference's format error; missing required flags exit 1."""
     d = os.path.join(GOLDEN, "small_example")
+    out = str(tmp_path / "o")
     p = subprocess.run([host_bin(), "-l", "ldfiles.txt", "-z", "zfiles.txt", "-n", "7000,7000", "-m",
-                        "eur_afr_small_test_snp_map", "-o", "/tmp/x"], cwd=d, capture_output=True, text=True)
+                        "eur_afr_small_test_snp_map", "-o", out], cwd=d, capture_output=True, text=True)
     assert p.returncode == 1 and "sample size is not in the right format" in p.stdout
     p = subprocess.run([host_bin(), "-l", "ldfiles.txt"], cwd=d, capture_output=True, text=True)
     assert p.returncode == 1 and "are required" in p.stdout
     # -b with the wrong -d: "config file is not the expected size" (postcal.cpp:434-437); -d 0: pipsort.cpp:190-193
-    base = [host_bin(), "-l", "ldfiles.txt", "-z", "zfiles.txt", "-m", "eur_afr_small_test_snp_map", "-n", "7000,7000", "-o", "/tmp/x",
+    base = [host_bin(), "-l", "ldfiles.txt", "-z", "zfiles.txt", "-m", "eur_afr_small_test_snp_map", "-n", "7000,7000", "-o", out,
             "-b", os.path.join(GOLDEN, "test_optional_configs", "all_configs_int16")]
     p = subprocess.run(base + ["-d", "71", "-e", "5"], cwd=d, capture_output=True, text=True)
     assert p.returncode == 1 and "config file is not the expected size" in p.stdout

@@ -29,17 +29,18 @@ def test_required_flags_and_argless_flags():
     assert p.returncode == 1                                                                   # pipsort.cpp:92-95: optarg == NULL
 
 
-def test_m_falls_through_into_n():
+def test_m_falls_through_into_n(tmp_path):
     """-m sets the snp_map AND the sample-size string (missing break, pipsort.cpp:128-132): with -n before -m the sizes
     are overwritten by the map's path and read_sigma rejects them."""
     d = os.path.join(GOLDEN, "small_example")
-    p = run(["-l", "ldfiles.txt", "-z", "zfiles.txt", "-n", "7000,7000", "-m", "eur_afr_small_test_snp_map", "-o", "/tmp/x"], d)
+    p = run(["-l", "ldfiles.txt", "-z", "zfiles.txt", "-n", "7000,7000", "-m", "eur_afr_small_test_snp_map", "-o",
+             str(tmp_path / "o")], d)
     assert p.returncode == 1 and "sample size is not in the right format" in p.stdout
 
 
-def test_explicit_configuration_flag_checks():
+def test_explicit_configuration_flag_checks(tmp_path):
     d = os.path.join(GOLDEN, "small_example")
-    base = ["-l", "ldfiles.txt", "-z", "zfiles.txt", "-m", "eur_afr_small_test_snp_map", "-n", "7000,7000", "-o", "/tmp/x", "-b",
+    base = ["-l", "ldfiles.txt", "-z", "zfiles.txt", "-m", "eur_afr_small_test_snp_map", "-n", "7000,7000", "-o", str(tmp_path / "o"), "-b",
             os.path.join(GOLDEN, "test_optional_configs", "all_configs_int16")]
     p = run(base + ["-d", "0", "-e", "5"], d)
     assert p.returncode == 1 and "Number of configs must be greater than 0" in p.stdout        # pipsort.cpp:190-193
