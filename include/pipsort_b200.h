@@ -41,6 +41,13 @@ extern "C" {
 #define PIPSORT_RAW_LD 4u     /* pipsort_locus.sigma holds the LD matrices as read from the -l files and K is ignored: the engine
                                  runs Model's pre-processing (PSD shift + eigen-decomposition, model.h:171-264) on the device */
 
+#define PIPSORT_PRIOR_CLASSES 8u /* class-resolved store: the accumulators are kept unweighted per prior class (subset size J,
+                                   number a of SNPs causal in both studies), so that one exhaustive pass serves any number of
+                                   priors (gamma, p) -- pipsort_read_prior_grid.  The locus's gamma / sharing_param stay the
+                                   engine's own prior: pipsort_read_accumulators, pipsort_finalize(_reset) and pipsort_fetch_results
+                                   report it.  Such an engine refuses pipsort_sss(_sharded), pipsort_score_union_configs*,
+                                   pipsort_score_given_configs* and pipsort_p2p_combine_finalize (PIPSORT_E_ARG). */
+
 typedef struct pipsort_engine pipsort_engine;
 
 /* Locus description = the PostCal constructor arguments the likelihood actually consumes
@@ -198,6 +205,23 @@ int pipsort_config_count(pipsort_engine* e, uint64_t* out);
  * receives the reference's mycount.                                                                    */
 int pipsort_posterior_exhaustive(const pipsort_locus* locus, int device, uint32_t flags, int c, const pipsort_outputs* out,
                                  uint64_t* n_configs);
+
+/* Results for a grid of priors from ONE pass (engine created with PIPSORT_PRIOR_CLASSES): outs[i] receives what an engine
+ * created with gamma[i] / sharing_param[i] would report after the same calls -- same layout and meaning as
+ * pipsort_read_accumulators (0.0 = nothing accumulated with a non-zero prior weight); n_configs (optional) the configuration
+ * count, the same for every prior.  The likelihood E_0(C0) E_1(C1) of an expanded configuration does not depend on the prior,
+ * and the prior pi'(J,a) (postcal.cpp:19-59) only on the subset size J and the number a of SNPs causal in both studies, so the
+ * store keeps one unweighted sum per (SNP, J, state, a') and per (J, a) and the weights are applied here: one finalize launch
+ * over all priors and one device-to-host copy.  Every prior is validated as pipsort_create does (gamma in (0,1), p in [0,1]);
+ * n_priors >= 1.  The store may be the sum of several engines' (pipsort_merge, an all-reduce of pipsort_accumulator_buffer,
+ * pipsort_p2p_reduce_to_root).                                                                      */
+int pipsort_read_prior_grid(pipsort_engine* e, int n_priors, const double* gamma, const double* sharing_param,
+                            const pipsort_outputs* outs, uint64_t* n_configs);
+
+/* One locus, a grid of priors, one call: pipsort_create (flags | PIPSORT_PRIOR_CLASSES) + pipsort_run_exhaustive over the whole
+ * rank space + pipsort_read_prior_grid + pipsort_destroy.  The locus's own gamma / sharing_param are validated but not reported. */
+int pipsort_posterior_exhaustive_grid(const pipsort_locus* locus, int device, uint32_t flags, int c, int n_priors, const double* gamma,
+                                      const double* sharing_param, const pipsort_outputs* outs, uint64_t* n_configs);
 
 /* The same for a list of loci (a fine-mapping run has thousands): software pipelines over three engines on three
  * streams each, driven by a few host threads (PIPSORT_BATCH_THREADS, default 3; lists of fewer than 8 loci: one), so that

@@ -65,6 +65,7 @@ struct AccDev {
     int NB;
     int bias;
     int Upad;
+    int ccls;          // 0: the store above;  C > 0: the class-resolved store of PIPSORT_PRIOR_CLASSES for size classes <= C (below)
     double* counters;  // tail of the same allocation as bins: [0] expanded configurations evaluated (the reference's
                        // mycount; exact below 2^53), [1 + f] number of times error f was raised.  Doubles, so that the
                        // ONE all-reduce(sum) that combines the stores of several GPUs carries them as well.
@@ -120,5 +121,22 @@ __device__ __forceinline__ void bin_add(const AccDev& a, int slot, int g, double
 }
 
 __device__ __forceinline__ void bin_add(const AccDev& a, int slot, int g, const XAcc& v) { bin_add(a, slot, g, v.M, v.N); }
+
+// Class-resolved store (PIPSORT_PRIOR_CLASSES, DESIGN.md section 5f): the same bins, but every accumulator is UNWEIGHTED and
+// resolved by prior class, so that any prior (gamma, p) can be applied when the results are read.
+//   per SNP g: G[g][J][t][a'] for J = 1..C, t = 0 / 1 / 2 (study 0 only / study 1 only / both), a' = 0..J-1 other SNPs of
+//              the subset causal in both studies -- slot cls_slot(J, t, a');
+//   scalars:   T[J][a] (J = 0..C, a = 0..J: every expanded configuration), N_0[J] / N_1[J] (study 0 / study 1 carries no
+//              causal SNP, the terms of S_NC0 / S_NC1) -- scalar k lives in slot cls_nslot(C) + k / Upad at column k % Upad.
+__host__ __device__ constexpr int cls_slot(int J, int t, int ap) { return 3 * J * (J - 1) / 2 + t * J + ap; }
+__host__ __device__ constexpr int cls_nslot(int C) { return 3 * C * (C + 1) / 2; }
+__host__ __device__ constexpr int cls_T(int J, int a) { return J * (J + 1) / 2 + a; }
+__host__ __device__ constexpr int cls_N(int C, int s, int J) { return (C + 1) * (C + 2) / 2 + s * (C + 1) + J; }
+__host__ __device__ constexpr int cls_nscal(int C) { return (C + 1) * (C + 2) / 2 + 2 * (C + 1); }
+
+// scalar k of the class-resolved store += M * 2^N
+__device__ __forceinline__ void scal_add(const AccDev& a, int k, double M, int N) {
+    bin_add(a, cls_nslot(a.ccls) + k / a.Upad, k % a.Upad, M, N);
+}
 
 }  // namespace pipsort

@@ -229,6 +229,125 @@ __global__ void __launch_bounds__(FIN_WARPS * 32) finalize_kernel(AccDev acc, in
     res[3 + (size_t)lane * U + g] = xlog_or_zero(mine, lane < 3 ? cx : cy);
 }
 
+// Layout of one prior of the grid read: pi'(J,a) as a (KMAX+1) x (KMAX+1) table (row J), then cx = -K/2 + U log(1-gamma).
+constexpr int PRIOR_STRIDE = (KMAX + 1) * (KMAX + 1) + 1;
+
+// class slot / scalar of the class-resolved store (common.cuh) read by ONE lane: the top three non-empty bins, as bins_read_warp
+__device__ inline XAcc bins_read_lane(const AccDev& a, int slot, int g, bool clear) {
+    double* p = bin_ptr(a, slot, g);
+    int top = -1;
+    for (int b = 0; b < a.NB; b++)
+        if (p[(size_t)b * a.Upad] > 0.0) top = b;
+    if (top < 0) return xacc_empty();
+    double M = p[(size_t)top * a.Upad];
+    if (top > 0) M += p[(size_t)(top - 1) * a.Upad] * 0x1p-512;
+    if (top > 1) M += (p[(size_t)(top - 2) * a.Upad] * 0x1p-512) * 0x1p-512;
+    if (clear)
+        for (int b = 0; b <= top; b++) p[(size_t)b * a.Upad] = 0.0;
+    const int hi = __double2hiint(M);
+    const int e = ((hi >> 20) & 0x7ff) - 1023;
+    M = __hiloint2double(hi - (e << 20), __double2loint(M));
+    return XAcc{M, 512 * top - a.bias + e};
+}
+
+// acc += w * v  (w >= 0 a prior weight; a zero weight or an empty v adds nothing)
+__device__ __forceinline__ void xadd_weighted(XAcc& acc, const XAcc& v, double w) {
+    const double m = v.M * w;
+    if (m > 0.0) xadd(acc, m, v.N);
+}
+
+// Finalize of the class-resolved store (PIPSORT_PRIOR_CLASSES, DESIGN.md section 5f) for n_priors priors: prior i is
+// pri[i * PRIOR_STRIDE ..] (PRIOR_STRIDE above) and its results go to res[i * (3 + 5 U) ..] in finalize_kernel's layout; the
+// counters follow the last prior (the same for every prior).  One warp per scalar output / union SNP: lane l reads the class
+// slots l, l + 32, .. once, then every prior costs one weighted warp sum per output.
+constexpr int GRID_LANE_SLOTS = (cls_nslot(KMAX) + 31) / 32;
+__global__ void __launch_bounds__(FIN_WARPS * 32) finalize_grid_kernel(AccDev acc, int U, int n_priors, const double* __restrict__ pri,
+                                                                       double cy, double* __restrict__ res, int clear) {
+    asm volatile("griddepcontrol.wait;" ::: "memory");
+    const int lane = threadIdx.x & 31;
+    const int w = blockIdx.x * FIN_WARPS + (threadIdx.x >> 5);
+    const int C = acc.ccls;
+    const size_t stride = 3 + (size_t)5 * U;
+    if (blockIdx.x == 0 && threadIdx.x < NCOUNTER) {
+        res[(size_t)n_priors * stride + threadIdx.x] = acc.counters[threadIdx.x];
+        if (clear) acc.counters[threadIdx.x] = 0.0;
+    }
+    if (w < 3) {   // total: T[J][a], weight pi'(J,a);  noCausal[s]: N_s[J], weight pi'(J,0)
+        const int n = w == 0 ? (C + 1) * (C + 2) / 2 : C + 1;
+        XAcc v[2];
+        int row[2];
+        for (int q = 0; q < 2; q++) {
+            const int k = lane + 32 * q;
+            v[q] = xacc_empty();
+            row[q] = -1;
+            if (k >= n) continue;
+            int J = 0, a = k;
+            if (w == 0) while (a > J) { J++; a -= J; }
+            else { J = k; a = 0; }
+            const int idx = w == 0 ? cls_T(J, a) : cls_N(C, w - 1, J);
+            v[q] = bins_read_lane(acc, cls_nslot(C) + idx / acc.Upad, idx % acc.Upad, clear != 0);
+            row[q] = J * (KMAX + 1) + a;
+        }
+        for (int i = 0; i < n_priors; i++) {
+            const double* pi = pri + (size_t)i * PRIOR_STRIDE;
+            XAcc s = xacc_empty();
+            for (int q = 0; q < 2; q++)
+                if (row[q] >= 0) xadd_weighted(s, v[q], pi[row[q]]);
+            s = xwarp_sum(s);
+            if (lane == 0) res[(size_t)i * stride + w] = xlog_or_zero(s, pi[PRIOR_STRIDE - 1]);
+        }
+        return;
+    }
+    const int g = w - 3;
+    if (g >= U) return;
+    XAcc v[GRID_LANE_SLOTS];
+    int row[GRID_LANE_SLOTS], st[GRID_LANE_SLOTS];
+    XAcc ys = xacc_empty(), yn = xacc_empty();      // likelihood-only sums: the same for every prior
+#pragma unroll
+    for (int q = 0; q < GRID_LANE_SLOTS; q++) {
+        const int k = lane + 32 * q;
+        v[q] = xacc_empty();
+        row[q] = 0; st[q] = -1;
+        if (k >= cls_nslot(C)) continue;
+        int J = 1, r = k;
+        while (r >= 3 * J) { r -= 3 * J; J++; }
+        const int t = r / J, ap = r - t * J;
+        v[q] = bins_read_lane(acc, k, g, clear != 0);
+        st[q] = t;
+        row[q] = J * (KMAX + 1) + ap + (t == 2 ? 1 : 0);
+        if (v[q].M > 0.0) xadd(t == 2 ? ys : yn, v[q].M, v[q].N);
+    }
+    ys = xwarp_sum(ys);
+    yn = xwarp_sum(yn);
+    if (lane == 0) {
+        res[3 + (size_t)3 * U + g] = xlog_or_zero(ys, cy);
+        res[3 + (size_t)4 * U + g] = xlog_or_zero(yn, cy);
+    }
+    for (int i = 0; i < n_priors; i++) {
+        const double* pi = pri + (size_t)i * PRIOR_STRIDE;
+        XAcc x[3] = {xacc_empty(), xacc_empty(), xacc_empty()};
+#pragma unroll
+        for (int q = 0; q < GRID_LANE_SLOTS; q++) {
+            if (st[q] < 0) continue;
+            const double wq = pi[row[q]];
+            if (st[q] == 0) xadd_weighted(x[0], v[q], wq);
+            else if (st[q] == 1) xadd_weighted(x[1], v[q], wq);
+            else xadd_weighted(x[2], v[q], wq);
+        }
+#pragma unroll
+        for (int t = 0; t < 3; t++) x[t] = xwarp_sum(x[t]);
+        XAcc p0 = x[0], p1 = x[1];
+        xmerge(p0, x[2]);
+        xmerge(p1, x[2]);
+        const double cx = pi[PRIOR_STRIDE - 1];
+        double* r = res + (size_t)i * stride + 3;
+        if (lane == 0) r[g] = xlog_or_zero(p0, cx);
+        else if (lane == 1) r[(size_t)U + g] = xlog_or_zero(p1, cx);
+        else if (lane == 2) r[(size_t)2 * U + g] = xlog_or_zero(x[2], cx);
+        else if (lane == 3 && i > 0) { r[(size_t)3 * U + g] = xlog_or_zero(ys, cy); r[(size_t)4 * U + g] = xlog_or_zero(yn, cy); }
+    }
+}
+
 // The root's half of the multi-GPU combine step fused with the finalize (accumulators of at most 32 bins): lane b of the warp
 // of a SNP takes bin b of the SNP's five accumulators from the root's own store AND from every peer's mailbox slot (polling
 // each element until it carries this epoch's flag, p2p.cuh), so the sum over the GPUs never goes back to memory; the root's
@@ -396,6 +515,12 @@ struct pipsort_engine {
     } p2p;
     PrepResult prep[2];             // PIPSORT_RAW_LD: what the on-device pre-processing found per study
     bool prepped = false;
+    // PIPSORT_PRIOR_CLASSES: the store is class-resolved (AccDev::ccls > 0); the engine's own prior as the grid finalize reads it
+    bool classes = false;
+    double* d_own_prior = nullptr;  // [PRIOR_STRIDE]
+    double* d_grid = nullptr;       // grid read: priors | results | counters
+    size_t cap_grid = 0;
+    std::vector<double> h_grid;
 };
 
 namespace {
@@ -496,7 +621,8 @@ int ensure_score_smem(pipsort_engine* e, int ws_kmax, size_t* bytes) {
     if (e->score_smem_set < ws_kmax) {
         size_t mx = SCORE_WARPS * warp_ws_bytes(KMAX);
         CU(cudaFuncSetAttribute(score_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mx));
-        CU(cudaFuncSetAttribute(exhaustive_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mx));
+        CU(cudaFuncSetAttribute(exhaustive_generic_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mx));
+        CU(cudaFuncSetAttribute(exhaustive_generic_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mx));
         e->score_smem_set = KMAX;
     }
     return 0;
@@ -578,8 +704,10 @@ void pipsort_destroy(pipsort_engine* e) {
     if (e->stream) cudaStreamSynchronize(e->stream);
     if (e->own_stream) {
         auto in_arena = [&](const void* q) { return e->arena && (const char*)q >= e->arena && (const char*)q < e->arena + e->arena_cap; };
-        if (e->exh.d_chunks && !in_arena(e->exh.d_chunks)) cudaFreeAsync(e->exh.d_chunks, e->own_stream);
-        if (e->exh.d_counter && !in_arena(e->exh.d_counter)) cudaFreeAsync(e->exh.d_counter, e->own_stream);
+        // (dev_alloc hands out separate allocations once the arena is full: those are in `allocs` and freed below, once)
+        auto owned = [&](const void* q) { return in_arena(q) || std::find(e->allocs.begin(), e->allocs.end(), q) != e->allocs.end(); };
+        if (e->exh.d_chunks && !owned(e->exh.d_chunks)) cudaFreeAsync(e->exh.d_chunks, e->own_stream);
+        if (e->exh.d_counter && !owned(e->exh.d_counter)) cudaFreeAsync(e->exh.d_counter, e->own_stream);
         for (void* p : e->allocs) cudaFreeAsync(p, e->own_stream);   // stream-ordered: no second synchronisation needed
         if (e->arena) cudaFreeAsync(e->arena, e->own_stream);
     }
@@ -596,6 +724,7 @@ void pipsort_destroy(pipsort_engine* e) {
     }
     for (cudaGraphExec_t x : e->graphs) cudaGraphExecDestroy(x);
     if (e->d_idx) cudaFree(e->d_idx);
+    if (e->d_grid) cudaFree(e->d_grid);
     if (e->d_upd) cudaFree(e->d_upd);
     if (e->d_out) cudaFree(e->d_out);
     if (e->own_stream && e->ev0 && e->ev1 && e->evk0 && e->evk1 && e->ev_up) {   // back to the per-device cache
@@ -614,6 +743,43 @@ void pipsort_destroy(pipsort_engine* e) {
 
     if (e->own_stream) cudaStreamDestroy(e->own_stream);
     delete e;
+}
+
+// The prior (gamma, p) of log_prior (postcal.cpp:19-59): pi[j][a] = pi'(j,a) = (gamma/(1-gamma))^j p^a ((1-p)/2)^(j-a), the
+// complete log prior logprior[j][a] (may be NULL), and *minpi = the smallest finite log pi'(j,a) with j <= kb.  pipsort_create
+// (the engine's own prior) and pipsort_read_prior_grid (every prior of a grid) both build their tables here.
+static int prior_tables(double gam, double p, int U, int kb, double (*pi)[KMAX + 1], double (*logprior)[KMAX + 1], double* minpi) {
+    if (!(gam > 0.0 && gam < 1.0)) return fail(PIPSORT_E_ARG, "gamma must be in (0,1)");
+    if (!(p >= 0.0 && p <= 1.0)) return fail(PIPSORT_E_ARG, "sharing_param must be in [0,1]");
+    double mn = 0.0;
+    for (int j = 0; j <= KMAX; j++)
+        for (int a = 0; a <= KMAX; a++) {
+            if (a > j) { pi[j][a] = 0.0; if (logprior) logprior[j][a] = 0.0; continue; }
+            double lp = 0.0, rel = 0.0;
+            if (p != 0.0) {                                   // postcal.cpp:27: the sharing term is skipped for p == 0
+                for (int i = 0; i < a; i++) lp += std::log(p);
+                for (int i = a; i < j; i++) lp += std::log((1.0 - p) * 0.5);
+                rel = lp;
+            }
+            for (int i = 0; i < j; i++) lp += std::log(gam);
+            lp += (U - j) * std::log(1.0 - gam);
+            rel += j * (std::log(gam) - std::log(1.0 - gam));
+            if (logprior) logprior[j][a] = lp;
+            pi[j][a] = std::exp(rel);                         // 0 when p == 1 and a < j
+            if (j <= kb && std::isfinite(rel)) mn = std::min(mn, rel);
+        }
+    if (minpi) *minpi = mn;
+    return 0;
+}
+
+// One prior of a grid read as the finalize kernel takes it (PRIOR_STRIDE doubles)
+static int grid_prior(const pipsort_engine* e, double gam, double p, double* out) {
+    double pi[KMAX + 1][KMAX + 1];
+    int rc = prior_tables(gam, p, e->U, e->kb, pi, nullptr, nullptr);
+    if (rc) return rc;
+    memcpy(out, pi, sizeof pi);
+    out[PRIOR_STRIDE - 1] = -0.5 * e->K + e->U * std::log(1.0 - gam);
+    return 0;
 }
 
 static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pipsort_engine* e) {
@@ -693,8 +859,10 @@ static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pips
     TR(1);
     // ---- arena: everything dev_alloc hands out below (estimate; the accumulator store is sized for 16 bins) ------------
     {
+        const size_t upad = (size_t)std::max((U + 3) & ~3, 4), kb = (size_t)std::min(KMAX, std::max(3, lc->max_causal));
+        const size_t nslot = (flags & PIPSORT_PRIOR_CLASSES) ? cls_nslot((int)kb) + (cls_nscal((int)kb) + upad - 1) / upad + 1 : NSLOT;
         size_t est = 64 * 256 + sizeof(LocusDev) + (size_t)(3 + 5 * U + NCOUNTER) * 8 + (size_t)(U + 2) * 8 +
-                     ((size_t)NSLOT * 16 * (size_t)std::max((U + 3) & ~3, 4) + NCOUNTER) * 8;
+                     (nslot * 16 * upad + NCOUNTER) * 8;
         est += ((size_t)e->sm_count * 12 + 256) * sizeof(int4) + 512;               // chunk descriptors of the exhaustive launch
         size_t nints = (size_t)6 * U + 2 * ((size_t)U / 32 + 8);
         for (int s = 0; s < S; s++) {
@@ -846,24 +1014,10 @@ static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pips
     TR(5);
     // ---- prior tables (log_prior, postcal.cpp:19-59) --------------------------------------------------
     const double gam = lc->gamma, p = lc->sharing_param;
-    if (!(gam > 0.0 && gam < 1.0)) return fail(PIPSORT_E_ARG, "gamma must be in (0,1)");
-    if (!(p >= 0.0 && p <= 1.0)) return fail(PIPSORT_E_ARG, "sharing_param must be in [0,1]");
     double minpi = 0.0;
-    for (int j = 0; j <= KMAX; j++)
-        for (int a = 0; a <= j; a++) {
-            double lp = 0.0, rel = 0.0;
-            if (p != 0.0) {                                   // postcal.cpp:27: the sharing term is skipped for p == 0
-                for (int i = 0; i < a; i++) lp += std::log(p);
-                for (int i = a; i < j; i++) lp += std::log((1.0 - p) * 0.5);
-                rel = lp;
-            }
-            for (int i = 0; i < j; i++) lp += std::log(gam);
-            lp += (U - j) * std::log(1.0 - gam);
-            rel += j * (std::log(gam) - std::log(1.0 - gam));
-            L.logprior[j][a] = lp;
-            L.pi[j][a] = std::exp(rel);                       // 0 when p == 1 and a < j
-            if (j <= e->kb && std::isfinite(rel)) minpi = std::min(minpi, rel);
-        }
+    if ((rc = prior_tables(gam, p, U, e->kb, L.pi, L.logprior, &minpi))) return rc;
+    e->classes = (flags & PIPSORT_PRIOR_CLASSES) != 0;
+    if (e->classes) minpi = 0.0;     // the class-resolved store holds unweighted sums: the range of the likelihood-only sums
     e->K = K_total;
     L.neg_half_K = -0.5 * K_total;
     L.null_l = (-K_total / 2 - std::sqrt(std::fabs(1.0))) + U * std::log(1.0 - gam);   // postcal.cpp:802-803
@@ -917,7 +1071,10 @@ static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pips
     acc.bias = (((int)std::ceil(-minexp_bits) + 511) / 512 + 1) * 512;
     acc.NB = ((int)std::ceil(maxexp_bits) + acc.bias) / 512 + 2;
     acc.Upad = std::max((U + 3) & ~3, 4);
-    e->bins_len = (size_t)NSLOT * acc.NB * acc.Upad + NCOUNTER;   // the counters ride in the tail of the store
+    acc.ccls = e->classes ? e->kb : 0;
+    // class-resolved: 3 c(c+1)/2 class slots per SNP, then as many rows as the scalars need (common.cuh)
+    const size_t nslot = e->classes ? (size_t)cls_nslot(e->kb) + (cls_nscal(e->kb) + acc.Upad - 1) / acc.Upad : (size_t)NSLOT;
+    e->bins_len = nslot * acc.NB * acc.Upad + NCOUNTER;   // the counters ride in the tail of the store
     if ((rc = dev_alloc(e, &acc.bins, e->bins_len))) return rc;
     acc.counters = acc.bins + (e->bins_len - NCOUNTER);
     if ((rc = dev_alloc(e, &e->d_res, 3 + (size_t)5 * U + NCOUNTER))) return rc;   // results | counters: one D2H per read
@@ -931,6 +1088,11 @@ static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pips
     e->exh.pin_stage_cap = e->exh.cap_chunks * sizeof(int4);
     e->exh.pin_stage = pin_slice(e, e->exh.pin_stage_cap);
     CU(cudaMemsetAsync(acc.bins, 0, e->bins_len * sizeof(double), e->stream));
+    if (e->classes) {   // the engine's own prior, as the grid finalize reads it (pipsort_finalize must not upload: graphs)
+        double own[PRIOR_STRIDE];
+        if ((rc = grid_prior(e, gam, p, own))) return rc;
+        if ((rc = dev_alloc(e, &e->d_own_prior, PRIOR_STRIDE)) || (rc = upload_small(e, e->d_own_prior, own, sizeof own))) return rc;
+    }
     // the caller's buffers and the local staging vectors must not be read after return: wait for the H2D copies only
     // (recorded in ev_up after the last of them); the preparation kernels and memsets keep running asynchronously.
     // e->L lives as long as the engine, so its upload needs no wait.
@@ -1122,7 +1284,8 @@ int pipsort_run_exhaustive(pipsort_engine* e, int c, uint64_t rank_begin, uint64
             const int chunk = (re - rb) >= (u64)e->sm_count * SCORE_WARPS * 64 ? 16 : 1;
             const u64 nchunks = (re - rb + chunk - 1) / chunk;
             const int blocks = (int)std::min<u64>((nchunks + SCORE_WARPS - 1) / SCORE_WARPS, (u64)e->sm_count * 8);
-            exhaustive_generic_kernel<<<blocks, SCORE_WARPS * 32, smem, e->stream>>>(e->L, j, rb, re, chunk, wk);
+            if (e->classes) exhaustive_generic_kernel<true><<<blocks, SCORE_WARPS * 32, smem, e->stream>>>(e->L, j, rb, re, chunk, wk);
+            else exhaustive_generic_kernel<false><<<blocks, SCORE_WARPS * 32, smem, e->stream>>>(e->L, j, rb, re, chunk, wk);
             e->launches++;
             CU(cudaGetLastError());
             if (dominant && !e->capturing) { CU(cudaEventRecord(e->evk1, e->stream)); e->evk_valid = true; }
@@ -1175,9 +1338,16 @@ static int launch_score_batch(pipsort_engine* e, const int32_t* d_idx, int64_t n
     return 0;
 }
 
+// what an engine with a class-resolved store (PIPSORT_PRIOR_CLASSES) refuses, and why
+static const char* CLASSES_NO_SCORE = "scoring given configurations is not supported on a PIPSORT_PRIOR_CLASSES engine (its store is "
+                                      "filled by the exhaustive pass only)";
+static const char* CLASSES_NO_SSS = "the shotgun search cannot run on a PIPSORT_PRIOR_CLASSES engine: its search trajectory depends on "
+                                    "the prior";
+
 int pipsort_score_union_configs_device(pipsort_engine* e, const int32_t* d_idx, int64_t n, int kmax,
                                        const uint8_t* d_make_updates, double* d_out) {
     if (!e) return fail(PIPSORT_E_ARG, "null engine");
+    if (e->classes) return fail(PIPSORT_E_ARG, "%s", CLASSES_NO_SCORE);
     if (n < 0 || kmax < 0 || kmax > e->kb) return fail(PIPSORT_E_ARG, "kmax=%d outside [0,%d]", kmax, e->kb);
     if (n == 0) return 0;
     CU(cudaSetDevice(e->device));
@@ -1187,6 +1357,7 @@ int pipsort_score_union_configs_device(pipsort_engine* e, const int32_t* d_idx, 
 int pipsort_score_union_configs(pipsort_engine* e, const int32_t* idx, int64_t n, int kmax, const uint8_t* make_updates,
                                 double* out_max_abs_l) {
     if (!e) return fail(PIPSORT_E_ARG, "null engine");
+    if (e->classes) return fail(PIPSORT_E_ARG, "%s", CLASSES_NO_SCORE);
     if (n < 0 || kmax < 0 || kmax > e->kb) return fail(PIPSORT_E_ARG, "kmax=%d outside [0,%d]", kmax, e->kb);
     if (n == 0) return 0;
     if (!idx && kmax > 0) return fail(PIPSORT_E_ARG, "null idx");
@@ -1205,6 +1376,7 @@ int pipsort_score_union_configs(pipsort_engine* e, const int32_t* idx, int64_t n
 
 int pipsort_score_given_configs_device(pipsort_engine* e, const int16_t* d_configs, int64_t num_configs, int num_groups) {
     if (!e) return fail(PIPSORT_E_ARG, "null engine");
+    if (e->classes) return fail(PIPSORT_E_ARG, "%s", CLASSES_NO_SCORE);
     if (num_configs < 0 || num_groups < 0) return fail(PIPSORT_E_ARG, "negative matrix dimension");
     if (num_configs == 0) return 0;
     if (!d_configs && num_groups > 0) return fail(PIPSORT_E_ARG, "null configs");
@@ -1265,6 +1437,7 @@ int pipsort_sss_reset(pipsort_engine* e) {
 
 int pipsort_sss(pipsort_engine* e, int max_causal, int max_iterations, int32_t* iterations, int32_t* stop_reason) {
     if (!e) return fail(PIPSORT_E_ARG, "null engine");
+    if (e->classes) return fail(PIPSORT_E_ARG, "%s", CLASSES_NO_SSS);
     const int c = max_causal, U = e->U;
     if (c < 0 || c > e->kb) return fail(PIPSORT_E_ARG, "max_causal=%d outside [0,%d] (max_causal given at create)", c, e->kb);
     if (U > SSS_MAX_U) return fail(PIPSORT_E_RANGE, "the search state packs union indices into 15 bits: U=%d > %d", U, SSS_MAX_U);
@@ -1357,6 +1530,7 @@ int pipsort_sss(pipsort_engine* e, int max_causal, int max_iterations, int32_t* 
 
 int pipsort_sss_sharded(pipsort_engine* e, int max_causal, int max_iterations, int32_t* iterations, int32_t* stop_reason) {
     if (!e) return fail(PIPSORT_E_ARG, "null engine");
+    if (e->classes) return fail(PIPSORT_E_ARG, "%s", CLASSES_NO_SSS);
     pipsort_engine::P2P& pp = e->p2p;
     if (!pp.connected) return fail(PIPSORT_E_ARG, "pipsort_p2p_connect has not been called");
     if (pp.world == 1) return pipsort_sss(e, max_causal, max_iterations, iterations, stop_reason);
@@ -1471,6 +1645,7 @@ int pipsort_sss_sharded(pipsort_engine* e, int max_causal, int max_iterations, i
 
 int pipsort_score_given_configs(pipsort_engine* e, const int16_t* configs, int64_t num_configs, int num_groups) {
     if (!e) return fail(PIPSORT_E_ARG, "null engine");
+    if (e->classes) return fail(PIPSORT_E_ARG, "%s", CLASSES_NO_SCORE);
     if (num_configs < 0 || num_groups < 0) return fail(PIPSORT_E_ARG, "negative matrix dimension");
     if (num_configs == 0) return 0;
     if (!configs && num_groups > 0) return fail(PIPSORT_E_ARG, "null configs");
@@ -1521,7 +1696,28 @@ static int flags_to_error(const double* c) {
     return 0;
 }
 
+// the finalize of a class-resolved store for n_priors priors (device table `pri`, PRIOR_STRIDE doubles each) into `res`
+static int finalize_grid_launch(pipsort_engine* e, int n_priors, const double* pri, double* res, bool clear) {
+    CU(cudaSetDevice(e->device));
+    static const bool no_pdl = getenv("PIPSORT_NO_PDL") != nullptr;
+    cudaLaunchConfig_t cfg;
+    memset(&cfg, 0, sizeof cfg);
+    cfg.gridDim = dim3((e->U + 3 + FIN_WARPS - 1) / FIN_WARPS);
+    cfg.blockDim = dim3(FIN_WARPS * 32);
+    cfg.stream = e->stream;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = at;
+    cfg.numAttrs = no_pdl ? 0 : 1;
+    CU(cudaLaunchKernelEx(&cfg, finalize_grid_kernel, e->L.acc, e->U, n_priors, pri, -0.5 * e->K, res, clear ? 1 : 0));
+    e->launches++;
+    return 0;
+}
+
 static int finalize_launch(pipsort_engine* e, bool clear) {
+    // a class-resolved store reports the engine's own prior: the grid finalize for that one prior, same result layout
+    if (e->classes) return finalize_grid_launch(e, 1, e->d_own_prior, e->d_res, clear);
     CU(cudaSetDevice(e->device));
     const int U = e->U;
     const double cy = -0.5 * e->K, cx = cy + U * std::log(1.0 - e->gamma);
@@ -1588,6 +1784,8 @@ int pipsort_read_accumulators(pipsort_engine* e, const pipsort_outputs* out) {
     return read_complete(e, out);
 }
 
+static void scatter_results(const pipsort_engine* e, const double* r, const pipsort_outputs* out);
+
 // second half: wait for the engine's stream, check the error counters, scatter into the caller's arrays
 static int read_complete(pipsort_engine* e, const pipsort_outputs* out) {
     const int U = e->U;
@@ -1596,7 +1794,13 @@ static int read_complete(pipsort_engine* e, const pipsort_outputs* out) {
     int rc = flags_to_error(hres + 3 + (size_t)5 * U);
     if (rc) return rc;
     e->last_read_count = (uint64_t)hres[3 + (size_t)5 * U];
-    const double* r = hres;
+    scatter_results(e, hres, out);
+    return 0;
+}
+
+// results in the finalize kernel's layout (3 + 5 U, internal order) -> the caller's arrays (snp_map / study order)
+static void scatter_results(const pipsort_engine* e, const double* r, const pipsort_outputs* out) {
+    const int U = e->U;
     if (out->total) *out->total = r[0];
     if (out->noCausal) { out->noCausal[0] = r[1]; out->noCausal[1] = r[2]; }
     r += 3;
@@ -1616,7 +1820,56 @@ static int read_complete(pipsort_engine* e, const pipsort_outputs* out) {
         if (out->sharedLL) out->sharedLL[ug] = r[(size_t)3 * U + g];
         if (out->notSharedLL) out->notSharedLL[ug] = r[(size_t)4 * U + g];
     }
+}
+
+int pipsort_read_prior_grid(pipsort_engine* e, int n_priors, const double* gamma, const double* sharing_param,
+                            const pipsort_outputs* outs, uint64_t* n_configs) {
+    if (!e) return fail(PIPSORT_E_ARG, "null engine");
+    if (!e->classes) return fail(PIPSORT_E_ARG, "the engine was not created with PIPSORT_PRIOR_CLASSES: its store holds one prior only");
+    if (n_priors < 1) return fail(PIPSORT_E_ARG, "n_priors=%d must be >= 1", n_priors);
+    if (!gamma || !sharing_param || !outs) return fail(PIPSORT_E_ARG, "null argument");
+    const size_t stride = 3 + (size_t)5 * e->U, npri = (size_t)n_priors * PRIOR_STRIDE;
+    const size_t need = npri + (size_t)n_priors * stride + NCOUNTER;
+    e->h_grid.resize(need);
+    for (int i = 0; i < n_priors; i++) {
+        int rc = grid_prior(e, gamma[i], sharing_param[i], e->h_grid.data() + (size_t)i * PRIOR_STRIDE);
+        if (rc) { const std::string why = g_err; return fail(rc, "prior %d: %s", i, why.c_str()); }
+    }
+    CU(cudaSetDevice(e->device));
+    if (e->cap_grid < need) {
+        if (e->d_grid) { CU(cudaStreamSynchronize(e->stream)); CU(cudaFree(e->d_grid)); e->d_grid = nullptr; }
+        CU(cudaMalloc(&e->d_grid, need * sizeof(double)));
+        e->cap_grid = need;
+    }
+    CU(cudaMemcpyAsync(e->d_grid, e->h_grid.data(), npri * sizeof(double), cudaMemcpyHostToDevice, e->stream));
+    int rc = finalize_grid_launch(e, n_priors, e->d_grid, e->d_grid + npri, false);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(e->h_grid.data() + npri, e->d_grid + npri, (need - npri) * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaStreamSynchronize(e->stream));
+    const double* res = e->h_grid.data() + npri;
+    if ((rc = flags_to_error(res + (size_t)n_priors * stride))) return rc;
+    e->last_read_count = (uint64_t)res[(size_t)n_priors * stride];
+    if (n_configs) *n_configs = e->last_read_count;
+    for (int i = 0; i < n_priors; i++) scatter_results(e, res + (size_t)i * stride, &outs[i]);
     return 0;
+}
+
+int pipsort_posterior_exhaustive_grid(const pipsort_locus* locus, int device, uint32_t flags, int c, int n_priors, const double* gamma,
+                                      const double* sharing_param, const pipsort_outputs* outs, uint64_t* n_configs) {
+    if (!outs) return fail(PIPSORT_E_ARG, "null argument");
+    if (n_priors < 1) return fail(PIPSORT_E_ARG, "n_priors=%d must be >= 1", n_priors);
+    pipsort_engine* e = nullptr;
+    int rc = pipsort_create(locus, device, flags | PIPSORT_PRIOR_CLASSES | PIPSORT_INTERNAL_NO_UPLOAD_WAIT |
+                                               (c >= 2 ? PIPSORT_INTERNAL_WITH_PAIRS : 0u), &e);
+    if (rc) return rc;
+    uint64_t total = 0;
+    rc = pipsort_total_ranks(e, c, &total);
+    if (!rc) rc = pipsort_run_exhaustive(e, c, 0, total);
+    if (!rc) rc = pipsort_read_prior_grid(e, n_priors, gamma, sharing_param, outs, n_configs);
+    std::string keep = g_err;
+    pipsort_destroy(e);
+    g_err = keep;
+    return rc;
 }
 
 int pipsort_posterior_exhaustive(const pipsort_locus* locus, int device, uint32_t flags, int c, const pipsort_outputs* out,
@@ -1850,6 +2103,9 @@ int pipsort_p2p_reduce_to_root_reset(pipsort_engine* e) {
 static int finalize_launch(pipsort_engine* e, bool clear);
 int pipsort_p2p_combine_finalize(pipsort_engine* e) {
     if (!e) return fail(PIPSORT_E_ARG, "null engine");
+    if (e->classes)
+        return fail(PIPSORT_E_ARG, "the fused combine + finalize reads the five-slot store only; on a PIPSORT_PRIOR_CLASSES engine "
+                                   "use pipsort_p2p_reduce_to_root and read the root");
     pipsort_engine::P2P& q = e->p2p;
     if (!q.connected) return fail(PIPSORT_E_ARG, "pipsort_p2p_connect has not been called");
     if (q.world == 1) return finalize_launch(e, true);

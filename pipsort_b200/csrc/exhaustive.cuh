@@ -181,14 +181,18 @@ inline int exhaustive_launch_all(const LocusDev& L, const LocusDev* Lg, int c, u
         if ((err = cudaMallocAsync(&sc->d_counter, 2 * sizeof(unsigned), stream)) != cudaSuccess) return (int)err;
         if ((err = cudaMemsetAsync(sc->d_counter, 0, 2 * sizeof(unsigned), stream)) != cudaSuccess) return (int)err;
     }
+    // the instantiation that matches the engine's store (class-resolved: PIPSORT_PRIOR_CLASSES)
+    const bool cr = L.acc.ccls > 0;
+    void (*kernel)(LocusDev, ExhAll, const LocusDev*) = cr ? exhaustive_all_kernel<true> : exhaustive_all_kernel<false>;
+    const size_t smem = cr ? EXH_SMEM_BYTES_CR : EXH_SMEM_BYTES;
     if (!sc->occ) {
         // (the attribute is per device: set it for every engine, not once per process)
-        if ((err = cudaFuncSetAttribute(exhaustive_all_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)EXH_SMEM_BYTES)) != cudaSuccess) return (int)err;
-        static int occ_cache = 0;    // a property of the kernel and the device generation: query once per process
+        if ((err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return (int)err;
+        static int occ_cache[2] = {0, 0};    // a property of the kernel and the device generation: query once per process
         static std::mutex occ_mutex;
         std::lock_guard<std::mutex> g(occ_mutex);
-        if (!occ_cache && (err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_cache, exhaustive_all_kernel, EXH_WARPS * 32, EXH_SMEM_BYTES)) != cudaSuccess) return (int)err;
-        sc->occ = occ_cache;
+        if (!occ_cache[cr] && (err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_cache[cr], kernel, EXH_WARPS * 32, smem)) != cudaSuccess) return (int)err;
+        sc->occ = occ_cache[cr];
     }
     const double forced = [] { const char* v = getenv("PIPSORT_EXH_CHUNK"); return v ? atof(v) : 0.0; }();   // experiments / tests
     if (!(sc->plan_valid && !(forced > 0.0) && sc->plan_c == c && sc->plan_rb == rank_begin && sc->plan_re == rank_end)) {
@@ -250,7 +254,7 @@ inline int exhaustive_launch_all(const LocusDev& L, const LocusDev* Lg, int c, u
     static_assert(sizeof(ExhChunkDesc) == sizeof(int4), "descriptor layout");
     if (sc->plan.n_total == 0) return 0;
     if (ev0 && (err = cudaEventRecord(ev0, stream)) != cudaSuccess) return (int)err;
-    exhaustive_all_kernel<<<sc->plan_blocks, EXH_WARPS * 32, EXH_SMEM_BYTES, stream>>>(L, sc->plan, Lg);
+    kernel<<<sc->plan_blocks, EXH_WARPS * 32, smem, stream>>>(L, sc->plan, Lg);
     if (ev1 && (err = cudaEventRecord(ev1, stream)) != cudaSuccess) return (int)err;
     (*launches)++;
     return (int)cudaGetLastError();

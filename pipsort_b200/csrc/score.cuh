@@ -102,14 +102,23 @@ __device__ __forceinline__ int pow3(int k) {
 
 // Scores the configuration whose internal union indices are in ws.g[0..k).  Warp-collective.
 // Returns (on every lane) the expansion value l with the largest |l|, 0.0 if there is none.
+// CR: class-resolved store (PIPSORT_PRIOR_CLASSES, common.cuh): the cells are kept per a' = a - [t == 2] instead of being
+// weighted with L.pi[k][a], and go unweighted to their (k, t, a') slots; the total per a, the no-causal sums per class
+template <bool CR = false>
 __device__ inline double score_config(const LocusDev& L, const WarpWS& ws, int k, bool upd, int lane) {
     const AccDev& acc = L.acc;
     if (k == 0) {  // postcal.cpp:793-822, sss_postcal.cpp:463-499
         if (upd && lane == 0) {
             const double einv = 0.36787944117144233;  // exp(-1): the "- sqrt(|1|)" of postcal.cpp:802
-            bin_add(acc, SCAL, S_TOTAL, einv, 0);
-            bin_add(acc, SCAL, S_NC0, einv, 0);
-            bin_add(acc, SCAL, S_NC1, einv, 0);
+            if (CR) {
+                scal_add(acc, cls_T(0, 0), einv, 0);
+                scal_add(acc, cls_N(acc.ccls, 0, 0), einv, 0);
+                scal_add(acc, cls_N(acc.ccls, 1, 0), einv, 0);
+            } else {
+                bin_add(acc, SCAL, S_TOTAL, einv, 0);
+                bin_add(acc, SCAL, S_NC0, einv, 0);
+                bin_add(acc, SCAL, S_NC1, einv, 0);
+            }
             count_add(acc, 1ull);
         }
         return L.null_l;
@@ -230,6 +239,33 @@ __device__ inline double score_config(const LocusDev& L, const WarpWS& ws, int k
             if ((in0 && !(P[0] & bit)) || (in1 && !(P[1] & bit))) continue;
             const int r0 = (in0 ? FULL : FULL ^ bit) & P[0], r1 = (in1 ? FULL : FULL ^ bit) & P[1];
             const int nr = en0[r0] + en1[r1];
+            if constexpr (CR) {
+                double sa[KMAX];                      // sa[a'] (registers: the index is resolved by the unrolled selects)
+#pragma unroll
+                for (int q = 0; q < KMAX; q++) sa[q] = 0.0;
+                for (int ep = lane; ep < n3m; ep += 32) {
+                    const int hi = ep / p3i, lo = ep - hi * p3i;
+                    const uint32_t pk = tab[(hi * 3 + t) * p3i + lo];
+                    const int m0 = pk & 255, m1 = (pk >> 8) & 255, ap = (int)(pk >> 16) - (t == 2 ? 1 : 0);
+                    const double v0 = em0[m0], v1 = em1[m1];
+                    if (v0 == 0.0 || v1 == 0.0) continue;
+                    int de = en0[m0] + en1[m1] - nr;
+                    de = min(de, 1000);
+                    const double v = v0 * v1 * pow2c(max(de, -2000));
+#pragma unroll
+                    for (int q = 0; q < KMAX; q++) sa[q] += q == ap ? v : 0.0;
+                }
+#pragma unroll
+                for (int q = 0; q < KMAX; q++) {
+                    if (q >= k) break;
+                    const double v = warp_sum(sa[q]);
+                    if (lane == 0) {
+                        bin_add(acc, cls_slot(k, t, q), g, v, nr);
+                        if (i == 0) scal_add(acc, cls_T(k, q + (t == 2 ? 1 : 0)), v, nr);
+                    }
+                }
+                continue;
+            }
             double sx = 0.0, sy = 0.0;
             for (int ep = lane; ep < n3m; ep += 32) {
                 const int hi = ep / p3i, lo = ep - hi * p3i;
@@ -253,8 +289,13 @@ __device__ inline double score_config(const LocusDev& L, const WarpWS& ws, int k
         }
     }
     if (lane == 0) {  // no causal SNP in a study: the other study carries all k (postcal.cpp:988-1000)
-        if ((FULL & ~P[0]) == 0) bin_add(acc, SCAL, S_NC1, L.pi[k][0] * em0[FULL], en0[FULL]);
-        if ((FULL & ~P[1]) == 0) bin_add(acc, SCAL, S_NC0, L.pi[k][0] * em1[FULL], en1[FULL]);
+        if (CR) {
+            if ((FULL & ~P[0]) == 0) scal_add(acc, cls_N(acc.ccls, 1, k), em0[FULL], en0[FULL]);
+            if ((FULL & ~P[1]) == 0) scal_add(acc, cls_N(acc.ccls, 0, k), em1[FULL], en1[FULL]);
+        } else {
+            if ((FULL & ~P[0]) == 0) bin_add(acc, SCAL, S_NC1, L.pi[k][0] * em0[FULL], en0[FULL]);
+            if ((FULL & ~P[1]) == 0) bin_add(acc, SCAL, S_NC0, L.pi[k][0] * em1[FULL], en1[FULL]);
+        }
         count_add(acc, (u64)nvalid);
     }
     return best;
@@ -301,6 +342,8 @@ score_batch_kernel(LocusDev L, const int* __restrict__ idx, long long n, int kma
 
 // Exhaustive enumeration of the j-subsets with in-class ranks [r_begin, r_end) (internal SNP order):
 // every warp takes chunks of `chunk` consecutive ranks, unranks the first and walks the rest.
+// CR: the class-resolved store (PIPSORT_PRIOR_CLASSES); the engine launches the instantiation that matches its store.
+template <bool CR>
 __global__ void __launch_bounds__(SCORE_WARPS * 32)
 exhaustive_generic_kernel(LocusDev L, int j, u64 r_begin, u64 r_end, int chunk, int ws_kmax) {
     extern __shared__ __align__(16) unsigned char smem[];
@@ -314,7 +357,7 @@ exhaustive_generic_kernel(LocusDev L, int j, u64 r_begin, u64 r_end, int chunk, 
         if (lane == 0) unrank_subset(lo, L.U, j, ws.g);
         __syncwarp();
         for (u64 r = lo; r < hi; r++) {
-            score_config(L, ws, j, true, lane);
+            score_config<CR>(L, ws, j, true, lane);
             __syncwarp();
             if (lane == 0) next_subset(L.U, j, ws.g);
             __syncwarp();

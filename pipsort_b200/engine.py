@@ -20,6 +20,7 @@ _lib = None
 KEEP_ORDER = 1
 GENERIC_ONLY = 2
 RAW_LD = 4
+PRIOR_CLASSES = 8
 IPC_HANDLE_BYTES = 64
 KMAX = 8
 
@@ -85,6 +86,10 @@ def lib():
         L.pipsort_sss_reset.argtypes = [vp]
         L.pipsort_sss_sharded.argtypes = [vp, i32, i32, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
         L.pipsort_read_accumulators.argtypes = [vp, C.POINTER(_Outputs)]
+        L.pipsort_read_prior_grid.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(_OutputsV),
+                                              C.POINTER(u64)]
+        L.pipsort_posterior_exhaustive_grid.argtypes = [C.POINTER(_LocusV), i32, C.c_uint32, i32, i32, C.POINTER(C.c_double),
+                                                        C.POINTER(C.c_double), C.POINTER(_OutputsV), C.POINTER(u64)]
         L.pipsort_finalize.argtypes = [vp]
         L.pipsort_finalize_reset.argtypes = [vp]
         L.pipsort_fetch_results.argtypes = [vp, C.POINTER(_Outputs)]
@@ -160,7 +165,7 @@ class Engine:
     """Device-resident locus + accumulators (the hot-path half of the reference's PostCal)."""
 
     def __init__(self, num_snps, sigma, z, d, K, snp_map, gamma=0.01, sharing_param=0.75, max_causal=3, device=0,
-                 keep_order=False, generic_only=False, raw_ld=False):
+                 keep_order=False, generic_only=False, raw_ld=False, prior_classes=False):
         self.num_snps = np.ascontiguousarray(num_snps, dtype=np.int32)
         if isinstance(sigma, (list, tuple)):
             sigma = np.concatenate([np.asarray(s, dtype=np.float64).ravel() for s in sigma])
@@ -179,8 +184,8 @@ class Engine:
                      self.U, smap.ctypes.data_as(C.POINTER(C.c_int32)), float(gamma), float(sharing_param),
                      int(max_causal))
         self._h = C.c_void_p()
-        _check(lib().pipsort_create(C.byref(loc), int(device), (KEEP_ORDER if keep_order else 0) | (GENERIC_ONLY if generic_only else 0) | (RAW_LD if raw_ld else 0),
-                                    C.byref(self._h)))
+        _check(lib().pipsort_create(C.byref(loc), int(device), (KEEP_ORDER if keep_order else 0) | (GENERIC_ONLY if generic_only else 0) |
+                                    (RAW_LD if raw_ld else 0) | (PRIOR_CLASSES if prior_classes else 0), C.byref(self._h)))
         self.max_causal = int(max_causal)
         self.device = int(device)
 
@@ -298,6 +303,15 @@ class Engine:
         cnt = C.c_uint64()
         _check(lib().pipsort_last_read_config_count(self._h, C.byref(cnt)))
         return Results(float(total[0]), post, nc, sp, sl, nl, int(cnt.value))
+
+    def read_prior_grid(self, priors) -> list:
+        """Results for every prior (gamma, p) of `priors` from the accumulators of ONE pass (an engine created with
+        prior_classes=True): each equals what an engine created with that prior reports (pipsort_read_prior_grid)."""
+        gam, p = _prior_arrays(priors)
+        outs, res = _grid_outputs(len(gam), self.N, self.S, self.U)
+        cnt = C.c_uint64()
+        _check(lib().pipsort_read_prior_grid(self._h, len(gam), _dp(gam), _dp(p), outs, C.byref(cnt)))
+        return res(int(cnt.value))
 
     def finalize(self, reset=False):
         """Bins -> log-space results on the device; reset=True also leaves the accumulators empty (no reset() needed before
@@ -430,6 +444,54 @@ def posterior_exhaustive(num_snps, sigma, z, d, K, snp_map, c, gamma=0.01, shari
     cnt = C.c_uint64()
     _check(lib().pipsort_posterior_exhaustive(C.byref(loc), int(device), RAW_LD if raw_ld else 0, int(c), C.byref(o), C.byref(cnt)))
     return Results(float(total[0]), post, nc, sp, sl, nl, int(cnt.value))
+
+
+def _prior_arrays(priors):
+    pr = np.asarray(priors, dtype=np.float64).reshape(-1, 2) if len(priors) else np.zeros((0, 2))
+    return np.ascontiguousarray(pr[:, 0]), np.ascontiguousarray(pr[:, 1])
+
+
+def _grid_outputs(n, N, S, U):
+    """pipsort_outputs[n] over one buffer, and a function that slices the buffer into Results once it is filled."""
+    w = 1 + N + S + 3 * U
+    buf = np.zeros((max(n, 1), w))
+    outs = (_OutputsV * max(n, 1))()
+    for i in range(n):
+        b0 = buf[i].ctypes.data
+        outs[i] = _OutputsV(b0, b0 + 8, b0 + 8 * (1 + N), b0 + 8 * (1 + N + S), b0 + 8 * (1 + N + S + U), b0 + 8 * (1 + N + S + 2 * U))
+
+    def results(cnt):
+        out = []
+        for i in range(n):
+            r = buf[i]
+            p2 = 1 + N + S
+            out.append(Results(float(r[0]), r[1:1 + N], r[1 + N:p2], r[p2:p2 + U], r[p2 + U:p2 + 2 * U], r[p2 + 2 * U:], cnt))
+        return out
+    return outs, results
+
+
+def posterior_exhaustive_grid(num_snps, sigma, z, d, K, snp_map, c, priors, device=0, raw_ld=False):
+    """One locus, a grid of priors (gamma, p), one exhaustive pass (pipsort_posterior_exhaustive_grid): a list of Results,
+    one per prior, each what posterior_exhaustive with that prior returns."""
+    num_snps = np.ascontiguousarray(num_snps, dtype=np.int32)
+    if isinstance(sigma, (list, tuple)):
+        sigma = np.concatenate([np.asarray(s, dtype=np.float64).ravel() for s in sigma])
+    if isinstance(z, (list, tuple)):
+        z = np.concatenate([np.asarray(v, dtype=np.float64).ravel() for v in z])
+    sigma = np.ascontiguousarray(sigma, dtype=np.float64).ravel()
+    z = np.ascontiguousarray(z, dtype=np.float64).ravel()
+    d = np.ascontiguousarray(d, dtype=np.float64)
+    smap = np.ascontiguousarray(snp_map, dtype=np.int32)
+    S, U, N = len(num_snps), int(smap.shape[1]), int(num_snps.sum())
+    gam, p = _prior_arrays(priors)
+    own = (float(gam[0]), float(p[0])) if len(gam) else (0.01, 0.75)     # the locus's own prior: validated, not reported
+    loc = _LocusV(S, num_snps.ctypes.data, sigma.ctypes.data, z.ctypes.data, d.ctypes.data, float(K), U, smap.ctypes.data,
+                  own[0], own[1], int(c))
+    outs, res = _grid_outputs(len(gam), N, S, U)
+    cnt = C.c_uint64()
+    _check(lib().pipsort_posterior_exhaustive_grid(C.byref(loc), int(device), RAW_LD if raw_ld else 0, int(c), len(gam), _dp(gam),
+                                                   _dp(p), outs, C.byref(cnt)))
+    return res(int(cnt.value))
 
 
 _LOCUS_DT = np.dtype([("num_studies", "<i4"), ("num_snps", "<u8"), ("sigma", "<u8"), ("z", "<u8"), ("d", "<u8"), ("K", "<f8"),

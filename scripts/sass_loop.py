@@ -1,7 +1,8 @@
 """Static look at the hot loop of exhaustive_all_kernel without a GPU: compiles only exhaustive_dev.cuh (a few seconds),
 finds the innermost loops that hold the MUFU.RSQ64H of the bordered step and prints, per loop, the instruction count, the
 sum of the stall counts the compiler encoded (= issue cycles of ONE warp running alone, scoreboard waits excluded), the
-opcode mix and the local-memory traffic (spills).   python scripts/sass_loop.py [-DEXH_...=...] [--dump file]"""
+opcode mix and the local-memory traffic (spills).   python scripts/sass_loop.py [-DEXH_...=...] [--dump file] [--classes]
+(--classes: the instantiation for the class-resolved store of PIPSORT_PRIOR_CLASSES instead of the default one)"""
 import os, re, subprocess, sys, tempfile
 from collections import Counter
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -17,7 +18,7 @@ def build(defs, out):
     os.unlink(src)
     if r.returncode:
         sys.exit(r.stderr)
-    info = [l for l in r.stderr.split("\n") if "exhaustive_all" in l or "registers" in l or "spill" in l]
+    info = [l for l in r.stderr.split("\n") if "exhaustive_all" in l or "registers" in l or "spill" in l or "smem" in l]
     return info
 
 
@@ -55,7 +56,8 @@ def main():
         print(l.strip())
     fns = parse(out)
     os.unlink(out)
-    name = [k for k in fns if "exhaustive_all_kernel" in k][0]
+    tag = "ILb1E" if "--classes" in sys.argv else "ILb0E"
+    name = [k for k in fns if "exhaustive_all_kernel" in k and tag in k][0]
     ins = fns[name]
     print("kernel instructions:", len(ins))
     loops = []
