@@ -122,6 +122,20 @@ __device__ __forceinline__ void bin_add(const AccDev& a, int slot, int g, double
 
 __device__ __forceinline__ void bin_add(const AccDev& a, int slot, int g, const XAcc& v) { bin_add(a, slot, g, v.M, v.N); }
 
+// The accumulator whose top non-empty bin is `top`, as M * 2^N with M in [1,2): that bin plus the two below it, each scaled
+// down by 2^512 per bin (what lies in lower bins is below one ulp of the sum).  bin(k) returns bin top - k; it is called
+// only for bins that exist, so that a reader from memory loads no more than it needs.
+template <class Bin>
+__device__ __forceinline__ XAcc bins_decode(int top, int bias, Bin bin) {
+    double M = bin(0);
+    if (top > 0) M += bin(1) * 0x1p-512;
+    if (top > 1) M += (bin(2) * 0x1p-512) * 0x1p-512;
+    const int hi = __double2hiint(M);
+    const int e = ((hi >> 20) & 0x7ff) - 1023;
+    M = __hiloint2double(hi - (e << 20), __double2loint(M));
+    return XAcc{M, 512 * top - bias + e};
+}
+
 // Class-resolved store (PIPSORT_PRIOR_CLASSES, DESIGN.md section 5f): the same bins, but every accumulator is UNWEIGHTED and
 // resolved by prior class, so that any prior (gamma, p) can be applied when the results are read.
 //   per SNP g: G[g][J][t][a'] for J = 1..C, t = 0 / 1 / 2 (study 0 only / study 1 only / both), a' = 0..J-1 other SNPs of

@@ -39,17 +39,32 @@ __device__ inline bool p2p_spin_ge(const volatile u64* p, u64 target) {
     return true;
 }
 
+// The mailbox word: a double v as {low half of v | flag}, {high half of v | flag}, flag = the low 32 bits of the epoch.
+__device__ __forceinline__ ulonglong2 p2p_encode(double v, u64 flag) {
+    const u64 b = (u64)__double_as_longlong(v), f = flag << 32;
+    return make_ulonglong2((b & 0xffffffffull) | f, (b >> 32) | f);
+}
+__device__ __forceinline__ bool p2p_arrived(const ulonglong2& w, u64 flag) { return (w.x >> 32) == flag && (w.y >> 32) == flag; }
+__device__ __forceinline__ double p2p_decode(const ulonglong2& w) {
+    return __longlong_as_double((long long)((w.x & 0xffffffffull) | (w.y << 32)));
+}
+__device__ __forceinline__ ulonglong2 p2p_load(const ulonglong2* src) {   // both words in one 16-byte load, past the caches
+    ulonglong2 w;
+    asm volatile("ld.volatile.global.v2.u64 {%0, %1}, [%2];" : "=l"(w.x), "=l"(w.y) : "l"(src));
+    return w;
+}
+
 // one element of a peer's slot: spins until both words carry this epoch's flag (8-byte stores are single-copy atomic)
 __device__ __forceinline__ double p2p_take(const ulonglong2* src, u64 flag, bool& ok) {
-    u64 w0, w1;
+    ulonglong2 w;
     const long long t0 = clock64();
     for (;;) {
-        asm volatile("ld.volatile.global.v2.u64 {%0, %1}, [%2];" : "=l"(w0), "=l"(w1) : "l"(src));
-        if ((w0 >> 32) == flag && (w1 >> 32) == flag) break;
+        w = p2p_load(src);
+        if (p2p_arrived(w, flag)) break;
         if (clock64() - t0 > P2P_SPIN_CYCLES) { ok = false; break; }
         __nanosleep(32);
     }
-    return __longlong_as_double((long long)((w0 & 0xffffffffull) | (w1 << 32)));
+    return p2p_decode(w);
 }
 
 __global__ void __launch_bounds__(256)
@@ -67,12 +82,12 @@ p2p_push_kernel(double* __restrict__ store, size_t n, ulonglong2* __restrict__ m
         ok = p2p_spin_ge(my_ctrl + 1, epoch_s - 1) ? 1 : 0;        // the root has consumed the previous epoch's slot
     }
     __syncthreads();
-    const u64 flag = (epoch_s & 0xffffffffull) << 32;
+    const u64 flag = epoch_s & 0xffffffffull;
     if (ok) {
         for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
-            const u64 b = (u64)__double_as_longlong(store[i]);
-            my_slot_at_root[i] = make_ulonglong2((b & 0xffffffffull) | flag, (b >> 32) | flag);
-            if (clear && b) store[i] = 0.0;          // what has been sent is gone: the push doubles as this rank's reset
+            const double v = store[i];
+            my_slot_at_root[i] = p2p_encode(v, flag);
+            if (clear && __double_as_longlong(v)) store[i] = 0.0;   // what has been sent is gone: the push doubles as this rank's reset
         }
     }
     __syncthreads();
@@ -93,19 +108,8 @@ p2p_merge_kernel(double* __restrict__ store, const ulonglong2* slots, size_t n, 
     bool ok = true;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
         double v = store[i];
-        for (int r = 0; r < peers.world; r++) {
-            if (r == my_rank) continue;
-            const volatile ulonglong2* src = slots + (size_t)r * slot_stride + i;
-            u64 w0, w1;
-            const long long t0 = clock64();
-            for (;;) {                                           // both halves carry this epoch's flag: the element is here
-                asm volatile("ld.volatile.global.v2.u64 {%0, %1}, [%2];" : "=l"(w0), "=l"(w1) : "l"(src));
-                if ((w0 >> 32) == flag && (w1 >> 32) == flag) break;
-                if (clock64() - t0 > P2P_SPIN_CYCLES) { ok = false; break; }
-                __nanosleep(32);
-            }
-            v += __longlong_as_double((long long)((w0 & 0xffffffffull) | (w1 << 32)));
-        }
+        for (int r = 0; r < peers.world; r++)
+            if (r != my_rank) v += p2p_take(slots + (size_t)r * slot_stride + i, flag, ok);
         store[i] = v;
     }
     if (!ok) atomicAdd(err_flag, 1.0);

@@ -136,6 +136,14 @@ __device__ __forceinline__ void xexp_pair(const double (&t)[2], double (&m)[2], 
 // natural log of an accumulator; caller handles M == 0 (empty)
 __device__ __forceinline__ double xlog(const XAcc& a) { return log(a.M) + (double)a.N * 0.6931471805599453094; }
 
+// log(M 2^N) + c ; 0.0 (the reference's "empty" sentinel, postcal.h:102-112) when nothing was added
+__device__ inline double xlog_or_zero(const XAcc& a, double c) {
+    if (!(a.M > 0.0)) return 0.0;
+    const double LN2_HI = 6.93147180369123816490e-01, LN2_LO = 1.90821492927058770002e-10;
+    const double n = (double)a.N;
+    return (n * LN2_HI + (log(a.M) + n * LN2_LO)) + c;
+}
+
 // warp-wide sum of XAccs: common exponent = max N over the warp (one REDUX), mantissas re-scaled
 // to it (terms more than 2^1022 below the warp maximum flush to zero: they are below one ulp of
 // the sum), then a plain shuffle tree.  Result valid in every lane.

@@ -2,6 +2,7 @@
 17-digit dumps of the reference's own `-q 1` runs, the oracle's restatement of the search, and -- at the size of
 BASELINE.json configs[4] (5000 SNPs per study, c = 5) -- sampled neighbours against the oracle plus size-independent
 properties of one batched neighbourhood."""
+import math
 import os
 import subprocess
 import tempfile
@@ -41,6 +42,34 @@ def test_sss_synthetic_matches_oracle_trajectory():
         r, iters, why = e.sss(4, max_iterations=60)
     assert iters == want.extra["n_iter"]
     assert_results_match(r, want)
+
+
+def test_sss_convergence_rule_reads_the_running_total():
+    """The convergence rule (sss_postcal.cpp:265-270) compares the running totals after consecutive rounds.  The reference
+    starts it at round 100, which no search we know reaches; PIPSORT_SSS_CONV_FROM=2 starts it at round 2.  On 12+12 SNPs
+    (c = 3, 9 rounds to the break condition) the totals the engine reports after k = 1..9 rounds predict the round at which
+    the rule stops the search."""
+    from pipsort_b200 import synth
+    SL = synth.make_locus(12, overlap=0.7, seed=18)
+    with engine_for(SL, 3) as e:
+        total = [None]                                   # total[k]: after k rounds
+        for k in range(1, 10):
+            r, iters, why = e.sss(3, max_iterations=k)
+            assert (iters, why) == (k, 0)
+            total.append(r.total)
+        # round i (counted from 0) stops the search when i >= 2 + 1 and 1 - exp(total[i] - total[i + 1]) <= 0.001
+        crit = {i: 1 - math.exp(total[i] - total[i + 1]) for i in range(3, 9)}
+        stops = [i for i in crit if crit[i] <= 0.001]
+        assert stops
+        stop = stops[0]
+        for i in range(3, stop + 1):                     # accumulation order varies: no round may sit on the threshold
+            assert abs(crit[i] - 0.001) > 1e-6, (i, crit[i])
+        os.environ["PIPSORT_SSS_CONV_FROM"] = "2"
+        try:
+            _, iters, why = e.sss(3)
+        finally:
+            os.environ.pop("PIPSORT_SSS_CONV_FROM", None)
+    assert (iters, why) == (stop, 2)
 
 
 def test_host_loop_and_device_state_agree_through_the_cli():
