@@ -153,4 +153,33 @@ __device__ __forceinline__ void scal_add(const AccDev& a, int k, double M, int N
     bin_add(a, cls_nslot(a.ccls) + k / a.Upad, k % a.Upad, M, N);
 }
 
+// Call-local device memory: allocated from the device's pool on `stream`, freed on the same stream when it leaves scope, on
+// every return path.
+template <class T>
+struct DevTemp {
+    T* p = nullptr;
+    cudaStream_t stream = nullptr;
+    DevTemp() = default;
+    DevTemp(const DevTemp&) = delete;   // one owner: freed once
+    void operator=(const DevTemp&) = delete;
+    ~DevTemp() { free(); }
+    void free() { if (p) cudaFreeAsync(p, stream); p = nullptr; }   // before scope exit: the memory is not needed any more
+    operator T*() const { return p; }
+    cudaError_t alloc(size_t count, cudaStream_t s) {
+        stream = s;
+        const cudaError_t err = cudaMallocAsync((void**)&p, (count ? count : 1) * sizeof(T), s);
+        if (err != cudaSuccess) { p = nullptr; cudaGetLastError(); }   // a refused request leaves no error pending
+        return err;
+    }
+};
+
+// Runs f when it leaves scope (handles and events of a call, released on every return path)
+template <class F>
+struct ScopeExit {
+    F f;
+    ~ScopeExit() { f(); }
+};
+template <class F>
+ScopeExit<F> scope_exit(F f) { return ScopeExit<F>{f}; }
+
 }  // namespace pipsort

@@ -433,7 +433,8 @@ __global__ void __launch_bounds__(256) dfma_peak_kernel(double* out, int iters, 
 struct pipsort_engine {
     int device = 0;
     cudaStream_t stream = nullptr, own_stream = nullptr;
-    void* l2_scratch = nullptr;
+    char* l2_scratch = nullptr;
+    size_t cap_l2 = 0;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, evk0 = nullptr, evk1 = nullptr, ev_up = nullptr;
     bool evk_valid = false;
     LocusDev L, L_host_copy;
@@ -445,7 +446,8 @@ struct pipsort_engine {
     std::vector<int> orig[2];       // study-local (internal order) -> original study index
     std::vector<int> loc[2];        // internal union index -> study-local index or -1
     std::vector<int> types;         // internal union index -> 0 shared, 1 only study 0, 2 only study 1, 3 nowhere
-    std::vector<void*> allocs;
+    struct Alloc { void* p; bool pinned; };
+    std::vector<Alloc> allocs;      // what did not come from the arena: device pool buffers and pinned host buffers
     char* pin = nullptr;            // pinned staging buffer of the stream kit (PIN_BYTES), bump-allocated, never reused
     size_t pin_off = 0;             // within an engine's life: an asynchronous copy may still be reading a slice
     bool defer_upload_sync = false; // one-call path: the caller's buffers outlive the call, no wait after the uploads
@@ -457,7 +459,7 @@ struct pipsort_engine {
     double* h_res_pin = nullptr;    // slice of the pinned staging buffer for the result read-back
     size_t bins_len = 0;
     u64 launches = 0;
-    // scratch for pipsort_score_union_configs (host buffers)
+    // scratch of pipsort_score_union_configs (callers with host buffers)
     int* d_idx = nullptr; unsigned char* d_upd = nullptr; double* d_out = nullptr;
     size_t cap_idx = 0, cap_upd = 0, cap_out = 0;
     int score_smem_set = 0;
@@ -475,7 +477,8 @@ struct pipsort_engine {
         double* d_out_l = nullptr; int* d_batch = nullptr; unsigned char* d_upd = nullptr; int* d_counter = nullptr;
         double* d_scored = nullptr; unsigned char* d_state = nullptr; int* d_pos_of = nullptr; double* d_total = nullptr;
         double* h_out_l = nullptr;  // pinned: [n_max] neighbour values, [n_max + 1] the running total
-        long long n_max = 0; int kmax = 0;
+        size_t cap_out_l = 0, cap_batch = 0, cap_upd = 0, cap_counter = 0, cap_scored = 0, cap_state = 0, cap_pos_of = 0,
+               cap_total = 0, cap_h_out_l = 0;
     } sss;
     // peer-memory combine (p2p.cuh): this rank's mailbox + the peers' mapped mailboxes
     struct P2P {
@@ -519,10 +522,14 @@ int kit_acquire(int device, StreamKit* k) {
         auto& c = kit_cache(device);
         if (!c.empty()) { *k = c.back(); c.pop_back(); return 0; }
     }
-    CU(cudaStreamCreateWithFlags(&k->stream, cudaStreamNonBlocking));
-    for (int i = 0; i < 4; i++) CU(cudaEventCreate(&k->ev[i]));
-    CU(cudaEventCreateWithFlags(&k->ev[4], cudaEventDisableTiming));
-    k->pin = nullptr;
+    *k = StreamKit{};
+    cudaError_t err = cudaStreamCreateWithFlags(&k->stream, cudaStreamNonBlocking);
+    for (int i = 0; i < 5 && err == cudaSuccess; i++) err = cudaEventCreateWithFlags(&k->ev[i], i < 4 ? cudaEventDefault : cudaEventDisableTiming);
+    if (err != cudaSuccess) {   // a kit is complete or not at all
+        for (cudaEvent_t ev : k->ev) if (ev) cudaEventDestroy(ev);
+        if (k->stream) cudaStreamDestroy(k->stream);
+        return fail(PIPSORT_E_CUDA, "stream / event creation failed: %s", cudaGetErrorString(err));
+    }
     if (cudaHostAlloc((void**)&k->pin, PIN_BYTES, cudaHostAllocDefault) != cudaSuccess) { k->pin = nullptr; cudaGetLastError(); }
     return 0;
 }
@@ -549,20 +556,62 @@ int pool_setup(int device) {
 
 // Device memory of an engine comes from ONE stream-ordered allocation made in pipsort_create (an arena with a bump
 // pointer): a locus needs ~25 arrays, and 25 cudaMallocAsync / cudaFreeAsync pairs are a visible part of a 0.3 ms
-// create-run-read-destroy cycle.  Requests the arena cannot hold (its size is an estimate) fall back to the pool.
+// create-run-read-destroy cycle.  Requests the arena cannot hold (its size is an estimate) fall back to the pool.  Every
+// buffer of an engine comes from dev_alloc or grow and goes back in release or pipsort_destroy; nothing is allocated while
+// a graph is being captured (its replays could not run until such a buffer were freed, and destroy would free it outside
+// the graph).
+const char* const CAPTURE_NO_ALLOC = "run the pass once before capturing it (the first run allocates what the pass needs)";
+
+// where a buffer may come from: the arena (then the pool when it is full), the pool only, pinned host memory
+enum class Mem { arena, pool, pinned };
+
 template <class T>
-int dev_alloc(pipsort_engine* e, T** p, size_t count) {
+int dev_alloc(pipsort_engine* e, T** p, size_t count, Mem where = Mem::arena) {
     const size_t bytes = (std::max<size_t>(count, 1) * sizeof(T) + 255) & ~(size_t)255;
-    if (e->arena && e->arena_off + bytes <= e->arena_cap) {
+    if (where == Mem::arena && e->arena && e->arena_off + bytes <= e->arena_cap) {
         *p = reinterpret_cast<T*>(e->arena + e->arena_off);
         e->arena_off += bytes;
         return 0;
     }
+    if (e->capturing) return fail(PIPSORT_E_ARG, "%s", CAPTURE_NO_ALLOC);
     void* q = nullptr;
-    CU(cudaMallocAsync(&q, bytes, e->own_stream));
-    e->allocs.push_back(q);
+    const bool pinned = where == Mem::pinned;
+    const cudaError_t err = pinned ? cudaMallocHost(&q, bytes) : cudaMallocAsync(&q, bytes, e->stream);
+    if (err != cudaSuccess) {
+        cudaGetLastError();                  // a refused request leaves no error pending for the engine's next call
+        return fail(PIPSORT_E_CUDA, "allocation of %zu bytes failed: %s", bytes, cudaGetErrorString(err));
+    }
+    e->allocs.push_back({q, pinned});
     *p = static_cast<T*>(q);
     return 0;
+}
+
+// frees a buffer from dev_alloc (stream-ordered; an arena slice stays where it is) and nulls the pointer
+template <class T>
+int release(pipsort_engine* e, T** p) {
+    void* q = *p;
+    *p = nullptr;
+    for (size_t i = 0; i < e->allocs.size(); i++) {
+        if (e->allocs[i].p != q) continue;
+        const bool pinned = e->allocs[i].pinned;
+        e->allocs.erase(e->allocs.begin() + i);
+        CU(pinned ? cudaFreeHost(q) : cudaFreeAsync(q, e->stream));
+        break;
+    }
+    return 0;
+}
+
+// a buffer of at least n elements in *p: keeps it when *cap >= n, else replaces it; on failure *p is null and *cap 0.
+// Buffers that grow on demand come from the pool (or pinned memory), never from the arena: the arena's room is for the locus.
+template <class T>
+int grow(pipsort_engine* e, T** p, size_t* cap, size_t n, Mem where = Mem::pool) {
+    if (*cap >= n) return 0;
+    if (e->capturing) return fail(PIPSORT_E_ARG, "%s", CAPTURE_NO_ALLOC);
+    *cap = 0;
+    int rc = release(e, p);
+    if (!rc) rc = dev_alloc(e, p, n, where);   // sets *p only when it succeeds
+    if (!rc) *cap = n;
+    return rc;
 }
 
 template <class T>
@@ -641,12 +690,17 @@ int mailbox_acquire(int device, int world, size_t bytes, int* slot) {
     auto& c = mailbox_cache();
     for (size_t i = 0; i < c.size(); i++)
         if (!c[i]->in_use && c[i]->device == device && c[i]->world == world && c[i]->bytes >= bytes) { c[i]->in_use = true; *slot = (int)i; return 0; }
-    MailboxEntry* m = new MailboxEntry{device, world, nullptr, bytes + bytes / 2, nullptr, 0, true};
-    CU(cudaMalloc(&m->mailbox, m->bytes));                   // cudaMalloc (not the pool): CUDA IPC needs it
-    CU(cudaMemset(m->mailbox, 0, m->bytes));
-    CU(cudaMalloc(&m->d_done, sizeof(unsigned)));
-    CU(cudaMemset(m->d_done, 0, sizeof(unsigned)));
-    c.push_back(m);
+    MailboxEntry m{device, world, nullptr, bytes + bytes / 2, nullptr, 0, true};
+    cudaError_t err = cudaMalloc(&m.mailbox, m.bytes);       // cudaMalloc (not the pool): CUDA IPC needs it
+    if (err == cudaSuccess) err = cudaMemset(m.mailbox, 0, m.bytes);
+    if (err == cudaSuccess) err = cudaMalloc(&m.d_done, sizeof(unsigned));
+    if (err == cudaSuccess) err = cudaMemset(m.d_done, 0, sizeof(unsigned));
+    if (err != cudaSuccess) {
+        if (m.mailbox) cudaFree(m.mailbox);
+        if (m.d_done) cudaFree(m.d_done);
+        return fail(PIPSORT_E_CUDA, "mailbox allocation failed: %s", cudaGetErrorString(err));
+    }
+    c.push_back(new MailboxEntry(m));
     *slot = (int)c.size() - 1;
     return 0;
 }
@@ -677,46 +731,11 @@ void pipsort_destroy(pipsort_engine* e) {
     if (!e) return;
     cudaSetDevice(e->device);
     if (e->stream) cudaStreamSynchronize(e->stream);
-    if (e->own_stream) {
-        auto in_arena = [&](const void* q) { return e->arena && (const char*)q >= e->arena && (const char*)q < e->arena + e->arena_cap; };
-        // (dev_alloc hands out separate allocations once the arena is full: those are in `allocs` and freed below, once)
-        auto owned = [&](const void* q) { return in_arena(q) || std::find(e->allocs.begin(), e->allocs.end(), q) != e->allocs.end(); };
-        if (e->exh.d_chunks && !owned(e->exh.d_chunks)) cudaFreeAsync(e->exh.d_chunks, e->own_stream);
-        if (e->exh.d_counter && !owned(e->exh.d_counter)) cudaFreeAsync(e->exh.d_counter, e->own_stream);
-        for (void* p : e->allocs) cudaFreeAsync(p, e->own_stream);   // stream-ordered: no second synchronisation needed
-        if (e->arena) cudaFreeAsync(e->arena, e->own_stream);
-    }
-    {
-        pipsort_engine::Sss& q = e->sss;
-        void* ps[] = {q.tab.klo, q.tab.khi, q.tab.val, q.d_out_l, q.d_batch, q.d_upd, q.d_counter, q.d_scored, q.d_state,
-                      q.d_pos_of, q.d_total};
-        for (void* p : ps) if (p) cudaFree(p);
-        if (q.h_out_l) cudaFreeHost(q.h_out_l);
-    }
-    {
-        pipsort_engine::P2P& q = e->p2p;
-        if (q.cache_slot >= 0) mailbox_release(q.cache_slot);   // mailbox, counters and peer mappings stay with the process
-    }
+    for (const pipsort_engine::Alloc& a : e->allocs) a.pinned ? cudaFreeHost(a.p) : cudaFreeAsync(a.p, e->own_stream);
+    if (e->arena) cudaFreeAsync(e->arena, e->own_stream);
+    if (e->p2p.cache_slot >= 0) mailbox_release(e->p2p.cache_slot);   // mailbox, counters and peer mappings stay with the process
     for (cudaGraphExec_t x : e->graphs) cudaGraphExecDestroy(x);
-    if (e->d_idx) cudaFree(e->d_idx);
-    if (e->d_grid) cudaFree(e->d_grid);
-    if (e->d_upd) cudaFree(e->d_upd);
-    if (e->d_out) cudaFree(e->d_out);
-    if (e->own_stream && e->ev0 && e->ev1 && e->evk0 && e->evk1 && e->ev_up) {   // back to the per-device cache
-        StreamKit k{e->own_stream, {e->ev0, e->ev1, e->evk0, e->evk1, e->ev_up}, e->pin};
-        if (e->l2_scratch) cudaFree(e->l2_scratch);
-        kit_release(e->device, k);
-        delete e;
-        return;
-    }
-    if (e->ev0) cudaEventDestroy(e->ev0);
-    if (e->ev1) cudaEventDestroy(e->ev1);
-    if (e->evk0) cudaEventDestroy(e->evk0);
-    if (e->evk1) cudaEventDestroy(e->evk1);
-    if (e->ev_up) cudaEventDestroy(e->ev_up);
-    if (e->l2_scratch) cudaFree(e->l2_scratch);
-
-    if (e->own_stream) cudaStreamDestroy(e->own_stream);
+    if (e->own_stream) kit_release(e->device, StreamKit{e->own_stream, {e->ev0, e->ev1, e->evk0, e->evk1, e->ev_up}, e->pin});
     delete e;
 }
 
@@ -755,6 +774,12 @@ static int grid_prior(const pipsort_engine* e, double gam, double p, double* out
     memcpy(out, pi, sizeof pi);
     out[PRIOR_STRIDE - 1] = -0.5 * e->K + e->U * std::log(1.0 - gam);
     return 0;
+}
+
+// slot rows of the accumulator store: the five per-SNP slots + the scalars' slot, or (class-resolved) 3 c(c+1)/2 class slots
+// per SNP and as many rows as the scalars need (common.cuh)
+static size_t store_rows(bool classes, int kb, size_t upad) {
+    return classes ? (size_t)cls_nslot(kb) + (cls_nscal(kb) + upad - 1) / upad : (size_t)NSLOT;
 }
 
 static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pipsort_engine* e) {
@@ -797,6 +822,7 @@ static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pips
     e->U = U;
     e->K = lc->K; e->gamma = lc->gamma; e->p = lc->sharing_param;
     e->kb = std::min(KMAX, std::max(3, lc->max_causal));
+    e->classes = (flags & PIPSORT_PRIOR_CLASSES) != 0;
     e->use_reg_kernel = !(flags & PIPSORT_GENERIC_ONLY);
 
     TR(0);
@@ -834,10 +860,9 @@ static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pips
     TR(1);
     // ---- arena: everything dev_alloc hands out below (estimate; the accumulator store is sized for 16 bins) ------------
     {
-        const size_t upad = (size_t)std::max((U + 3) & ~3, 4), kb = (size_t)std::min(KMAX, std::max(3, lc->max_causal));
-        const size_t nslot = (flags & PIPSORT_PRIOR_CLASSES) ? cls_nslot((int)kb) + (cls_nscal((int)kb) + upad - 1) / upad + 1 : NSLOT;
+        const size_t upad = (size_t)std::max((U + 3) & ~3, 4);
         size_t est = 64 * 256 + sizeof(LocusDev) + (size_t)(3 + 5 * U + NCOUNTER) * 8 + (size_t)(U + 2) * 8 +
-                     (nslot * 16 * upad + NCOUNTER) * 8;
+                     (store_rows(e->classes, e->kb, upad) * 16 * upad + NCOUNTER) * 8;
         est += ((size_t)e->sm_count * 12 + 256) * sizeof(int4) + 512;               // chunk descriptors of the exhaustive launch
         size_t nints = (size_t)6 * U + 2 * ((size_t)U / 32 + 8);
         for (int s = 0; s < S; s++) {
@@ -900,17 +925,16 @@ static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pips
     TR(3);
     // all host -> device copies of the caller's buffers first, then one event: pipsort_create returns when they are done
     double *up_sigma[2] = {nullptr, nullptr}, *up_z[2] = {nullptr, nullptr};
-    bool up_sigma_temp[2] = {false, false};
+    DevTemp<double> big_sigma[2];   // a large LD matrix is needed only until the preparation launch has read it
     {
         size_t so = 0, zo = 0;
         for (int s = 0; s < S; s++) {
             const size_t nr = (size_t)lc->num_snps[s];
             if (nr * nr * 8 <= ((size_t)4 << 20)) {          // small: from the arena (stays allocated, a few hundred KB)
                 if ((rc = dev_alloc(e, &up_sigma[s], nr * nr))) return rc;
-                up_sigma_temp[s] = false;
             } else {
-                CU(cudaMallocAsync(&up_sigma[s], std::max<size_t>(nr * nr, 1) * sizeof(double), e->stream));
-                up_sigma_temp[s] = true;
+                CU(big_sigma[s].alloc(nr * nr, e->stream));
+                up_sigma[s] = big_sigma[s];
             }
             CU(cudaMemcpyAsync(up_sigma[s], lc->sigma + so, nr * nr * sizeof(double), cudaMemcpyHostToDevice, e->stream));
             if ((rc = dev_upload(e, &up_z[s], lc->z + zo, nr))) return rc;
@@ -934,7 +958,7 @@ static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pips
         if (flags & PIPSORT_RAW_LD) {   // model.h:171-264 on the device: PSD shift + eigen-decomposition -> effective LD, K_s
             std::string why;
             const int prc = prep_study_device(e->stream, n_raw, d_sigma, d_zraw, &e->prep[s], &why, &e->launches);
-            if (prc) { if (up_sigma_temp[s]) cudaFreeAsync(d_sigma, e->stream); return fail(prc == -3 ? PIPSORT_E_RANGE : PIPSORT_E_CUDA, "pre-processing of study %d: %s", s, why.c_str()); }
+            if (prc) return fail(prc == -3 ? PIPSORT_E_RANGE : PIPSORT_E_CUDA, "pre-processing of study %d: %s", s, why.c_str());
             K_total += e->prep[s].K;
             e->prepped = true;
         }
@@ -982,8 +1006,7 @@ static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pips
             e->launches++;
             CU(cudaGetLastError());
         }
-        for (int s = 0; s < S; s++)
-            if (up_sigma_temp[s]) CU(cudaFreeAsync(up_sigma[s], e->stream));
+        for (DevTemp<double>& b : big_sigma) b.free();   // stream-ordered: after the launch that reads it
     }
 
     TR(5);
@@ -991,7 +1014,6 @@ static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pips
     const double gam = lc->gamma, p = lc->sharing_param;
     double minpi = 0.0;
     if ((rc = prior_tables(gam, p, U, e->kb, L.pi, L.logprior, &minpi))) return rc;
-    e->classes = (flags & PIPSORT_PRIOR_CLASSES) != 0;
     if (e->classes) minpi = 0.0;     // the class-resolved store holds unweighted sums: the range of the likelihood-only sums
     e->K = K_total;
     L.neg_half_K = -0.5 * K_total;
@@ -1047,9 +1069,7 @@ static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pips
     acc.NB = ((int)std::ceil(maxexp_bits) + acc.bias) / 512 + 2;
     acc.Upad = std::max((U + 3) & ~3, 4);
     acc.ccls = e->classes ? e->kb : 0;
-    // class-resolved: 3 c(c+1)/2 class slots per SNP, then as many rows as the scalars need (common.cuh)
-    const size_t nslot = e->classes ? (size_t)cls_nslot(e->kb) + (cls_nscal(e->kb) + acc.Upad - 1) / acc.Upad : (size_t)NSLOT;
-    e->bins_len = nslot * acc.NB * acc.Upad + NCOUNTER;   // the counters ride in the tail of the store
+    e->bins_len = store_rows(e->classes, e->kb, acc.Upad) * acc.NB * acc.Upad + NCOUNTER;   // the counters ride in the tail of the store
     if ((rc = dev_alloc(e, &acc.bins, e->bins_len))) return rc;
     acc.counters = acc.bins + (e->bins_len - NCOUNTER);
     if ((rc = dev_alloc(e, &e->d_res, 3 + (size_t)5 * U + NCOUNTER))) return rc;   // results | counters: one D2H per read
@@ -1059,7 +1079,6 @@ static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pips
     CU(cudaMemsetAsync(e->exh.d_counter, 0, 2 * sizeof(unsigned), e->stream));
     e->exh.cap_chunks = (size_t)e->sm_count * 12 + 256;     // one chunk per resident warp + singles tiles: the small-locus plan
     if ((rc = dev_alloc(e, &e->exh.d_chunks, e->exh.cap_chunks))) return rc;
-    e->exh.chunks_in_arena = true;
     e->exh.pin_stage_cap = e->exh.cap_chunks * sizeof(int4);
     e->exh.pin_stage = pin_slice(e, e->exh.pin_stage_cap);
     CU(cudaMemsetAsync(acc.bins, 0, e->bins_len * sizeof(double), e->stream));
@@ -1110,25 +1129,20 @@ int pipsort_preprocess_study(int device, int32_t n, const double* ld, const doub
     if (rcp) return rcp;
     cudaStream_t st;
     CU(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
-    double *dA = nullptr, *dz = nullptr;
+    auto destroy_stream = scope_exit([&] { cudaStreamSynchronize(st); cudaStreamDestroy(st); });   // after the buffers below
+    DevTemp<double> dA, dz;
     const size_t nn = (size_t)n * n;
     PrepResult r;
     std::string why;
     unsigned long long launches = 0;
-    int prc = 0;
-    cudaError_t err = cudaMallocAsync(&dA, std::max<size_t>(nn, 1) * sizeof(double), st);
-    if (err == cudaSuccess) err = cudaMallocAsync(&dz, std::max<size_t>(n, 1) * sizeof(double), st);
-    if (err == cudaSuccess && n) err = cudaMemcpyAsync(dA, ld, nn * sizeof(double), cudaMemcpyHostToDevice, st);
-    if (err == cudaSuccess && n) err = cudaMemcpyAsync(dz, z, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st);
-    if (err == cudaSuccess) prc = prep_study_device(st, n, dA, dz, &r, &why, &launches);
-    if (err == cudaSuccess && !prc && n) err = cudaMemcpyAsync(sigma_eff, dA, nn * sizeof(double), cudaMemcpyDeviceToHost, st);
-    if (err == cudaSuccess) err = cudaStreamSynchronize(st);
-    if (dA) cudaFreeAsync(dA, st);
-    if (dz) cudaFreeAsync(dz, st);
-    cudaStreamSynchronize(st);
-    cudaStreamDestroy(st);
-    if (err != cudaSuccess) return fail(PIPSORT_E_CUDA, "pre-processing failed: %s", cudaGetErrorString(err));
+    CU(dA.alloc(nn, st));
+    CU(dz.alloc(n, st));
+    if (n) CU(cudaMemcpyAsync(dA, ld, nn * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (n) CU(cudaMemcpyAsync(dz, z, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st));
+    const int prc = prep_study_device(st, n, dA, dz, &r, &why, &launches);
     if (prc) return fail(prc == -3 ? PIPSORT_E_RANGE : PIPSORT_E_CUDA, "pre-processing: %s", why.c_str());
+    if (n) CU(cudaMemcpyAsync(sigma_eff, dA, nn * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
     if (info) { info->add_diag = r.add_diag; info->K = r.K; info->min_abs_eig = r.min_abs_eig; info->n_negative = r.n_negative; info->psd_iterations = r.psd_iterations; }
     return 0;
 }
@@ -1217,7 +1231,7 @@ int pipsort_run_exhaustive(pipsort_engine* e, int c, uint64_t rank_begin, uint64
     const int jreg = e->use_reg_kernel ? std::min(std::min(c, 3), e->U) : -1;
     if (jreg >= 2 && !e->L.st[0].WP) {
         // first exhaustive run with pairs / triples: build the tables { W_ij, E_s{i,j} } (16 (n_s + 1)^2 bytes per study, once)
-        if (e->capturing) return fail(PIPSORT_E_ARG, "run the pass once before capturing it (the first run builds the pair tables)");
+        if (e->capturing) return fail(PIPSORT_E_ARG, "%s", CAPTURE_NO_ALLOC);
         PairTablesArgs pt;
         for (int s = 0; s < 2; s++) {
             StudyDev& st = e->L.st[s];
@@ -1240,8 +1254,11 @@ int pipsort_run_exhaustive(pipsort_engine* e, int c, uint64_t rank_begin, uint64
     }
     if (jreg >= 0) {
         const bool timed = jdom <= jreg && !e->capturing;
-        if ((rc = exhaustive_launch_all(e->L, e->d_L, c, rank_begin, rank_end, e->sm_count, e->stream, &e->launches, &e->exh,
-                                        &e->cost_model, timed ? e->evk0 : nullptr, timed ? e->evk1 : nullptr)))
+        if ((rc = exhaustive_plan(e->L, c, rank_begin, rank_end, e->sm_count, &e->exh, &e->cost_model)))
+            return fail(PIPSORT_E_CUDA, "exhaustive kernel launch failed: %s", cudaGetErrorString((cudaError_t)rc));
+        const size_t nd = e->exh.plan.n_total;     // a larger plan gets headroom: plans differ a little between rank ranges
+        if (nd > e->exh.cap_chunks && (rc = grow(e, &e->exh.d_chunks, &e->exh.cap_chunks, nd + nd / 4 + 64))) return rc;
+        if ((rc = exhaustive_launch(e->L, e->d_L, e->stream, &e->launches, &e->exh, timed ? e->evk0 : nullptr, timed ? e->evk1 : nullptr)))
             return fail(PIPSORT_E_CUDA, "exhaustive kernel launch failed: %s", cudaGetErrorString((cudaError_t)rc));
         if (timed) e->evk_valid = true;
     }
@@ -1338,13 +1355,12 @@ int pipsort_score_union_configs(pipsort_engine* e, const int32_t* idx, int64_t n
     if (!idx && kmax > 0) return fail(PIPSORT_E_ARG, "null idx");
     CU(cudaSetDevice(e->device));
     const size_t ni = (size_t)n * std::max(kmax, 1);
-    if (e->cap_idx < ni) { if (e->d_idx) cudaFree(e->d_idx); CU(cudaMalloc(&e->d_idx, ni * sizeof(int))); e->cap_idx = ni; }
-    if (e->cap_upd < (size_t)n) { if (e->d_upd) cudaFree(e->d_upd); CU(cudaMalloc(&e->d_upd, n)); e->cap_upd = n; }
-    if (e->cap_out < (size_t)n) { if (e->d_out) cudaFree(e->d_out); CU(cudaMalloc(&e->d_out, n * sizeof(double))); e->cap_out = n; }
+    int rc;
+    if ((rc = grow(e, &e->d_idx, &e->cap_idx, ni)) || (rc = grow(e, &e->d_upd, &e->cap_upd, n)) || (rc = grow(e, &e->d_out, &e->cap_out, n)))
+        return rc;
     if (kmax > 0) CU(cudaMemcpyAsync(e->d_idx, idx, (size_t)n * kmax * sizeof(int), cudaMemcpyHostToDevice, e->stream));
     if (make_updates) CU(cudaMemcpyAsync(e->d_upd, make_updates, n, cudaMemcpyHostToDevice, e->stream));
-    int rc = pipsort_score_union_configs_device(e, e->d_idx, n, kmax, make_updates ? e->d_upd : nullptr, e->d_out);
-    if (rc) return rc;
+    if ((rc = pipsort_score_union_configs_device(e, e->d_idx, n, kmax, make_updates ? e->d_upd : nullptr, e->d_out))) return rc;
     if (out_max_abs_l) CU(cudaMemcpyAsync(out_max_abs_l, e->d_out, n * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
     return check_flags(e);      // one synchronisation: the values and the error counters (a refused row, a singular block)
 }
@@ -1373,31 +1389,28 @@ static int sss_conv_from() {
     return v ? std::max(0, atoi(v)) : 99;
 }
 
-static int sss_table_alloc(SssTable* t, u64 cap, cudaStream_t st) {
-    t->mask = cap - 1;
-    CU(cudaMalloc(&t->klo, cap * sizeof(u64)));
-    CU(cudaMalloc(&t->khi, cap * sizeof(u64)));
-    CU(cudaMalloc(&t->val, cap * sizeof(double)));
-    CU(cudaMemsetAsync(t->khi, 0, cap * sizeof(u64), st));
-    return 0;
-}
-
 static int sss_table_reserve(pipsort_engine* e, u64 need) {   // capacity >= 2 * need
-    pipsort_engine::Sss& q = e->sss;
-    u64 cap = q.tab.khi ? q.tab.mask + 1 : 0;
+    SssTable& t = e->sss.tab;
+    const u64 cap = t.khi ? t.mask + 1 : 0;
     if (cap >= 2 * need && cap) return 0;
     u64 ncap = std::max<u64>(cap, 1u << 16);
     while (ncap < 2 * need) ncap <<= 1;
-    SssTable nt{nullptr, nullptr, nullptr, 0};
-    int rc = sss_table_alloc(&nt, ncap, e->stream);
-    if (rc) return rc;
-    if (q.tab.khi) {
-        sss_rehash_kernel<<<(unsigned)((cap + 255) / 256), 256, 0, e->stream>>>(q.tab, nt);
-        e->launches++;
-        CU(cudaStreamSynchronize(e->stream));
-        cudaFree(q.tab.klo); cudaFree(q.tab.khi); cudaFree(q.tab.val);
+    SssTable nt{nullptr, nullptr, nullptr, ncap - 1};
+    int rc;
+    if ((rc = dev_alloc(e, &nt.klo, ncap, Mem::pool)) || (rc = dev_alloc(e, &nt.khi, ncap, Mem::pool)) ||
+        (rc = dev_alloc(e, &nt.val, ncap, Mem::pool))) {
+        release(e, &nt.klo); release(e, &nt.khi);
+        return rc;
     }
-    q.tab = nt;
+    CU(cudaMemsetAsync(nt.khi, 0, ncap * sizeof(u64), e->stream));
+    if (t.khi) {
+        sss_rehash_kernel<<<(unsigned)((cap + 255) / 256), 256, 0, e->stream>>>(t, nt);
+        e->launches++;
+        CU(cudaGetLastError());
+    }
+    SssTable old = t;
+    t = nt;
+    if ((rc = release(e, &old.klo)) || (rc = release(e, &old.khi)) || (rc = release(e, &old.val))) return rc;
     return 0;
 }
 
@@ -1425,24 +1438,14 @@ static int sss_run(pipsort_engine* e, int c, int max_iterations, int32_t* iterat
     pipsort_engine::Sss& q = e->sss;
     const int kmax = std::max(c, 1);
     const long long n_max = (long long)U * std::max(c, 1) + c + U + 1;
-    if (q.n_max < n_max || q.kmax != kmax) {
-        void* ps[] = {q.d_out_l, q.d_batch, q.d_upd, q.d_counter, q.d_scored, q.d_state, q.d_pos_of, q.d_total};
-        for (void* p : ps) if (p) cudaFree(p);
-        if (q.h_out_l) cudaFreeHost(q.h_out_l);
-        q.h_out_l = nullptr;
-        CU(cudaMalloc(&q.d_out_l, (size_t)(n_max + 1) * sizeof(double)));
-        CU(cudaMalloc(&q.d_batch, (size_t)(n_max + 1) * kmax * sizeof(int)));
-        CU(cudaMalloc(&q.d_upd, (size_t)(n_max + 1)));
-        CU(cudaMalloc(&q.d_counter, 2 * sizeof(int)));
-        CU(cudaMalloc(&q.d_scored, (size_t)(n_max + 1) * sizeof(double)));
-        CU(cudaMalloc(&q.d_state, (size_t)(n_max + 1)));
-        CU(cudaMalloc(&q.d_pos_of, (size_t)(n_max + 1) * sizeof(int)));
-        CU(cudaMalloc(&q.d_total, sizeof(double)));
-        CU(cudaMallocHost(&q.h_out_l, (size_t)(n_max + 2) * sizeof(double)));
-        q.n_max = n_max; q.kmax = kmax;
-    }
-    int rc = pipsort_sss_reset(e);
-    if (rc) return rc;
+    const size_t m = (size_t)n_max + 1;
+    int rc;
+    if ((rc = grow(e, &q.d_out_l, &q.cap_out_l, m)) || (rc = grow(e, &q.d_batch, &q.cap_batch, m * kmax)) ||
+        (rc = grow(e, &q.d_upd, &q.cap_upd, m)) || (rc = grow(e, &q.d_counter, &q.cap_counter, 2)) ||
+        (rc = grow(e, &q.d_scored, &q.cap_scored, m)) || (rc = grow(e, &q.d_state, &q.cap_state, m)) ||
+        (rc = grow(e, &q.d_pos_of, &q.cap_pos_of, m)) || (rc = grow(e, &q.d_total, &q.cap_total, 1)) ||
+        (rc = grow(e, &q.h_out_l, &q.cap_h_out_l, m + 1, Mem::pinned)) || (rc = pipsort_sss_reset(e)))
+        return rc;
     const size_t acc_len = p2p_acc_len(e), half = p2p_sss_half(e), stride = p2p_slot_len(e);
     if (world > 1 && (size_t)n_max + (size_t)e->L.acc.NB > half) return fail(PIPSORT_E_ARG, "mailbox too small for this max_causal");
     double* errf = e->L.acc.counters + 1 + ERR_P2P_TIMEOUT;
@@ -1551,12 +1554,13 @@ int pipsort_score_given_configs(pipsort_engine* e, const int16_t* configs, int64
     // stream the matrix through two pinned-size device chunks so that arbitrarily large files (it is mmapped by the
     // caller, postcal.cpp:429) never need more than a bounded staging buffer
     const int64_t rows_per_chunk = std::max<int64_t>(1, ((int64_t)64 << 20) / std::max(1, num_groups * 2));
-    int16_t* d_buf[2] = {nullptr, nullptr};
+    DevTemp<int16_t> d_buf[2];
     cudaEvent_t done[2] = {nullptr, nullptr};
+    auto destroy_events = scope_exit([&] { for (cudaEvent_t ev : done) if (ev) cudaEventDestroy(ev); });
     const int64_t cap = std::min(rows_per_chunk, num_configs);
     int rc = 0;
     for (int i = 0; i < 2 && !rc; i++) {
-        if (cudaMallocAsync((void**)&d_buf[i], (size_t)cap * std::max(1, num_groups) * sizeof(int16_t), e->stream) != cudaSuccess ||
+        if (d_buf[i].alloc((size_t)cap * std::max(1, num_groups), e->stream) != cudaSuccess ||
             cudaEventCreateWithFlags(&done[i], cudaEventDisableTiming) != cudaSuccess)
             rc = fail(PIPSORT_E_CUDA, "staging buffer allocation failed");
         if (num_configs <= cap) break;
@@ -1570,10 +1574,6 @@ int pipsort_score_given_configs(pipsort_engine* e, const int16_t* configs, int64
                             e->stream) != cudaSuccess) { rc = fail(PIPSORT_E_CUDA, "H2D copy of the configuration matrix failed"); break; }
         rc = pipsort_score_given_configs_device(e, d_buf[cur], nr, num_groups);
         if (!rc && cudaEventRecord(done[cur], e->stream) != cudaSuccess) rc = fail(PIPSORT_E_CUDA, "event record failed");
-    }
-    for (int i = 0; i < 2; i++) {
-        if (d_buf[i]) cudaFreeAsync(d_buf[i], e->stream);
-        if (done[i]) cudaEventDestroy(done[i]);
     }
     if (rc) return rc;
     return check_flags(e);
@@ -1734,14 +1734,10 @@ int pipsort_read_prior_grid(pipsort_engine* e, int n_priors, const double* gamma
         if (rc) { const std::string why = g_err; return fail(rc, "prior %d: %s", i, why.c_str()); }
     }
     CU(cudaSetDevice(e->device));
-    if (e->cap_grid < need) {
-        if (e->d_grid) { CU(cudaStreamSynchronize(e->stream)); CU(cudaFree(e->d_grid)); e->d_grid = nullptr; }
-        CU(cudaMalloc(&e->d_grid, need * sizeof(double)));
-        e->cap_grid = need;
-    }
+    int rc;
+    if ((rc = grow(e, &e->d_grid, &e->cap_grid, need))) return rc;
     CU(cudaMemcpyAsync(e->d_grid, e->h_grid.data(), npri * sizeof(double), cudaMemcpyHostToDevice, e->stream));
-    int rc = finalize_grid_launch(e, n_priors, e->d_grid, e->d_grid + npri, false);
-    if (rc) return rc;
+    if ((rc = finalize_grid_launch(e, n_priors, e->d_grid, e->d_grid + npri, false))) return rc;
     CU(cudaMemcpyAsync(e->h_grid.data() + npri, e->d_grid + npri, (need - npri) * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
     CU(cudaStreamSynchronize(e->stream));
     const double* res = e->h_grid.data() + npri;
@@ -1893,15 +1889,13 @@ int pipsort_enumerate(pipsort_engine* e, int c, uint64_t rank, uint32_t expansio
     if (rc) return rc;
     if (rank >= total) return fail(PIPSORT_E_ARG, "rank out of range");
     CU(cudaSetDevice(e->device));
-    int* d = nullptr;
-    CU(cudaMalloc(&d, (2 * KMAX + 1) * sizeof(int)));
+    DevTemp<int> d;
+    CU(d.alloc(2 * KMAX + 1, e->stream));
     enumerate_kernel<<<1, 32, 0, e->stream>>>(e->U, e->d_snp_map, c, rank, expansion, d, d + KMAX, (unsigned*)(d + 2 * KMAX));
     e->launches++;
     int h[2 * KMAX + 1];
-    cudaError_t err = cudaMemcpyAsync(h, d, sizeof h, cudaMemcpyDeviceToHost, e->stream);
-    if (err == cudaSuccess) err = cudaStreamSynchronize(e->stream);
-    cudaFree(d);
-    if (err != cudaSuccess) return fail(PIPSORT_E_CUDA, "enumerate failed: %s", cudaGetErrorString(err));
+    CU(cudaMemcpyAsync(h, d, sizeof h, cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaStreamSynchronize(e->stream));
     for (int i = 0; i < c; i++) { out_union_idx[i] = h[i]; out_state[i] = h[KMAX + i]; }
     if (n_expansions) *n_expansions = (uint32_t)h[2 * KMAX];
     return 0;
@@ -1921,10 +1915,10 @@ int pipsort_merge(pipsort_engine* dst, pipsort_engine* src) {
     CU(cudaSetDevice(src->device));
     CU(cudaStreamSynchronize(src->stream));
     CU(cudaSetDevice(dst->device));
-    double* tmp = nullptr;
+    DevTemp<double> tmp;
     const double* from = src->L.acc.bins;
     if (src->device != dst->device) {
-        CU(cudaMalloc(&tmp, dst->bins_len * sizeof(double)));
+        CU(tmp.alloc(dst->bins_len, dst->stream));
         CU(cudaMemcpyPeerAsync(tmp, dst->device, src->L.acc.bins, src->device, dst->bins_len * sizeof(double), dst->stream));
         from = tmp;
     }
@@ -1932,7 +1926,6 @@ int pipsort_merge(pipsort_engine* dst, pipsort_engine* src) {
     dst->launches++;
     CU(cudaGetLastError());
     CU(cudaStreamSynchronize(dst->stream));
-    if (tmp) CU(cudaFree(tmp));
     return 0;   // the configuration count and the error counters are part of the store
 }
 
@@ -2155,7 +2148,8 @@ int pipsort_flush_l2(pipsort_engine* e) {
     if (!e) return fail(PIPSORT_E_ARG, "null engine");
     CU(cudaSetDevice(e->device));
     const size_t bytes = (size_t)256 << 20;   // L2 is 126 MB
-    if (!e->l2_scratch) CU(cudaMalloc(&e->l2_scratch, bytes));
+    int rc = grow(e, &e->l2_scratch, &e->cap_l2, bytes);
+    if (rc) return rc;
     CU(cudaMemsetAsync(e->l2_scratch, 0x5a, bytes, e->stream));
     return 0;
 }
@@ -2192,9 +2186,10 @@ int pipsort_measure_fp64_peak(int device, double* flops_per_sec) {
     CU(cudaSetDevice(device));
     cudaDeviceProp prop;
     CU(cudaGetDeviceProperties(&prop, device));
-    double* d = nullptr;
-    CU(cudaMalloc(&d, sizeof(double)));
-    cudaEvent_t a, b;
+    DevTemp<double> d;
+    CU(d.alloc(1, 0));
+    cudaEvent_t a = nullptr, b = nullptr;
+    auto destroy_events = scope_exit([&] { if (a) cudaEventDestroy(a); if (b) cudaEventDestroy(b); });
     CU(cudaEventCreate(&a));
     CU(cudaEventCreate(&b));
     const int blocks = prop.multiProcessorCount * 8, threads = 256, iters = 4096;
@@ -2209,9 +2204,6 @@ int pipsort_measure_fp64_peak(int device, double* flops_per_sec) {
         const double fl = 2.0 * 64.0 * iters * (double)blocks * threads;
         if (rep > 0) best = std::max(best, fl / (ms * 1e-3));
     }
-    cudaEventDestroy(a);
-    cudaEventDestroy(b);
-    cudaFree(d);
     *flops_per_sec = best;
     return 0;
 }

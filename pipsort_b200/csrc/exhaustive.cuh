@@ -14,16 +14,15 @@
 
 namespace pipsort {
 
-struct ExhScratch {           // owned by the engine, reused across launches
+struct ExhScratch {           // owned by the engine, reused across launches; the engine allocates both buffers
     int4* d_chunks = nullptr;     // chunk descriptors of the plan on the device
     size_t cap_chunks = 0;
-    bool chunks_in_arena = false; // the buffer belongs to the engine's arena: never freed on its own
     unsigned* d_counter = nullptr;   // [0] work-queue head, [1] finished blocks (the kernel re-arms both)
     int occ = 0;                  // resident blocks per SM of exhaustive_all_kernel
     char* pin_stage = nullptr;    // pinned staging slice for the FIRST descriptor upload (later ones may overlap an in-flight copy)
     size_t pin_stage_cap = 0;
     std::shared_ptr<const std::vector<ExhChunkDesc>> host_plan;   // keeps a pageable upload source alive
-    // the plan of the last launch (a pass is usually repeated with the same c and rank range)
+    // the plan of the last launch (a pass is usually repeated with the same c and rank range); valid once it is uploaded
     bool plan_valid = false;
     int plan_c = 0;
     unsigned long long plan_rb = 0, plan_re = 0;
@@ -168,24 +167,18 @@ inline std::shared_ptr<const std::vector<ExhChunkDesc>> exh_plan_chunks(const Ex
     return plan;
 }
 
-// Launches ONE kernel for the size classes 0..min(c,3) restricted to the global union-subset rank range
-// [rank_begin, rank_end) (size-then-lexicographic order over the internal SNP order).  Returns a cudaError_t.
-// ev0 / ev1 (optional) are recorded immediately around the kernel launch: the host-side planning is NOT part of the
-// kernel's device time.
-inline int exhaustive_launch_all(const LocusDev& L, const LocusDev* Lg, int c, u64 rank_begin, u64 rank_end, int sm_count,
-                                 cudaStream_t stream, unsigned long long* launches, ExhScratch* sc, const ExhCostModel* M,
-                                 cudaEvent_t ev0 = nullptr, cudaEvent_t ev1 = nullptr) {
+// The plan of ONE kernel for the size classes 0..min(c,3) restricted to the global union-subset rank range
+// [rank_begin, rank_end) (size-then-lexicographic order over the internal SNP order).  Returns a cudaError_t.  Unless the
+// plan of the last launch is reused, sc->plan.n_total descriptors then have to fit sc->d_chunks before exhaustive_launch.
+inline int exhaustive_plan(const LocusDev& L, int c, u64 rank_begin, u64 rank_end, int sm_count, ExhScratch* sc,
+                           const ExhCostModel* M) {
     const int U = L.U;
     cudaError_t err;
-    if (!sc->d_counter) {
-        if ((err = cudaMallocAsync(&sc->d_counter, 2 * sizeof(unsigned), stream)) != cudaSuccess) return (int)err;
-        if ((err = cudaMemsetAsync(sc->d_counter, 0, 2 * sizeof(unsigned), stream)) != cudaSuccess) return (int)err;
-    }
     // the instantiation that matches the engine's store (class-resolved: PIPSORT_PRIOR_CLASSES)
     const bool cr = L.acc.ccls > 0;
-    void (*kernel)(LocusDev, ExhAll, const LocusDev*) = cr ? exhaustive_all_kernel<true> : exhaustive_all_kernel<false>;
-    const size_t smem = cr ? EXH_SMEM_BYTES_CR : EXH_SMEM_BYTES;
     if (!sc->occ) {
+        void (*kernel)(LocusDev, ExhAll, const LocusDev*) = cr ? exhaustive_all_kernel<true> : exhaustive_all_kernel<false>;
+        const size_t smem = cr ? EXH_SMEM_BYTES_CR : EXH_SMEM_BYTES;
         // (the attribute is per device: set it for every engine, not once per process)
         if ((err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return (int)err;
         static int occ_cache[2] = {0, 0};    // a property of the kernel and the device generation: query once per process
@@ -195,66 +188,68 @@ inline int exhaustive_launch_all(const LocusDev& L, const LocusDev* Lg, int c, u
         sc->occ = occ_cache[cr];
     }
     const double forced = [] { const char* v = getenv("PIPSORT_EXH_CHUNK"); return v ? atof(v) : 0.0; }();   // experiments / tests
-    if (!(sc->plan_valid && !(forced > 0.0) && sc->plan_c == c && sc->plan_rb == rank_begin && sc->plan_re == rank_end)) {
-        ExhAll A;
-        memset(&A, 0, sizeof A);
-        u64 off = 0;
-        bool have3 = false, have2 = false;
-        int n1_tiles = 0, tile1_0 = 0, do_null = 0;
-        for (int j = 0; j <= std::min(std::min(c, 3), U); j++) {
-            const u64 cnt = exh_binom(U, j);
-            const u64 lo = std::max<u64>(rank_begin, off), hi = std::min<u64>(rank_end, off + cnt);
-            if (lo < hi) {
-                const u64 rb = lo - off, re = hi - off;
-                if (j == 0) do_null = 1;
-                else if (j == 1) { A.x1_lo = (int)rb; A.x1_hi = (int)re; tile1_0 = A.x1_lo >> 5; n1_tiles = ((A.x1_hi - 1) >> 5) - tile1_0 + 1; }
-                else if (j == 2) have2 = exh_class_params(A.p2, U, 2, rb, re);
-                else have3 = exh_class_params(A.p3, U, 3, rb, re);
-            }
-            off += cnt;
+    if (sc->plan_valid && !(forced > 0.0) && sc->plan_c == c && sc->plan_rb == rank_begin && sc->plan_re == rank_end) return 0;
+    ExhAll A;
+    memset(&A, 0, sizeof A);
+    u64 off = 0;
+    bool have3 = false, have2 = false;
+    int n1_tiles = 0, tile1_0 = 0, do_null = 0;
+    for (int j = 0; j <= std::min(std::min(c, 3), U); j++) {
+        const u64 cnt = exh_binom(U, j);
+        const u64 lo = std::max<u64>(rank_begin, off), hi = std::min<u64>(rank_end, off + cnt);
+        if (lo < hi) {
+            const u64 rb = lo - off, re = hi - off;
+            if (j == 0) do_null = 1;
+            else if (j == 1) { A.x1_lo = (int)rb; A.x1_hi = (int)re; tile1_0 = A.x1_lo >> 5; n1_tiles = ((A.x1_hi - 1) >> 5) - tile1_0 + 1; }
+            else if (j == 2) have2 = exh_class_params(A.p2, U, 2, rb, re);
+            else have3 = exh_class_params(A.p3, U, 3, rb, re);
         }
-        const int occ = std::max(1, sc->occ);
-        const int slots = sm_count * occ * EXH_WARPS;
-        const ExhPlanKey key{U, c, slots, rank_begin, rank_end, forced > 0.0 ? forced : 0.0, M ? M->hash : 0};
-        auto plan = exh_plan_chunks(key, have3, A.p3, have2, n1_tiles, tile1_0, do_null, M);
-        A.n_total = (unsigned)plan->size();
-        sc->plan_valid = false;
-        if (A.n_total) {
-            if (plan->size() >= 0xfff00000ull) return (int)cudaErrorInvalidValue;   // 32-bit work queue (never in practice)
-            if (sc->cap_chunks < plan->size()) {     // (rarely for a buffer that came from the engine's arena)
-                // an earlier buffer may still be read by a queued launch: stream-ordered free
-                if (sc->d_chunks && sc->cap_chunks && !sc->chunks_in_arena) cudaFreeAsync(sc->d_chunks, stream);
-                sc->chunks_in_arena = false;
-                sc->cap_chunks = plan->size() + plan->size() / 4 + 64;
-                if ((err = cudaMallocAsync(&sc->d_chunks, sc->cap_chunks * sizeof(int4), stream)) != cudaSuccess) return (int)err;
-            }
-            const size_t bytes = plan->size() * sizeof(ExhChunkDesc);
-            const void* src = plan->data();
-            sc->host_plan = plan;                    // the copy below may still be reading it after this call returns
-            if (sc->pin_stage && bytes <= sc->pin_stage_cap) {
-                memcpy(sc->pin_stage, plan->data(), bytes);
-                src = sc->pin_stage;
-                sc->pin_stage = nullptr;             // one use
-            }
-            if ((err = cudaMemcpyAsync(sc->d_chunks, src, bytes, cudaMemcpyHostToDevice, stream)) != cudaSuccess) return (int)err;
-        }
-        static const bool debug = getenv("PIPSORT_EXH_DEBUG") != nullptr;
-        if (debug) {
-            double st = 0; unsigned mx = 0;
-            for (const ExhChunkDesc& d : *plan) { const unsigned n = d.nsteps_kind & 0x0fffffff; st += n; mx = std::max(mx, n); }
-            fprintf(stderr, "[exhaustive] U=%d c=%d slots=%d chunks=%u steps=%.0f longest=%u cost3=%.0f\n", U, c, slots, A.n_total, st, mx,
-                    have3 ? exh_class_steps(*M, 3, A.p3.a_lo, A.p3.a_hi, true) : 0.0);
-        }
-        A.chunks = sc->d_chunks;
-        A.counter = sc->d_counter;
-        sc->plan = A;
-        sc->plan_blocks = (int)std::min<u64>(((u64)A.n_total + EXH_WARPS - 1) / EXH_WARPS, (u64)sm_count * occ);
-        sc->plan_valid = true; sc->plan_c = c; sc->plan_rb = rank_begin; sc->plan_re = rank_end;
+        off += cnt;
     }
+    const int occ = std::max(1, sc->occ);
+    const int slots = sm_count * occ * EXH_WARPS;
+    const ExhPlanKey key{U, c, slots, rank_begin, rank_end, forced > 0.0 ? forced : 0.0, M ? M->hash : 0};
+    auto plan = exh_plan_chunks(key, have3, A.p3, have2, n1_tiles, tile1_0, do_null, M);
+    if (plan->size() >= 0xfff00000ull) return (int)cudaErrorInvalidValue;   // 32-bit work queue (never in practice)
+    A.n_total = (unsigned)plan->size();
+    static const bool debug = getenv("PIPSORT_EXH_DEBUG") != nullptr;
+    if (debug) {
+        double st = 0; unsigned mx = 0;
+        for (const ExhChunkDesc& d : *plan) { const unsigned n = d.nsteps_kind & 0x0fffffff; st += n; mx = std::max(mx, n); }
+        fprintf(stderr, "[exhaustive] U=%d c=%d slots=%d chunks=%u steps=%.0f longest=%u cost3=%.0f\n", U, c, slots, A.n_total, st, mx,
+                have3 ? exh_class_steps(*M, 3, A.p3.a_lo, A.p3.a_hi, true) : 0.0);
+    }
+    sc->host_plan = plan;                    // the upload may still be reading it after exhaustive_launch returns
+    sc->plan = A;
+    sc->plan_blocks = (int)std::min<u64>(((u64)A.n_total + EXH_WARPS - 1) / EXH_WARPS, (u64)sm_count * occ);
+    sc->plan_valid = false; sc->plan_c = c; sc->plan_rb = rank_begin; sc->plan_re = rank_end;
+    return 0;
+}
+
+// Uploads a new plan to sc->d_chunks and launches it.  Returns a cudaError_t.  ev0 / ev1 (optional) are recorded
+// immediately around the kernel launch: the host-side planning is NOT part of the kernel's device time.
+inline int exhaustive_launch(const LocusDev& L, const LocusDev* Lg, cudaStream_t stream, unsigned long long* launches, ExhScratch* sc,
+                             cudaEvent_t ev0 = nullptr, cudaEvent_t ev1 = nullptr) {
     static_assert(sizeof(ExhChunkDesc) == sizeof(int4), "descriptor layout");
+    cudaError_t err;
+    if (!sc->plan_valid && sc->plan.n_total) {
+        const size_t bytes = sc->host_plan->size() * sizeof(ExhChunkDesc);
+        const void* src = sc->host_plan->data();
+        if (sc->pin_stage && bytes <= sc->pin_stage_cap) {
+            memcpy(sc->pin_stage, src, bytes);
+            src = sc->pin_stage;
+            sc->pin_stage = nullptr;             // one use
+        }
+        if ((err = cudaMemcpyAsync(sc->d_chunks, src, bytes, cudaMemcpyHostToDevice, stream)) != cudaSuccess) return (int)err;
+        sc->plan.chunks = sc->d_chunks;
+        sc->plan.counter = sc->d_counter;
+    }
+    sc->plan_valid = true;
     if (sc->plan.n_total == 0) return 0;
+    const bool cr = L.acc.ccls > 0;
     if (ev0 && (err = cudaEventRecord(ev0, stream)) != cudaSuccess) return (int)err;
-    kernel<<<sc->plan_blocks, EXH_WARPS * 32, smem, stream>>>(L, sc->plan, Lg);
+    if (cr) exhaustive_all_kernel<true><<<sc->plan_blocks, EXH_WARPS * 32, EXH_SMEM_BYTES_CR, stream>>>(L, sc->plan, Lg);
+    else exhaustive_all_kernel<false><<<sc->plan_blocks, EXH_WARPS * 32, EXH_SMEM_BYTES, stream>>>(L, sc->plan, Lg);
     if (ev1 && (err = cudaEventRecord(ev1, stream)) != cudaSuccess) return (int)err;
     (*launches)++;
     return (int)cudaGetLastError();

@@ -240,34 +240,23 @@ inline int prep_study_device(cudaStream_t stream, int n, double* dA, const doubl
     if (!cs.ok) { *why = "cuSOLVER (libcusolver.so.11) could not be loaded"; return -1; }
     cusolverDnHandle_t h = nullptr;
     if (cs.Create(&h) != CUSOLVER_STATUS_SUCCESS) { *why = "cusolverDnCreate failed"; return -2; }
-    double *dW = nullptr, *dwork = nullptr, *dev = nullptr, *dt = nullptr, *dscal = nullptr;
-    int *dipiv = nullptr, *dinfo = nullptr;
-    int rc = 0;
+    auto destroy_handle = scope_exit([&] { cudaStreamSynchronize(stream); cs.Destroy(h); });   // after the buffers below
+    DevTemp<double> dW, dwork, dev, dt, dscal;
+    DevTemp<int> dipiv, dinfo, dflag;
     const size_t nn = (size_t)n * n;
-    auto cleanup = [&]() {
-        if (dW) cudaFreeAsync(dW, stream);
-        if (dwork) cudaFreeAsync(dwork, stream);
-        if (dev) cudaFreeAsync(dev, stream);
-        if (dt) cudaFreeAsync(dt, stream);
-        if (dscal) cudaFreeAsync(dscal, stream);
-        if (dipiv) cudaFreeAsync(dipiv, stream);
-        if (dinfo) cudaFreeAsync(dinfo, stream);
-        cudaStreamSynchronize(stream);
-        cs.Destroy(h);
-    };
-#define PREP_CU(call) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) { *why = std::string(#call " failed: ") + cudaGetErrorString(e__); cleanup(); return -2; } } while (0)
-#define PREP_CS(call) do { cusolverStatus_t s__ = (call); if (s__ != CUSOLVER_STATUS_SUCCESS) { *why = std::string(#call " failed: status ") + std::to_string((int)s__); cleanup(); return -2; } } while (0)
+#define PREP_CU(call) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) { *why = std::string(#call " failed: ") + cudaGetErrorString(e__); return -2; } } while (0)
+#define PREP_CS(call) do { cusolverStatus_t s__ = (call); if (s__ != CUSOLVER_STATUS_SUCCESS) { *why = std::string(#call " failed: status ") + std::to_string((int)s__); return -2; } } while (0)
     PREP_CS(cs.SetStream(h, stream));
     int lw_lu = 0, lw_ev = 0;
-    PREP_CU(cudaMallocAsync(&dW, nn * sizeof(double), stream));
-    PREP_CU(cudaMallocAsync(&dev, (size_t)n * sizeof(double), stream));
-    PREP_CU(cudaMallocAsync(&dt, (size_t)n * sizeof(double), stream));
-    PREP_CU(cudaMallocAsync(&dscal, 4 * sizeof(double), stream));
-    PREP_CU(cudaMallocAsync(&dipiv, (size_t)n * sizeof(int), stream));
-    PREP_CU(cudaMallocAsync(&dinfo, sizeof(int), stream));
+    PREP_CU(dW.alloc(nn, stream));
+    PREP_CU(dev.alloc(n, stream));
+    PREP_CU(dt.alloc(n, stream));
+    PREP_CU(dscal.alloc(4, stream));
+    PREP_CU(dipiv.alloc(n, stream));
+    PREP_CU(dinfo.alloc(1, stream));
     PREP_CS(cs.Dgetrf_bufferSize(h, n, n, dW, n, &lw_lu));
     PREP_CS(cs.Dsyevd_bufferSize(h, CUSOLVER_EIG_MODE_VECTOR, CUBLAS_FILL_MODE_UPPER, n, dW, n, dev, &lw_ev));
-    PREP_CU(cudaMallocAsync(&dwork, (size_t)std::max(std::max(lw_lu, lw_ev), 1) * sizeof(double), stream));
+    PREP_CU(dwork.alloc(std::max(std::max(lw_lu, lw_ev), 1), stream));
     const unsigned blocks = (unsigned)((nn + 255) / 256);
 
     static const bool trace = getenv("PIPSORT_TRACE_PREP") != nullptr;
@@ -282,9 +271,8 @@ inline int prep_study_device(cudaStream_t stream, int n, double* dA, const doubl
     static const int chol_min = [] { const char* v = getenv("PIPSORT_PREP_CHOL_MIN"); return v ? atoi(v) : 1024; }();
     bool use_chol = cs.chol && n >= chol_min;
     int lw_ch = 0;
-    int* dflag = nullptr;
     if (use_chol) {
-        PREP_CU(cudaMallocAsync(&dflag, 2 * sizeof(int), stream));
+        PREP_CU(dflag.alloc(2, stream));
         PREP_CU(cudaMemsetAsync(dflag, 0, 2 * sizeof(int), stream));
         prep_is_symmetric_kernel<<<blocks, 256, 0, stream>>>(dA, n, dflag);
         int asym = 0;
@@ -296,7 +284,6 @@ inline int prep_study_device(cudaStream_t stream, int n, double* dA, const doubl
             if (lw_ch > std::max(std::max(lw_lu, lw_ev), 1)) use_chol = false;   // (never: potrf needs less than getrf / syevd)
         }
     }
-    auto cleanup2 = [&]() { if (dflag) cudaFreeAsync(dflag, stream); };
     for (;;) {
         bool certified = false;
         if (use_chol) {                             // can this shift be shown to fail without its LU?
@@ -329,7 +316,7 @@ inline int prep_study_device(cudaStream_t stream, int n, double* dA, const doubl
         }
         iters++;
         addDiag += 0.01;                        // accumulated exactly like util.cpp:219
-        if (iters > 100000) { *why = "the LD matrix never reached a positive determinant"; cleanup2(); cleanup(); return -3; }
+        if (iters > 100000) { *why = "the LD matrix never reached a positive determinant"; return -3; }
     }
     const auto t_psd = tnow();
     if (trace) fprintf(stderr, "[prep] PSD loop: %d shifts (%d LU factorizations, %d Cholesky certificates) %.1f ms (shift %.2f)\n", iters,
@@ -357,8 +344,6 @@ inline int prep_study_device(cudaStream_t stream, int n, double* dA, const doubl
             PREP_CU(cudaStreamSynchronize(stream));
             if (trace) fprintf(stderr, "[prep] positive definite: K by Cholesky solve %.1f ms\n", tms(t_psd, tnow()));
             res->add_diag = addDiag; res->K = Kc; res->min_abs_eig = 0.0; res->n_negative = 0; res->psd_iterations = iters;
-            cleanup2();
-            cleanup();
             return 0;
         }
         PREP_CU(cudaMemcpyAsync(dW, dA, nn * sizeof(double), cudaMemcpyDeviceToDevice, stream));   // not definite: the eigen path
@@ -374,18 +359,16 @@ inline int prep_study_device(cudaStream_t stream, int n, double* dA, const doubl
     PREP_CU(cudaMemcpyAsync(sc, dscal, sizeof sc, cudaMemcpyDeviceToHost, stream));
     PREP_CU(cudaStreamSynchronize(stream));
     if (trace) fprintf(stderr, "[prep] eigen-decomposition + K: %.1f ms\n", tms(t_psd, tnow()));
-    if (info != 0) { *why = "cusolverDnDsyevd did not converge (info " + std::to_string(info) + ")"; cleanup(); return -2; }
+    if (info != 0) { *why = "cusolverDnDsyevd did not converge (info " + std::to_string(info) + ")"; return -2; }
     if (sc[2] > 0) {
         prep_abs_fix_kernel<<<blocks, 256, 0, stream>>>(dA, dW, dev, n);
         *launches += 1;
     }
     PREP_CU(cudaGetLastError());
     res->add_diag = addDiag; res->K = sc[0]; res->min_abs_eig = sc[1]; res->n_negative = (int)sc[2]; res->psd_iterations = iters;
-    cleanup2();
-    cleanup();
 #undef PREP_CU
 #undef PREP_CS
-    return rc;
+    return 0;
 }
 
 }  // namespace pipsort
