@@ -87,7 +87,8 @@ struct LocusDev {
     double null_l;                        // -K/2 - 1 + U log(1-gamma)   (postcal.cpp:797-803)
     double cx;                            // -K/2 + U log(1-gamma): what the prior-weighted sums leave out
     double rho;                           // pi'(j, a+1) / pi'(j, a) = p / ((1-p)/2)   (1 when p == 0: postcal.cpp:27)
-    int lane_ok;                          // the prior factorises with a finite rho (p < 1): score_lane.cuh may be used
+    int lane_ok;                          // the prior factorises with a finite rho (p < 1) and every value score_lane.cuh
+                                          // forms fits a double (engine.cu lane_peak_bits): that kernel may be used
     const uint32_t* exptab[KMAX + 1];     // exptab[k][e] = m0 | m1 << 8 | a << 16 for expansion e of a k-subset
     // x tiles of the exhaustive kernel (exh_plan.h, ExhTiles): lane l of tile t is x = tile_lo[t] + l, valid when
     // x >= tile_vmin[t]; tile_of[x] = the tile of x.  Tiles never straddle a boundary between SNP types.

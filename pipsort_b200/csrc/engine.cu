@@ -766,6 +766,27 @@ static int prior_tables(double gam, double p, int U, int kb, double (*pi)[KMAX +
     return 0;
 }
 
+// log2 of the largest value score_lane.cuh can form under the prior (pi'(k,0) tables, rho = p / ((1-p)/2) finite and
+// non-zero), plus 2 LANE_KMAX bits for its sums.  For a row of k SNPs in a warp-step of K >= k SNPs it forms the weights
+// w0[j] = pi'(k,0) rho^(j-K) and w1[j] = rho^j (j = 0..K), multiplies them by a table entry (1 for the empty mask, below
+// 2^450 for any other) and forms the terms pi'(k,0) rho^a E_0 E_1 (0 <= a <= k) of the expansions.  Its factorised sum
+// meets w0[1] E = pi'(k,0) rho^(1-K) E even where every term of the expansions is small: at p = 2e-39 and gamma =
+// 0.99999 that is inf for E near 2^450 although rho^8 is a normal double.
+static double lane_peak_bits(const double (*pi)[KMAX + 1], double rho) {
+    const double lr = std::log2(rho), fast = std::log2(FAST_LIMIT);
+    double peak = -INFINITY;
+    for (int K = 1; K <= LANE_KMAX; K++)
+        for (int k = 1; k <= K; k++) {
+            const double lp = std::log2(pi[k][0]);
+            for (int j = 0; j <= K; j++) {
+                const double e = j > 0 ? fast : 0.0;
+                peak = std::max(peak, std::max(lp + (j - K) * lr, j * lr) + e);
+            }
+            for (int a = 0; a <= k; a++) peak = std::max(peak, lp + a * lr + 2.0 * fast);
+        }
+    return peak + 2 * LANE_KMAX;
+}
+
 // One prior of a grid read as the finalize kernel takes it (PRIOR_STRIDE doubles)
 static int grid_prior(const pipsort_engine* e, double gam, double p, double* out) {
     double pi[KMAX + 1][KMAX + 1];
@@ -1022,7 +1043,7 @@ static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pips
     L.rho = p == 0.0 ? 1.0 : p / ((1.0 - p) * 0.5);
     {
         const double r8 = std::pow(L.rho, KMAX);
-        L.lane_ok = p < 1.0 && std::isfinite(r8) && r8 > 0.0 && std::isfinite(1.0 / r8);
+        L.lane_ok = p < 1.0 && std::isfinite(r8) && r8 > 0.0 && std::isfinite(1.0 / r8) && lane_peak_bits(L.pi, L.rho) < 1000.0;
     }
 
     // ---- expansion tables: digit i of e = state of SNP i (0: study 0 only, 1: study 1 only, 2: both) ---
@@ -1382,8 +1403,9 @@ int pipsort_score_given_configs_device(pipsort_engine* e, const int16_t* d_confi
 
 // ---- stochastic shotgun search -----------------------------------------------------------------------------
 // first round whose running total is consulted by the convergence rule (sss_postcal.cpp:265-270: "iter >= 100" compares the
-// totals after rounds 99 and 100).  The reference's value unless PIPSORT_SSS_CONV_FROM overrides it: the search of every
-// locus we have seen ends long before round 100, so the tests lower the threshold to exercise that path.
+// totals after rounds 99 and 100).  The reference's value unless PIPSORT_SSS_CONV_FROM overrides it: a search on a locus
+// with a few strong SNPs ends long before round 100, so tests lower the threshold to exercise the rule on such loci (on
+// loci with nearly flat likelihoods the search reaches round 100 by itself, tests/search_loci.py).
 static int sss_conv_from() {
     const char* v = getenv("PIPSORT_SSS_CONV_FROM");
     return v ? std::max(0, atoi(v)) : 99;
@@ -1434,6 +1456,10 @@ static int sss_run(pipsort_engine* e, int c, int max_iterations, int32_t* iterat
     if (c < 0 || c > e->kb) return fail(PIPSORT_E_ARG, "max_causal=%d outside [0,%d] (max_causal given at create)", c, e->kb);
     if (U > SSS_MAX_U) return fail(PIPSORT_E_RANGE, "the search state packs union indices into 15 bits: U=%d > %d", U, SSS_MAX_U);
     if (max_iterations < 0) return fail(PIPSORT_E_ARG, "negative iteration count");
+    // at p = 1 every non-empty configuration has an expansion of prior 0, so its largest-|l| value is -inf: the draws
+    // would weigh a group by nan (the reference then reads past its neighbourhood list)
+    if (c > 0 && e->p == 1.0)
+        return fail(PIPSORT_E_ARG, "the shotgun search is undefined at sharing_param = 1 (every neighbour scores -inf)");
     CU(cudaSetDevice(e->device));
     pipsort_engine::Sss& q = e->sss;
     const int kmax = std::max(c, 1);

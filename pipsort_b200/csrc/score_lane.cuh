@@ -25,7 +25,8 @@
 //
 // Numeric range: everything above is ordinary doubles, valid while every E_s(mask) < 2^450 (DESIGN.md "range").  A
 // configuration that meets a larger value is handed to the mantissa/exponent code of score.cuh (whole warp, rare).
-// Loci with p == 1 (rho infinite) and batches with more than LANE_KMAX SNPs per configuration use score.cuh throughout.
+// Loci with p == 1 (rho infinite), priors under which the weights below leave the double range (engine.cu lane_peak_bits)
+// and batches with more than LANE_KMAX SNPs per configuration use score.cuh throughout.
 #pragma once
 #include "exhaustive_dev.cuh"
 #include "score.cuh"

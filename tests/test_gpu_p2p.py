@@ -169,8 +169,8 @@ def _sss_worker(rank, world, initfile, outdir):
             assert iters == 9 and why == 1
             if rank == 0:
                 assert_results_match(r, want)
-            # ... and with the convergence rule switched on from round 2 (the reference starts at round 100, which no search
-            # we know reaches): the running total every rank consults is the sum over ALL ranks' partial accumulators, so
+            # ... and with the convergence rule switched on from round 2 (the reference starts at round 100, which this search
+            # never reaches): the running total every rank consults is the sum over ALL ranks' partial accumulators, so
             # the split search must stop in the same round with the same accumulators as the search on one GPU
             os.environ["PIPSORT_SSS_CONV_FROM"] = "2"
             try:

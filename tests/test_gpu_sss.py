@@ -46,7 +46,8 @@ def test_sss_synthetic_matches_oracle_trajectory():
 
 def test_sss_convergence_rule_reads_the_running_total():
     """The convergence rule (sss_postcal.cpp:265-270) compares the running totals after consecutive rounds.  The reference
-    starts it at round 100, which no search we know reaches; PIPSORT_SSS_CONV_FROM=2 starts it at round 2.  On 12+12 SNPs
+    starts it at round 100, which a search on this locus never reaches (test_gpu_search_range.py runs searches that stop
+    there); PIPSORT_SSS_CONV_FROM=2 starts it at round 2.  On 12+12 SNPs
     (c = 3, 9 rounds to the break condition) the totals the engine reports after k = 1..9 rounds predict the round at which
     the rule stops the search."""
     from pipsort_b200 import synth
