@@ -214,7 +214,8 @@ int pipsort_posterior_exhaustive(const pipsort_locus* locus, int device, uint32_
  * store keeps one unweighted sum per (SNP, J, state, a') and per (J, a) and the weights are applied here: one finalize launch
  * over all priors and one device-to-host copy.  Every prior is validated as pipsort_create does (gamma in (0,1), p in [0,1]);
  * n_priors >= 1.  The store may be the sum of several engines' (pipsort_merge, an all-reduce of pipsort_accumulator_buffer,
- * pipsort_p2p_reduce_to_root).                                                                      */
+ * pipsort_p2p_reduce_to_root).  When every block leaves postValues, sharedPips, sharedLL and notSharedLL NULL, only total and
+ * noCausal are formed and copied back (an evidence read: the same values, bit for bit, at a fraction of the cost).       */
 int pipsort_read_prior_grid(pipsort_engine* e, int n_priors, const double* gamma, const double* sharing_param,
                             const pipsort_outputs* outs, uint64_t* n_configs);
 
@@ -229,6 +230,19 @@ int pipsort_posterior_exhaustive_grid(const pipsort_locus* locus, int device, ui
  * the current ones.  loci[i] -> outs[i] (and n_configs[i], optional).  Stops at the first error.                    */
 int pipsort_posterior_exhaustive_batch(const pipsort_locus* loci, int32_t n_loci, int device, uint32_t flags, int c,
                                        const pipsort_outputs* outs, uint64_t* n_configs);
+
+/* A grid of priors for a list of loci: pipsort_posterior_exhaustive_grid for every locus, pipelined as
+ * pipsort_posterior_exhaustive_batch pipelines the ordinary pass (same flags; PIPSORT_PRIOR_CLASSES is implied).  Locus i and
+ * prior j go to outs[i * n_priors + j], n_configs[i] (optional) receives locus i's configuration count.  Every prior is
+ * validated once, before any device work (gamma in (0,1), p in [0,1], n_priors >= 1; PIPSORT_E_ARG names a bad prior); each
+ * locus's own gamma / sharing_param is validated as pipsort_create does but not reported.  n_loci == 0 returns 0.  Any
+ * member of an output block may be NULL.  When a locus's blocks leave postValues, sharedPips, sharedLL and notSharedLL all
+ * NULL, its read is an evidence read: the finalize forms total and noCausal only and copies back 3 doubles per prior --
+ * the values the full read gives, bit for bit (the scan over p of a sensitivity analysis needs no more; pipsort_read_prior_grid
+ * makes the same choice).  Stops at the first error, as pipsort_posterior_exhaustive_batch does.                      */
+int pipsort_posterior_exhaustive_grid_batch(const pipsort_locus* loci, int32_t n_loci, int device, uint32_t flags, int c,
+                                            int n_priors, const double* gamma, const double* sharing_param,
+                                            const pipsort_outputs* outs, uint64_t* n_configs);
 
 /* The same count as it was when pipsort_read_accumulators last ran (it travels with the results: no extra device
  * round trip).                                                                                     */

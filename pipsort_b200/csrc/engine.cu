@@ -237,14 +237,16 @@ __device__ __forceinline__ void xadd_weighted(XAcc& acc, const XAcc& v, double w
 // pri[i * PRIOR_STRIDE ..] (PRIOR_STRIDE above) and its results go to res[i * (3 + 5 U) ..] in finalize_kernel's layout; the
 // counters follow the last prior (the same for every prior).  One warp per scalar output / union SNP: lane l reads the class
 // slots l, l + 32, .. once, then every prior costs one weighted warp sum per output.
+// evidence != 0 (launched with one block): the three scalars only, total | noCausal[0] | noCausal[1] at res[i * 3 ..], by the
+// same warps as the full read, so that their values are bit-identical to it.
 constexpr int GRID_LANE_SLOTS = (cls_nslot(KMAX) + 31) / 32;
 __global__ void __launch_bounds__(FIN_WARPS * 32) finalize_grid_kernel(AccDev acc, int U, int n_priors, const double* __restrict__ pri,
-                                                                       double cy, double* __restrict__ res, int clear) {
+                                                                       double cy, double* __restrict__ res, int clear, int evidence) {
     asm volatile("griddepcontrol.wait;" ::: "memory");
     const int lane = threadIdx.x & 31;
     const int w = blockIdx.x * FIN_WARPS + (threadIdx.x >> 5);
     const int C = acc.ccls;
-    const size_t stride = 3 + (size_t)5 * U;
+    const size_t stride = evidence ? 3 : 3 + (size_t)5 * U;
     if (blockIdx.x == 0 && threadIdx.x < NCOUNTER) {
         res[(size_t)n_priors * stride + threadIdx.x] = acc.counters[threadIdx.x];
         if (clear) acc.counters[threadIdx.x] = 0.0;
@@ -276,7 +278,7 @@ __global__ void __launch_bounds__(FIN_WARPS * 32) finalize_grid_kernel(AccDev ac
         return;
     }
     const int g = w - 3;
-    if (g >= U) return;
+    if (evidence || g >= U) return;
     XAcc v[GRID_LANE_SLOTS];
     int row[GRID_LANE_SLOTS], st[GRID_LANE_SLOTS];
     XAcc ys = xacc_empty(), yn = xacc_empty();      // likelihood-only sums: the same for every prior
@@ -497,8 +499,10 @@ struct pipsort_engine {
     bool classes = false;
     double* d_own_prior = nullptr;  // [PRIOR_STRIDE]
     double* d_grid = nullptr;       // grid read: priors | results | counters
-    size_t cap_grid = 0;
-    std::vector<double> h_grid;
+    double* h_grid = nullptr;       // its host side, pinned (a slice of the staging buffer when it fits there, else grown)
+    size_t cap_grid = 0, cap_h_grid = 0;
+    int grid_n = 0;                 // the grid read in flight: number of priors, whether it is an evidence read
+    bool grid_evidence = false;
 };
 
 namespace {
@@ -787,13 +791,23 @@ static double lane_peak_bits(const double (*pi)[KMAX + 1], double rho) {
     return peak + 2 * LANE_KMAX;
 }
 
-// One prior of a grid read as the finalize kernel takes it (PRIOR_STRIDE doubles)
-static int grid_prior(const pipsort_engine* e, double gam, double p, double* out) {
-    double pi[KMAX + 1][KMAX + 1];
-    int rc = prior_tables(gam, p, e->U, e->kb, pi, nullptr, nullptr);
-    if (rc) return rc;
-    memcpy(out, pi, sizeof pi);
-    out[PRIOR_STRIDE - 1] = -0.5 * e->K + e->U * std::log(1.0 - gam);
+// Priors of a grid read as the finalize kernel takes them (PRIOR_STRIDE doubles each), except that the last slot holds
+// log(1 - gamma): grid_cx turns it into a locus's cx.  pi' does not depend on the locus, so a list of loci builds the tables
+// once.  Every prior is validated as pipsort_create does; a bad one is named.
+static double grid_cx(const pipsort_engine* e, double log1m_gamma) { return -0.5 * e->K + e->U * log1m_gamma; }
+
+static int grid_tables(int n_priors, const double* gamma, const double* sharing_param, std::vector<double>* tab) {
+    tab->resize((size_t)n_priors * PRIOR_STRIDE);
+    for (int i = 0; i < n_priors; i++) {
+        double pi[KMAX + 1][KMAX + 1];
+        if (prior_tables(gamma[i], sharing_param[i], 0, 0, pi, nullptr, nullptr)) {
+            const std::string why = g_err;
+            return fail(PIPSORT_E_ARG, "prior %d: %s", i, why.c_str());
+        }
+        double* out = tab->data() + (size_t)i * PRIOR_STRIDE;
+        memcpy(out, pi, sizeof pi);
+        out[PRIOR_STRIDE - 1] = std::log(1.0 - gamma[i]);
+    }
     return 0;
 }
 
@@ -1104,9 +1118,11 @@ static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pips
     e->exh.pin_stage = pin_slice(e, e->exh.pin_stage_cap);
     CU(cudaMemsetAsync(acc.bins, 0, e->bins_len * sizeof(double), e->stream));
     if (e->classes) {   // the engine's own prior, as the grid finalize reads it (pipsort_finalize must not upload: graphs)
-        double own[PRIOR_STRIDE];
-        if ((rc = grid_prior(e, gam, p, own))) return rc;
-        if ((rc = dev_alloc(e, &e->d_own_prior, PRIOR_STRIDE)) || (rc = upload_small(e, e->d_own_prior, own, sizeof own))) return rc;
+        std::vector<double> own;
+        if ((rc = grid_tables(1, &gam, &p, &own))) return rc;
+        own[PRIOR_STRIDE - 1] = grid_cx(e, own[PRIOR_STRIDE - 1]);
+        if ((rc = dev_alloc(e, &e->d_own_prior, PRIOR_STRIDE)) ||
+            (rc = upload_small(e, e->d_own_prior, own.data(), PRIOR_STRIDE * sizeof(double)))) return rc;
     }
     // the caller's buffers and the local staging vectors must not be read after return: wait for the H2D copies only
     // (recorded in ev_up after the last of them); the preparation kernels and memsets keep running asynchronously.
@@ -1620,13 +1636,14 @@ static int flags_to_error(const double* c) {
     return 0;
 }
 
-// the finalize of a class-resolved store for n_priors priors (device table `pri`, PRIOR_STRIDE doubles each) into `res`
-static int finalize_grid_launch(pipsort_engine* e, int n_priors, const double* pri, double* res, bool clear) {
+// the finalize of a class-resolved store for n_priors priors (device table `pri`, PRIOR_STRIDE doubles each) into `res`;
+// evidence: the three scalars per prior only (one block)
+static int finalize_grid_launch(pipsort_engine* e, int n_priors, const double* pri, double* res, bool clear, bool evidence = false) {
     CU(cudaSetDevice(e->device));
     static const bool no_pdl = getenv("PIPSORT_NO_PDL") != nullptr;
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof cfg);
-    cfg.gridDim = dim3((e->U + 3 + FIN_WARPS - 1) / FIN_WARPS);
+    cfg.gridDim = dim3(evidence ? 1 : (e->U + 3 + FIN_WARPS - 1) / FIN_WARPS);
     cfg.blockDim = dim3(FIN_WARPS * 32);
     cfg.stream = e->stream;
     cudaLaunchAttribute at[1];
@@ -1634,7 +1651,7 @@ static int finalize_grid_launch(pipsort_engine* e, int n_priors, const double* p
     at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at;
     cfg.numAttrs = no_pdl ? 0 : 1;
-    CU(cudaLaunchKernelEx(&cfg, finalize_grid_kernel, e->L.acc, e->U, n_priors, pri, -0.5 * e->K, res, clear ? 1 : 0));
+    CU(cudaLaunchKernelEx(&cfg, finalize_grid_kernel, e->L.acc, e->U, n_priors, pri, -0.5 * e->K, res, clear ? 1 : 0, evidence ? 1 : 0));
     e->launches++;
     return 0;
 }
@@ -1746,32 +1763,74 @@ static void scatter_results(const pipsort_engine* e, const double* r, const pips
     }
 }
 
+// A grid read whose output blocks leave every per-SNP member NULL needs the three scalars per prior only: the evidence read
+static bool evidence_only(const pipsort_outputs* outs, int n) {
+    for (int i = 0; i < n; i++)
+        if (outs[i].postValues || outs[i].sharedPips || outs[i].sharedLL || outs[i].notSharedLL) return false;
+    return true;
+}
+
+// first half of a grid read (tables from grid_tables): the locus's prior tables and the results go through one pinned
+// buffer, priors | results | counters as d_grid, so that the upload, the finalize and the read-back are enqueued without
+// blocking.  The staging buffer serves it when it fits: a list of loci creates an engine per locus, and a pinned
+// allocation of its own would cost each locus a cudaMallocHost and a cudaFreeHost.
+static int grid_read_enqueue(pipsort_engine* e, int n_priors, const double* tab, bool evidence) {
+    const size_t stride = evidence ? 3 : 3 + (size_t)5 * e->U, npri = (size_t)n_priors * PRIOR_STRIDE;
+    const size_t need = npri + (size_t)n_priors * stride + NCOUNTER;
+    CU(cudaSetDevice(e->device));
+    int rc;
+    if ((rc = grow(e, &e->d_grid, &e->cap_grid, need))) return rc;
+    if (e->cap_h_grid < need) {
+        char* s = e->h_grid ? nullptr : pin_slice(e, need * sizeof(double));
+        if (s) { e->h_grid = reinterpret_cast<double*>(s); e->cap_h_grid = need; }
+        else if ((rc = grow(e, &e->h_grid, &e->cap_h_grid, need, Mem::pinned))) return rc;
+    }
+    memcpy(e->h_grid, tab, npri * sizeof(double));
+    for (int i = 0; i < n_priors; i++) {
+        double& cx = e->h_grid[(size_t)i * PRIOR_STRIDE + PRIOR_STRIDE - 1];
+        cx = grid_cx(e, cx);
+    }
+    CU(cudaMemcpyAsync(e->d_grid, e->h_grid, npri * sizeof(double), cudaMemcpyHostToDevice, e->stream));
+    if ((rc = finalize_grid_launch(e, n_priors, e->d_grid, e->d_grid + npri, false, evidence))) return rc;
+    CU(cudaMemcpyAsync(e->h_grid + npri, e->d_grid + npri, (need - npri) * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+    e->grid_n = n_priors;
+    e->grid_evidence = evidence;
+    return 0;
+}
+
+// second half: wait for the engine's stream, check the error counters, scatter prior i into outs[i]
+static int grid_read_complete(pipsort_engine* e, const pipsort_outputs* outs, uint64_t* n_configs) {
+    CU(cudaStreamSynchronize(e->stream));
+    const size_t stride = e->grid_evidence ? 3 : 3 + (size_t)5 * e->U;
+    const double* res = e->h_grid + (size_t)e->grid_n * PRIOR_STRIDE;
+    const double* counters = res + (size_t)e->grid_n * stride;
+    int rc = flags_to_error(counters);
+    if (rc) return rc;
+    e->last_read_count = (uint64_t)counters[0];
+    if (n_configs) *n_configs = e->last_read_count;
+    for (int i = 0; i < e->grid_n; i++) {
+        const double* r = res + (size_t)i * stride;
+        if (e->grid_evidence) {     // nothing per SNP to scatter
+            if (outs[i].total) *outs[i].total = r[0];
+            if (outs[i].noCausal) { outs[i].noCausal[0] = r[1]; outs[i].noCausal[1] = r[2]; }
+        } else {
+            scatter_results(e, r, &outs[i]);
+        }
+    }
+    return 0;
+}
+
 int pipsort_read_prior_grid(pipsort_engine* e, int n_priors, const double* gamma, const double* sharing_param,
                             const pipsort_outputs* outs, uint64_t* n_configs) {
     if (!e) return fail(PIPSORT_E_ARG, "null engine");
     if (!e->classes) return fail(PIPSORT_E_ARG, "the engine was not created with PIPSORT_PRIOR_CLASSES: its store holds one prior only");
     if (n_priors < 1) return fail(PIPSORT_E_ARG, "n_priors=%d must be >= 1", n_priors);
     if (!gamma || !sharing_param || !outs) return fail(PIPSORT_E_ARG, "null argument");
-    const size_t stride = 3 + (size_t)5 * e->U, npri = (size_t)n_priors * PRIOR_STRIDE;
-    const size_t need = npri + (size_t)n_priors * stride + NCOUNTER;
-    e->h_grid.resize(need);
-    for (int i = 0; i < n_priors; i++) {
-        int rc = grid_prior(e, gamma[i], sharing_param[i], e->h_grid.data() + (size_t)i * PRIOR_STRIDE);
-        if (rc) { const std::string why = g_err; return fail(rc, "prior %d: %s", i, why.c_str()); }
-    }
-    CU(cudaSetDevice(e->device));
-    int rc;
-    if ((rc = grow(e, &e->d_grid, &e->cap_grid, need))) return rc;
-    CU(cudaMemcpyAsync(e->d_grid, e->h_grid.data(), npri * sizeof(double), cudaMemcpyHostToDevice, e->stream));
-    if ((rc = finalize_grid_launch(e, n_priors, e->d_grid, e->d_grid + npri, false))) return rc;
-    CU(cudaMemcpyAsync(e->h_grid.data() + npri, e->d_grid + npri, (need - npri) * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
-    CU(cudaStreamSynchronize(e->stream));
-    const double* res = e->h_grid.data() + npri;
-    if ((rc = flags_to_error(res + (size_t)n_priors * stride))) return rc;
-    e->last_read_count = (uint64_t)res[(size_t)n_priors * stride];
-    if (n_configs) *n_configs = e->last_read_count;
-    for (int i = 0; i < n_priors; i++) scatter_results(e, res + (size_t)i * stride, &outs[i]);
-    return 0;
+    std::vector<double> tab;
+    int rc = grid_tables(n_priors, gamma, sharing_param, &tab);
+    if (!rc) rc = grid_read_enqueue(e, n_priors, tab.data(), evidence_only(outs, n_priors));
+    if (!rc) rc = grid_read_complete(e, outs, n_configs);
+    return rc;
 }
 
 int pipsort_posterior_exhaustive_grid(const pipsort_locus* locus, int device, uint32_t flags, int c, int n_priors, const double* gamma,
@@ -1821,20 +1880,27 @@ int pipsort_posterior_exhaustive(const pipsort_locus* locus, int device, uint32_
     return rc;
 }
 
+// The grid read of a list of loci (pipsort_posterior_exhaustive_grid_batch): n priors whose tables are built once
+// (grid_tables); locus i reports into outs[i * n ..].  n == 0: the ordinary read, locus i into outs[i].
+struct GridRead { int n; const double* tab; };
+
 // loci first, first + stride, first + 2 stride, ... through a software pipeline over DEPTH engines, each on its own stream:
 // while locus i is being evaluated the uploads and the preparation launches of the next one are already queued, and the
 // results of the one DEPTH before are being copied back.  Every locus still pays its own host -> device copy, kernels and
 // device -> host read; only the waiting overlaps.  `stop` is raised by the first worker that fails.
 static int batch_worker(const pipsort_locus* loci, int32_t n_loci, int first, int stride, int device, uint32_t flags, int c,
-                        const pipsort_outputs* outs, uint64_t* n_configs, std::atomic<int>* stop, std::string* err) {
+                        const GridRead& grid, const pipsort_outputs* outs, uint64_t* n_configs, std::atomic<int>* stop,
+                        std::string* err) {
     constexpr int DEPTH = 3;
     pipsort_engine* inflight[DEPTH] = {nullptr, nullptr, nullptr};
     int idx_of[DEPTH] = {-1, -1, -1};
     int rc = 0;
+    if (grid.n) flags |= PIPSORT_PRIOR_CLASSES;
     auto finish = [&](int slot) -> int {       // results of the locus in pipeline slot `slot`
         pipsort_engine*& e = inflight[slot];
-        int r = read_complete(e, &outs[idx_of[slot]]);
-        if (!r && n_configs) n_configs[idx_of[slot]] = e->last_read_count;
+        const int i = idx_of[slot];
+        int r = grid.n ? grid_read_complete(e, &outs[(size_t)i * grid.n], nullptr) : read_complete(e, &outs[i]);
+        if (!r && n_configs) n_configs[i] = e->last_read_count;
         std::string keep = g_err;
         pipsort_destroy(e);
         g_err = keep;
@@ -1854,7 +1920,7 @@ static int batch_worker(const pipsort_locus* loci, int32_t n_loci, int first, in
         uint64_t total = 0;
         rc = pipsort_total_ranks(e, c, &total);
         if (!rc) rc = pipsort_run_exhaustive(e, c, 0, total);
-        if (!rc) rc = read_enqueue(e);
+        if (!rc) rc = grid.n ? grid_read_enqueue(e, grid.n, grid.tab, evidence_only(&outs[(size_t)i * grid.n], grid.n)) : read_enqueue(e);
     }
     // drain in issue order (also after an error: every engine still in flight is destroyed)
     for (int d = 0; d < DEPTH; d++) {
@@ -1867,9 +1933,9 @@ static int batch_worker(const pipsort_locus* loci, int32_t n_loci, int first, in
     return rc;
 }
 
-int pipsort_posterior_exhaustive_batch(const pipsort_locus* loci, int32_t n_loci, int device, uint32_t flags, int c,
-                                       const pipsort_outputs* outs, uint64_t* n_configs) {
-    if (n_loci < 0 || (n_loci > 0 && (!loci || !outs))) return fail(PIPSORT_E_ARG, "bad argument");
+// the host threads of a batch (PIPSORT_BATCH_THREADS), each running batch_worker over its share of the loci
+static int batch_run(const pipsort_locus* loci, int32_t n_loci, int device, uint32_t flags, int c, const GridRead& grid,
+                     const pipsort_outputs* outs, uint64_t* n_configs) {
     // The host side of a small locus (a dozen runtime calls, ~60 us) costs as much as its evaluation on the device: long lists
     // are issued by several host threads (PIPSORT_BATCH_THREADS, default 3), each with its own pipeline over its own engines
     // and streams, loci dealt round robin.  The kernels of different loci then also overlap on the device -- a 150-SNP
@@ -1882,12 +1948,30 @@ int pipsort_posterior_exhaustive_batch(const pipsort_locus* loci, int32_t n_loci
     std::vector<int> rcs(T, 0);
     std::vector<std::thread> th;
     for (int t = 1; t < T; t++)
-        th.emplace_back([&, t] { rcs[t] = batch_worker(loci, n_loci, t, T, device, flags, c, outs, n_configs, &stop, &errs[t]); });
-    rcs[0] = batch_worker(loci, n_loci, 0, T, device, flags, c, outs, n_configs, &stop, &errs[0]);
+        th.emplace_back([&, t] { rcs[t] = batch_worker(loci, n_loci, t, T, device, flags, c, grid, outs, n_configs, &stop, &errs[t]); });
+    rcs[0] = batch_worker(loci, n_loci, 0, T, device, flags, c, grid, outs, n_configs, &stop, &errs[0]);
     for (auto& x : th) x.join();
     for (int t = 0; t < T; t++)
         if (rcs[t]) { g_err = errs[t]; return rcs[t]; }
     return 0;
+}
+
+int pipsort_posterior_exhaustive_batch(const pipsort_locus* loci, int32_t n_loci, int device, uint32_t flags, int c,
+                                       const pipsort_outputs* outs, uint64_t* n_configs) {
+    if (n_loci < 0 || (n_loci > 0 && (!loci || !outs))) return fail(PIPSORT_E_ARG, "bad argument");
+    return batch_run(loci, n_loci, device, flags, c, GridRead{0, nullptr}, outs, n_configs);
+}
+
+int pipsort_posterior_exhaustive_grid_batch(const pipsort_locus* loci, int32_t n_loci, int device, uint32_t flags, int c,
+                                            int n_priors, const double* gamma, const double* sharing_param,
+                                            const pipsort_outputs* outs, uint64_t* n_configs) {
+    if (n_loci < 0 || (n_loci > 0 && (!loci || !outs))) return fail(PIPSORT_E_ARG, "bad argument");
+    if (n_priors < 1) return fail(PIPSORT_E_ARG, "n_priors=%d must be >= 1", n_priors);
+    if (!gamma || !sharing_param) return fail(PIPSORT_E_ARG, "null argument");
+    std::vector<double> tab;
+    int rc = grid_tables(n_priors, gamma, sharing_param, &tab);
+    if (rc || !n_loci) return rc;
+    return batch_run(loci, n_loci, device, flags, c, GridRead{n_priors, tab.data()}, outs, n_configs);
 }
 
 int pipsort_last_read_config_count(const pipsort_engine* e, uint64_t* out) {

@@ -72,6 +72,9 @@ def lib():
         L.pipsort_posterior_exhaustive.argtypes = [C.POINTER(_LocusV), i32, C.c_uint32, i32, C.POINTER(_OutputsV), C.POINTER(u64)]
         L.pipsort_posterior_exhaustive_batch.argtypes = [C.POINTER(_LocusV), C.c_int32, i32, C.c_uint32, i32,
                                                          C.POINTER(_OutputsV), C.POINTER(u64)]
+        L.pipsort_posterior_exhaustive_grid_batch.argtypes = [C.POINTER(_LocusV), C.c_int32, i32, C.c_uint32, i32, i32,
+                                                              C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(_OutputsV),
+                                                              C.POINTER(u64)]
         L.pipsort_destroy.argtypes = [vp]
         L.pipsort_destroy.restype = None
         L.pipsort_reset.argtypes = [vp]
@@ -304,12 +307,18 @@ class Engine:
         _check(lib().pipsort_last_read_config_count(self._h, C.byref(cnt)))
         return Results(float(total[0]), post, nc, sp, sl, nl, int(cnt.value))
 
-    def read_prior_grid(self, priors) -> list:
+    def read_prior_grid(self, priors, evidence_only=False):
         """Results for every prior (gamma, p) of `priors` from the accumulators of ONE pass (an engine created with
-        prior_classes=True): each equals what an engine created with that prior reports (pipsort_read_prior_grid)."""
+        prior_classes=True): each equals what an engine created with that prior reports (pipsort_read_prior_grid).
+        evidence_only=True: the evidence read, an ndarray [n_priors, 3] of (total, noCausal[0], noCausal[1])."""
         gam, p = _prior_arrays(priors)
-        outs, res = _grid_outputs(len(gam), self.N, self.S, self.U)
         cnt = C.c_uint64()
+        if evidence_only:
+            ev = np.zeros((len(gam), 3))
+            outs = _evidence_outputs(ev)
+            _check(lib().pipsort_read_prior_grid(self._h, len(gam), _dp(gam), _dp(p), outs, C.byref(cnt)))
+            return ev
+        outs, res = _grid_outputs(len(gam), self.N, self.S, self.U)
         _check(lib().pipsort_read_prior_grid(self._h, len(gam), _dp(gam), _dp(p), outs, C.byref(cnt)))
         return res(int(cnt.value))
 
@@ -470,6 +479,16 @@ def _grid_outputs(n, N, S, U):
     return outs, results
 
 
+def _evidence_outputs(ev):
+    """pipsort_outputs over the rows of ev [k, 3] (total, noCausal[0], noCausal[1]); every per-SNP member NULL."""
+    ev = ev.reshape(-1, 3)
+    outs = (_OutputsV * max(len(ev), 1))()
+    for i in range(len(ev)):
+        b0 = ev[i].ctypes.data
+        outs[i] = _OutputsV(b0, None, b0 + 8, None, None, None)
+    return outs
+
+
 def posterior_exhaustive_grid(num_snps, sigma, z, d, K, snp_map, c, priors, device=0, raw_ld=False):
     """One locus, a grid of priors (gamma, p), one exhaustive pass (pipsort_posterior_exhaustive_grid): a list of Results,
     one per prior, each what posterior_exhaustive with that prior returns."""
@@ -514,9 +533,14 @@ class LocusBatch:
     structs (numpy structured arrays filled column by column) that point into the caller's host arrays, and ONE result
     buffer for all loci.  run() is the C-ABI call and nothing else; results() slices the buffer into Results.
     loci: sequence of dicts with the keys of posterior_exhaustive's arguments (num_snps, sigma, z, d, K, snp_map and
-    optionally gamma, sharing_param); sigma / z flat float64 arrays (studies concatenated)."""
+    optionally gamma, sharing_param); sigma / z flat float64 arrays (studies concatenated).
+    priors: a list of (gamma, p) -- run() is then pipsort_posterior_exhaustive_grid_batch, one result block per locus and
+    prior (results() gives a list of Results per locus); evidence_only=True leaves every per-SNP member NULL (the evidence
+    read) and the buffer holds (total, noCausal[0], noCausal[1]) per locus and prior, read with evidence()."""
 
-    def __init__(self, loci, c, device=0, raw_ld=False):
+    def __init__(self, loci, c, device=0, raw_ld=False, priors=None, evidence_only=False):
+        if evidence_only and priors is None:
+            raise ValueError("evidence_only needs priors")
         n = self.n = len(loci)
         self.c, self.device, self.flags = int(c), int(device), RAW_LD if raw_ld else 0
         f64, i32 = np.dtype(np.float64), np.dtype(np.int32)
@@ -538,38 +562,73 @@ class LocusBatch:
         la["gamma"] = [Lc.get("gamma", 0.01) for Lc in loci]
         la["sharing_param"] = [Lc.get("sharing_param", 0.75) for Lc in loci]
         la["max_causal"] = self.c
-        # one result buffer: per locus total | postValues[N] | noCausal[S] | sharedPips[U] | sharedLL[U] | notSharedLL[U]
-        off = self.off = np.zeros(n + 1, dtype=np.int64)
-        np.cumsum(1 + N + S + 3 * U, out=off[1:])
-        buf = self.buf = np.empty(int(off[-1]))
-        b0 = buf.ctypes.data + 8 * off[:-1]
-        oa = self.oa = np.zeros(n, dtype=_OUT_DT)
-        oa["total"] = b0
-        oa["postValues"] = b0 + 8
-        oa["noCausal"] = b0 + 8 * (1 + N)
-        oa["sharedPips"] = b0 + 8 * (1 + N + S)
-        oa["sharedLL"] = b0 + 8 * (1 + N + S + U)
-        oa["notSharedLL"] = b0 + 8 * (1 + N + S + 2 * U)
+        self.priors = None if priors is None else _prior_arrays(priors)
+        self.evidence_only = bool(evidence_only)
+        k = self.k = 1 if priors is None else len(self.priors[0])      # result blocks per locus: locus i, prior j -> i * k + j
+        if evidence_only:
+            buf = self.buf = np.empty(n * k * 3)
+            b0 = buf.ctypes.data + 24 * np.arange(n * k, dtype=np.int64)
+            oa = self.oa = np.zeros(n * k, dtype=_OUT_DT)              # per-SNP members NULL
+            oa["total"] = b0
+            oa["noCausal"] = b0 + 8
+        else:
+            # one result buffer: per block total | postValues[N] | noCausal[S] | sharedPips[U] | sharedLL[U] | notSharedLL[U]
+            Nb, Sb, Ub = np.repeat(N, k), np.repeat(S, k), np.repeat(U, k)
+            off = self.off = np.zeros(n * k + 1, dtype=np.int64)
+            np.cumsum(1 + Nb + Sb + 3 * Ub, out=off[1:])
+            buf = self.buf = np.empty(int(off[-1]))
+            b0 = buf.ctypes.data + 8 * off[:-1]
+            oa = self.oa = np.zeros(n * k, dtype=_OUT_DT)
+            oa["total"] = b0
+            oa["postValues"] = b0 + 8
+            oa["noCausal"] = b0 + 8 * (1 + Nb)
+            oa["sharedPips"] = b0 + 8 * (1 + Nb + Sb)
+            oa["sharedLL"] = b0 + 8 * (1 + Nb + Sb + Ub)
+            oa["notSharedLL"] = b0 + 8 * (1 + Nb + Sb + 2 * Ub)
         self.cnt = np.zeros(n, dtype=np.uint64)
-        self._args = (C.cast(la.ctypes.data, C.POINTER(_LocusV)), n, self.device, self.flags, self.c,
-                      C.cast(oa.ctypes.data, C.POINTER(_OutputsV)), C.cast(self.cnt.ctypes.data, C.POINTER(C.c_uint64)))
+        lp, op = C.cast(la.ctypes.data, C.POINTER(_LocusV)), C.cast(oa.ctypes.data, C.POINTER(_OutputsV))
+        cp = C.cast(self.cnt.ctypes.data, C.POINTER(C.c_uint64))
+        if priors is None:
+            self._args = (lp, n, self.device, self.flags, self.c, op, cp)
+        else:
+            gam, p = self.priors
+            self._args = (lp, n, self.device, self.flags, self.c, k, _dp(gam), _dp(p), op, cp)
 
     def run(self):
-        """pipsort_posterior_exhaustive_batch: host buffers in, host buffers out."""
-        if self.n:
+        """pipsort_posterior_exhaustive_batch (pipsort_posterior_exhaustive_grid_batch with priors): host buffers in, host
+        buffers out."""
+        if self.priors is not None:         # the priors are validated even for an empty list
+            _check(lib().pipsort_posterior_exhaustive_grid_batch(*self._args))
+        elif self.n:
             _check(lib().pipsort_posterior_exhaustive_batch(*self._args))
         return self
 
     def results(self):
-        out, buf = [], self.buf
+        """A Results per locus; with priors, a list of Results (one per prior) per locus."""
+        if self.evidence_only:
+            raise ValueError("an evidence-only batch has no per-SNP results: use evidence()")
+        out, buf, k = [], self.buf, self.k
         offl, Nl, Sl, Ul, cl = self.off.tolist(), self.N.tolist(), self.S.tolist(), self.U.tolist(), self.cnt.tolist()
         for i in range(self.n):
-            o, Ni, Si, Ui = offl[i], Nl[i], Sl[i], Ul[i]
-            p1 = o + 1 + Ni
-            p2 = p1 + Si
-            out.append(Results(float(buf[o]), buf[o + 1:p1], buf[p1:p2], buf[p2:p2 + Ui], buf[p2 + Ui:p2 + 2 * Ui],
-                               buf[p2 + 2 * Ui:p2 + 3 * Ui], cl[i]))
+            blocks = []
+            for o in offl[i * k:(i + 1) * k]:
+                Ni, Si, Ui = Nl[i], Sl[i], Ul[i]
+                p1 = o + 1 + Ni
+                p2 = p1 + Si
+                blocks.append(Results(float(buf[o]), buf[o + 1:p1], buf[p1:p2], buf[p2:p2 + Ui], buf[p2 + Ui:p2 + 2 * Ui],
+                                      buf[p2 + 2 * Ui:p2 + 3 * Ui], cl[i]))
+            out.append(blocks if self.priors is not None else blocks[0])
         return out
+
+    def evidence(self):
+        """ndarray [n_loci, n_priors, 3] of (total, noCausal[0], noCausal[1]) (a batch with priors)."""
+        if self.priors is None:
+            raise ValueError("evidence() needs a batch with priors")
+        if self.evidence_only:
+            return self.buf.reshape(self.n, self.k, 3).copy()
+        o = self.off[:-1]
+        nc = o + 1 + np.repeat(self.N, self.k)
+        return np.stack([self.buf[o], self.buf[nc], self.buf[nc + 1]], axis=-1).reshape(self.n, self.k, 3)
 
 
 def posterior_exhaustive_batch(loci, c, device=0, raw_ld=False):
@@ -577,6 +636,14 @@ def posterior_exhaustive_batch(loci, c, device=0, raw_ld=False):
     the uploads / preparation of the next locus and the read-back of the previous one overlap the current evaluation.
     Returns a list of Results.  (LocusBatch separates building the argument block from the call itself.)"""
     return LocusBatch(loci, c, device, raw_ld).run().results()
+
+
+def posterior_exhaustive_grid_batch(loci, c, priors, device=0, raw_ld=False, evidence_only=False):
+    """A grid of priors (gamma, p) for a list of loci in one call (pipsort_posterior_exhaustive_grid_batch): one exhaustive
+    pass per locus, pipelined as posterior_exhaustive_batch.  Returns a list (per locus) of lists (per prior) of Results,
+    or with evidence_only=True the ndarray [n_loci, n_priors, 3] of (total, noCausal[0], noCausal[1])."""
+    B = LocusBatch(loci, c, device, raw_ld, priors=priors, evidence_only=evidence_only).run()
+    return B.evidence() if evidence_only else B.results()
 
 
 def preprocess_study(ld, z, device=0):
