@@ -201,8 +201,8 @@ int pipsort_config_count(pipsort_engine* e, uint64_t* out);
 
 /* One locus, one call: what Model::run does with a fresh PostCal (model.h:265-276: new PostCal, findOptimalSetGreedy ->
  * computeTotalLikelihood, read the result members) -- pipsort_create + pipsort_run_exhaustive over the whole rank space +
- * pipsort_read_accumulators + pipsort_destroy.  Host buffers in (locus), host buffers out (out); n_configs (optional)
- * receives the reference's mycount.                                                                    */
+ * pipsort_read_accumulators + pipsort_destroy, as pipsort_posterior_exhaustive_batch runs them for a list of one locus.
+ * Host buffers in (locus), host buffers out (out); n_configs (optional) receives the reference's mycount.        */
 int pipsort_posterior_exhaustive(const pipsort_locus* locus, int device, uint32_t flags, int c, const pipsort_outputs* out,
                                  uint64_t* n_configs);
 
@@ -220,7 +220,9 @@ int pipsort_read_prior_grid(pipsort_engine* e, int n_priors, const double* gamma
                             const pipsort_outputs* outs, uint64_t* n_configs);
 
 /* One locus, a grid of priors, one call: pipsort_create (flags | PIPSORT_PRIOR_CLASSES) + pipsort_run_exhaustive over the whole
- * rank space + pipsort_read_prior_grid + pipsort_destroy.  The locus's own gamma / sharing_param are validated but not reported. */
+ * rank space + pipsort_read_prior_grid + pipsort_destroy, as pipsort_posterior_exhaustive_grid_batch runs them for a list of one
+ * locus: every prior is validated before any device work.  The locus's own gamma / sharing_param are validated but not
+ * reported. */
 int pipsort_posterior_exhaustive_grid(const pipsort_locus* locus, int device, uint32_t flags, int c, int n_priors, const double* gamma,
                                       const double* sharing_param, const pipsort_outputs* outs, uint64_t* n_configs);
 

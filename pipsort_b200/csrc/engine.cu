@@ -15,6 +15,7 @@
 #include <random>
 #include <string>
 #include <thread>
+#include <utility>
 #include <vector>
 
 #include "../../include/pipsort_b200.h"
@@ -168,11 +169,57 @@ __device__ inline XAcc bins_from_lanes(double v, int bias) {
 //      postValues study 0, postValues study 1, sharedPips, sharedLL, notSharedLL
 // One warp per union SNP (plus one warp per scalar).
 constexpr int FIN_WARPS = 8;
+
+// the five results of union SNP g from its accumulators x[X1 .. YN]: five logarithms, one lane each
+__device__ __forceinline__ void snp_results(const XAcc (&x)[5], int U, int g, int lane, double cx, double cy, double* __restrict__ res) {
+    if (lane >= 5) return;
+    XAcc p0 = x[X1], p1 = x[X2];
+    xmerge(p0, x[X3]);
+    xmerge(p1, x[X3]);
+    const XAcc mine = lane == 0 ? p0 : (lane == 1 ? p1 : (lane == 2 ? x[X3] : (lane == 3 ? x[YS] : x[YN])));
+    res[3 + (size_t)lane * U + g] = xlog_or_zero(mine, lane < 3 ? cx : cy);
+}
+
+// The finalize of the five-slot store with at most 32 bins: the counters row, the scalar warps and the per-SNP warps, lane b
+// reading bin b.  take(idx) returns element idx of the store (the counters in its tail) and leaves it zero when the read
+// clears.  Every thread returns to the caller, whose epilogue may have a barrier.
+template <class Take>
+__device__ __forceinline__ void finalize_lanes(const AccDev& acc, int U, double cx, double cy, double* __restrict__ res, Take take) {
+    const int lane = threadIdx.x & 31;
+    const int w = blockIdx.x * FIN_WARPS + (threadIdx.x >> 5);
+    if (blockIdx.x == 0 && threadIdx.x < NCOUNTER)
+        res[3 + (size_t)5 * U + threadIdx.x] = take((size_t)(acc.counters - acc.bins) + threadIdx.x);
+    if (w < 3) {
+        const double v = lane < acc.NB ? take(((size_t)SCAL * acc.NB + lane) * acc.Upad + w) : 0.0;
+        const XAcc x = bins_from_lanes(v, acc.bias);
+        if (lane == 0) res[w] = xlog_or_zero(x, cx);
+        return;
+    }
+    const int g = w - 3;
+    if (g >= U) return;
+    double v[5];
+#pragma unroll
+    for (int k = 0; k < 5; k++) v[k] = lane < acc.NB ? take(((size_t)k * acc.NB + lane) * acc.Upad + g) : 0.0;   // X1 .. YN
+    XAcc x[5];
+#pragma unroll
+    for (int k = 0; k < 5; k++) x[k] = bins_from_lanes(v[k], acc.bias);
+    snp_results(x, U, g, lane, cx, cy, res);
+}
+
 __global__ void __launch_bounds__(FIN_WARPS * 32) finalize_kernel(AccDev acc, int U, double cx, double cy, double* __restrict__ res,
                                                                   int clear) {
     // launched with programmatic stream serialization: the blocks may become resident while the kernel before them in
     // the stream is still draining; nothing of the accumulator store is touched before that kernel has completed
     asm volatile("griddepcontrol.wait;" ::: "memory");
+    if (acc.NB <= 32) {
+        finalize_lanes(acc, U, cx, cy, res, [&](size_t idx) {
+            const double v = acc.bins[idx];
+            if (clear && v != 0.0) acc.bins[idx] = 0.0;
+            return v;
+        });
+        return;
+    }
+    // more bins than lanes: every warp scans its accumulators
     const int lane = threadIdx.x & 31;
     const int w = blockIdx.x * FIN_WARPS + (threadIdx.x >> 5);
     if (blockIdx.x == 0 && threadIdx.x < NCOUNTER) {
@@ -186,29 +233,10 @@ __global__ void __launch_bounds__(FIN_WARPS * 32) finalize_kernel(AccDev acc, in
     }
     const int g = w - 3;
     if (g >= U) return;
-    XAcc x1, x2, x3, ys, yn;
-    if (acc.NB <= 32) {
-        double v[5];
+    XAcc x[5];
 #pragma unroll
-        for (int k = 0; k < 5; k++) {   // X1 X2 X3 YS YN
-            double* q = bin_ptr(acc, k, g) + (size_t)lane * acc.Upad;
-            v[k] = lane < acc.NB ? *q : 0.0;
-            if (clear && lane < acc.NB && v[k] != 0.0) *q = 0.0;
-        }
-        x1 = bins_from_lanes(v[X1], acc.bias); x2 = bins_from_lanes(v[X2], acc.bias); x3 = bins_from_lanes(v[X3], acc.bias);
-        ys = bins_from_lanes(v[YS], acc.bias); yn = bins_from_lanes(v[YN], acc.bias);
-    } else {
-        x1 = bins_read_warp(acc, X1, g, lane, clear != 0); x2 = bins_read_warp(acc, X2, g, lane, clear != 0);
-        x3 = bins_read_warp(acc, X3, g, lane, clear != 0);
-        ys = bins_read_warp(acc, YS, g, lane, clear != 0); yn = bins_read_warp(acc, YN, g, lane, clear != 0);
-    }
-    if (lane >= 5) return;
-    XAcc p0 = x1, p1 = x2;
-    xmerge(p0, x3);
-    xmerge(p1, x3);
-    // five logarithms: one lane each
-    const XAcc mine = lane == 0 ? p0 : (lane == 1 ? p1 : (lane == 2 ? x3 : (lane == 3 ? ys : yn)));
-    res[3 + (size_t)lane * U + g] = xlog_or_zero(mine, lane < 3 ? cx : cy);
+    for (int k = 0; k < 5; k++) x[k] = bins_read_warp(acc, k, g, lane, clear != 0);
+    snp_results(x, U, g, lane, cx, cy, res);
 }
 
 // Layout of one prior of the grid read: pi'(J,a) as a (KMAX+1) x (KMAX+1) table (row J), then cx = -K/2 + U log(1-gamma).
@@ -327,87 +355,22 @@ __global__ void __launch_bounds__(FIN_WARPS * 32) finalize_grid_kernel(AccDev ac
     }
 }
 
-// The root's half of the multi-GPU combine step fused with the finalize (accumulators of at most 32 bins): lane b of the warp
-// of a SNP takes bin b of the SNP's five accumulators from the root's own store AND from every peer's mailbox slot (polling
-// each element until it carries this epoch's flag, p2p.cuh), so the sum over the GPUs never goes back to memory; the root's
-// store is left empty.  The last block posts `consumed` to the peers.  Replaces p2p_merge_kernel + finalize_kernel.
+// The root's half of the multi-GPU combine step fused with the finalize (accumulators of at most 32 bins): every element the
+// finalize reads is the root's own, summed with every peer's mailbox copy (p2p_gather), so the sum over the GPUs never goes
+// back to memory; the root's store is left empty.  Replaces p2p_merge_kernel + finalize_kernel.
 __global__ void __launch_bounds__(FIN_WARPS * 32)
 finalize_merge_kernel(AccDev acc, int U, double cx, double cy, double* __restrict__ res, const ulonglong2* slots, size_t slot_stride,
-                      size_t bins_len, u64* __restrict__ my_ctrl, P2PPeers peers, int my_rank, unsigned* __restrict__ done,
-                      double* __restrict__ err_flag) {
+                      u64* __restrict__ my_ctrl, P2PPeers peers, int my_rank, unsigned* __restrict__ done, double* __restrict__ err_flag) {
     asm volatile("griddepcontrol.wait;" ::: "memory");
-    const u64 epoch = *(volatile u64*)(my_ctrl + 2) + 1;           // stable until the last block bumps it below
+    const u64 epoch = *(volatile u64*)(my_ctrl + 2) + 1;           // stable until the last block bumps it in p2p_root_done
     const u64 flag = epoch & 0xffffffffull;
-    const int lane = threadIdx.x & 31;
-    const int w = blockIdx.x * FIN_WARPS + (threadIdx.x >> 5);
     bool ok = true;
-    auto take = [&](size_t idx) -> double {                        // element idx of the store, summed over all GPUs; own copy cleared
-        double v = acc.bins[idx];
+    finalize_lanes(acc, U, cx, cy, res, [&](size_t idx) {
+        const double v = acc.bins[idx];
         if (v != 0.0) acc.bins[idx] = 0.0;
-        if (peers.world <= 8) {
-            // all peers' copies are requested at once (one round trip, not one per peer: with 7 peers the serial polls were
-            // most of the step at N = 8), re-requested until each carries this epoch's flag, then added in rank order
-            ulonglong2 wr[8];
-            unsigned pend = 0;
-#pragma unroll
-            for (int r = 0; r < 8; r++)
-                if (r < peers.world && r != my_rank) {
-                    wr[r] = p2p_load(slots + (size_t)r * slot_stride + idx);
-                    pend |= 1u << r;
-                }
-            const long long t0 = clock64();
-            for (;;) {
-#pragma unroll
-                for (int r = 0; r < 8; r++)
-                    if ((pend >> r & 1) && p2p_arrived(wr[r], flag)) pend &= ~(1u << r);
-                if (!pend) break;
-                if (clock64() - t0 > P2P_SPIN_CYCLES) { ok = false; break; }
-                __nanosleep(32);
-#pragma unroll
-                for (int r = 0; r < 8; r++)
-                    if (pend >> r & 1) wr[r] = p2p_load(slots + (size_t)r * slot_stride + idx);
-            }
-#pragma unroll
-            for (int r = 0; r < 8; r++)
-                if (r < peers.world && r != my_rank) v += p2p_decode(wr[r]);
-            return v;
-        }
-        for (int r = 0; r < peers.world; r++)
-            if (r != my_rank) v += p2p_take(slots + (size_t)r * slot_stride + idx, flag, ok);
-        return v;
-    };
-    if (blockIdx.x == 0 && threadIdx.x < NCOUNTER) res[3 + (size_t)5 * U + threadIdx.x] = take(bins_len - NCOUNTER + threadIdx.x);
-    if (w < 3) {
-        const double v = lane < acc.NB ? take(((size_t)SCAL * acc.NB + lane) * acc.Upad + w) : 0.0;
-        const XAcc x = bins_from_lanes(v, acc.bias);
-        if (lane == 0) res[w] = xlog_or_zero(x, cx);
-    } else if (w - 3 < U) {
-        const int g = w - 3;
-        double v[5];
-#pragma unroll
-        for (int k = 0; k < 5; k++) v[k] = lane < acc.NB ? take(((size_t)k * acc.NB + lane) * acc.Upad + g) : 0.0;
-        const XAcc x1 = bins_from_lanes(v[X1], acc.bias), x2 = bins_from_lanes(v[X2], acc.bias), x3 = bins_from_lanes(v[X3], acc.bias);
-        const XAcc ys = bins_from_lanes(v[YS], acc.bias), yn = bins_from_lanes(v[YN], acc.bias);
-        if (lane < 5) {
-            XAcc p0 = x1, p1 = x2;
-            xmerge(p0, x3);
-            xmerge(p1, x3);
-            const XAcc mine = lane == 0 ? p0 : (lane == 1 ? p1 : (lane == 2 ? x3 : (lane == 3 ? ys : yn)));
-            res[3 + (size_t)lane * U + g] = xlog_or_zero(mine, lane < 3 ? cx : cy);
-        }
-    }
-    if (!ok) atomicAdd(err_flag, 1.0);
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        const unsigned d = atomicAdd(done, 1u);
-        if (d == gridDim.x - 1) {                    // every block has read the slots: the peers may overwrite them
-            *done = 0;
-            my_ctrl[2] = epoch;
-            __threadfence_system();
-            for (int r = 0; r < peers.world; r++)
-                if (r != my_rank) *(volatile u64*)(peers.ctrl[r] + 1) = epoch;
-        }
-    }
+        return p2p_gather(v, slots, slot_stride, idx, peers, my_rank, flag, ok);
+    });
+    p2p_root_done(ok, epoch, my_ctrl, peers, my_rank, done, err_flag);
 }
 
 __global__ void add_bins_kernel(double* __restrict__ dst, const double* __restrict__ src, size_t n) {
@@ -501,8 +464,11 @@ struct pipsort_engine {
     double* d_grid = nullptr;       // grid read: priors | results | counters
     double* h_grid = nullptr;       // its host side, pinned (a slice of the staging buffer when it fits there, else grown)
     size_t cap_grid = 0, cap_h_grid = 0;
-    int grid_n = 0;                 // the grid read in flight: number of priors, whether it is an evidence read
-    bool grid_evidence = false;
+    // where the read in flight lands on the host (read_back, grid_read_enqueue): read_n output blocks of read_stride doubles,
+    // each in finalize_kernel's layout, then the counters
+    const double* h_read = nullptr;
+    int read_n = 0;
+    size_t read_stride = 0;
 };
 
 namespace {
@@ -724,6 +690,29 @@ int peer_map(int device, const cudaIpcMemHandle_t& h, void** base) {
 }
 inline ulonglong2* p2p_slots(void* base) { return reinterpret_cast<ulonglong2*>(static_cast<char*>(base) + P2P_HDR_BYTES); }
 
+// Launches `kernel` on the engine's stream with programmatic stream serialization (PDL): its blocks may become resident
+// while the kernel before it is still draining, and wait for it with griddepcontrol.wait.  PIPSORT_NO_PDL=1: plain launches.
+template <class... P, class... A>
+int launch_pdl(pipsort_engine* e, void (*kernel)(P...), unsigned blocks, unsigned threads, A&&... args) {
+    static const bool no_pdl = getenv("PIPSORT_NO_PDL") != nullptr;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg;
+    memset(&cfg, 0, sizeof cfg);
+    cfg.gridDim = dim3(blocks);
+    cfg.blockDim = dim3(threads);
+    cfg.stream = e->stream;
+    cfg.attrs = at;
+    cfg.numAttrs = no_pdl ? 0 : 1;
+    CU(cudaLaunchKernelEx(&cfg, kernel, std::forward<A>(args)...));
+    e->launches++;
+    return 0;
+}
+
+// blocks of a finalize: one warp per scalar and per union SNP
+unsigned finalize_blocks(const pipsort_engine* e) { return (e->U + 3 + FIN_WARPS - 1) / FIN_WARPS; }
+
 }  // namespace
 
 extern "C" {
@@ -731,6 +720,7 @@ extern "C" {
 const char* pipsort_last_error(void) { return g_err.c_str(); }
 const char* pipsort_version(void) { return "pipsort_b200 0.1 (sm_100a)"; }
 
+// never sets the last error: a caller may destroy an engine after a failure without losing its message
 void pipsort_destroy(pipsort_engine* e) {
     if (!e) return;
     cudaSetDevice(e->device);
@@ -1150,7 +1140,7 @@ int pipsort_create(const pipsort_locus* lc, int device, uint32_t flags, pipsort_
     pipsort_engine* e = new pipsort_engine();
     e->defer_upload_sync = (flags & PIPSORT_INTERNAL_NO_UPLOAD_WAIT) != 0;
     int rc = create_impl(lc, device, flags, e);
-    if (rc) { std::string keep = g_err; pipsort_destroy(e); g_err = keep; return rc; }
+    if (rc) { pipsort_destroy(e); return rc; }
     *out = e;
     return 0;
 }
@@ -1491,7 +1481,6 @@ static int sss_run(pipsort_engine* e, int c, int max_iterations, int32_t* iterat
     const size_t acc_len = p2p_acc_len(e), half = p2p_sss_half(e), stride = p2p_slot_len(e);
     if (world > 1 && (size_t)n_max + (size_t)e->L.acc.NB > half) return fail(PIPSORT_E_ARG, "mailbox too small for this max_causal");
     double* errf = e->L.acc.counters + 1 + ERR_P2P_TIMEOUT;
-    const double cx = -0.5 * e->K + U * std::log(1.0 - e->gamma);     // as finalize_launch: total = log(sum) + cx
 
     const int conv_from = sss_conv_from();
     std::mt19937 gen(12345);                                             // sss_postcal.cpp:138
@@ -1534,7 +1523,8 @@ static int sss_run(pipsort_engine* e, int c, int max_iterations, int32_t* iterat
             e->launches++;
         }
         if (iter >= conv_from) {                                         // the running sum is only consulted from here on
-            sss_total_kernel<<<1, 32, 0, e->stream>>>(e->L.acc, sh, (long long)n_max, cx, q.d_total, errf);
+            // total = log(sum) + cx, as the finalize
+            sss_total_kernel<<<1, 32, 0, e->stream>>>(e->L.acc, sh, (long long)n_max, e->L.cx, q.d_total, errf);
             e->launches++;
         }
         CU(cudaGetLastError());
@@ -1640,42 +1630,16 @@ static int flags_to_error(const double* c) {
 // evidence: the three scalars per prior only (one block)
 static int finalize_grid_launch(pipsort_engine* e, int n_priors, const double* pri, double* res, bool clear, bool evidence = false) {
     CU(cudaSetDevice(e->device));
-    static const bool no_pdl = getenv("PIPSORT_NO_PDL") != nullptr;
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof cfg);
-    cfg.gridDim = dim3(evidence ? 1 : (e->U + 3 + FIN_WARPS - 1) / FIN_WARPS);
-    cfg.blockDim = dim3(FIN_WARPS * 32);
-    cfg.stream = e->stream;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = no_pdl ? 0 : 1;
-    CU(cudaLaunchKernelEx(&cfg, finalize_grid_kernel, e->L.acc, e->U, n_priors, pri, -0.5 * e->K, res, clear ? 1 : 0, evidence ? 1 : 0));
-    e->launches++;
-    return 0;
+    return launch_pdl(e, finalize_grid_kernel, evidence ? 1 : finalize_blocks(e), FIN_WARPS * 32, e->L.acc, e->U, n_priors, pri,
+                      e->L.neg_half_K, res, clear ? 1 : 0, evidence ? 1 : 0);
 }
 
 static int finalize_launch(pipsort_engine* e, bool clear) {
     // a class-resolved store reports the engine's own prior: the grid finalize for that one prior, same result layout
     if (e->classes) return finalize_grid_launch(e, 1, e->d_own_prior, e->d_res, clear);
     CU(cudaSetDevice(e->device));
-    const int U = e->U;
-    const double cy = -0.5 * e->K, cx = cy + U * std::log(1.0 - e->gamma);
-    static const bool no_pdl = getenv("PIPSORT_NO_PDL") != nullptr;
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof cfg);
-    cfg.gridDim = dim3((U + 3 + FIN_WARPS - 1) / FIN_WARPS);
-    cfg.blockDim = dim3(FIN_WARPS * 32);
-    cfg.stream = e->stream;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = no_pdl ? 0 : 1;
-    CU(cudaLaunchKernelEx(&cfg, finalize_kernel, e->L.acc, U, cx, cy, e->d_res, clear ? 1 : 0));
-    e->launches++;
-    return 0;
+    return launch_pdl(e, finalize_kernel, finalize_blocks(e), FIN_WARPS * 32, e->L.acc, e->U, e->L.cx, e->L.neg_half_K, e->d_res,
+                      clear ? 1 : 0);
 }
 
 int pipsort_finalize(pipsort_engine* e) {
@@ -1697,25 +1661,43 @@ int pipsort_last_kernel_ms(pipsort_engine* e, float* ms) {
     return 0;
 }
 
-// first half of a read: finalize kernel + device -> host copy of the results, enqueued, not waited for
-static int read_enqueue(pipsort_engine* e) {
-    int rcf = pipsort_finalize(e);
-    if (rcf) return rcf;
+// device -> host copy of the last finalize's results (d_res), enqueued, not waited for
+static int read_back(pipsort_engine* e) {
     if (!e->h_res_pin) e->h_res_pin = reinterpret_cast<double*>(pin_slice(e, e->h_res.size() * sizeof(double)));
     double* hres = e->h_res_pin ? e->h_res_pin : e->h_res.data();
     CU(cudaMemcpyAsync(hres, e->d_res, e->h_res.size() * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+    e->h_read = hres;
+    e->read_n = 1;
+    e->read_stride = 3 + (size_t)5 * e->U;
     return 0;
 }
 
-static int read_complete(pipsort_engine* e, const pipsort_outputs* out);
+// first half of a read: finalize kernel + device -> host copy of the results
+static int read_enqueue(pipsort_engine* e) {
+    int rcf = pipsort_finalize(e);
+    if (rcf) return rcf;
+    return read_back(e);
+}
+
+static void scatter_results(const pipsort_engine* e, const double* r, const pipsort_outputs* out);
+
+// second half of a read or a grid read: wait for the engine's stream, check the error counters, scatter output block i into
+// outs[i]
+static int read_complete(pipsort_engine* e, const pipsort_outputs* outs) {
+    CU(cudaStreamSynchronize(e->stream));
+    const double* counters = e->h_read + (size_t)e->read_n * e->read_stride;
+    int rc = flags_to_error(counters);
+    if (rc) return rc;
+    e->last_read_count = (uint64_t)counters[0];
+    for (int i = 0; i < e->read_n; i++) scatter_results(e, e->h_read + (size_t)i * e->read_stride, &outs[i]);
+    return 0;
+}
 
 int pipsort_fetch_results(pipsort_engine* e, const pipsort_outputs* out) {
     if (!e || !out) return fail(PIPSORT_E_ARG, "null argument");
     CU(cudaSetDevice(e->device));
-    if (!e->h_res_pin) e->h_res_pin = reinterpret_cast<double*>(pin_slice(e, e->h_res.size() * sizeof(double)));
-    double* hres = e->h_res_pin ? e->h_res_pin : e->h_res.data();
-    CU(cudaMemcpyAsync(hres, e->d_res, e->h_res.size() * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
-    return read_complete(e, out);
+    int rc = read_back(e);
+    return rc ? rc : read_complete(e, out);
 }
 
 int pipsort_read_accumulators(pipsort_engine* e, const pipsort_outputs* out) {
@@ -1725,21 +1707,8 @@ int pipsort_read_accumulators(pipsort_engine* e, const pipsort_outputs* out) {
     return read_complete(e, out);
 }
 
-static void scatter_results(const pipsort_engine* e, const double* r, const pipsort_outputs* out);
-
-// second half: wait for the engine's stream, check the error counters, scatter into the caller's arrays
-static int read_complete(pipsort_engine* e, const pipsort_outputs* out) {
-    const int U = e->U;
-    double* hres = e->h_res_pin ? e->h_res_pin : e->h_res.data();
-    CU(cudaStreamSynchronize(e->stream));
-    int rc = flags_to_error(hres + 3 + (size_t)5 * U);
-    if (rc) return rc;
-    e->last_read_count = (uint64_t)hres[3 + (size_t)5 * U];
-    scatter_results(e, hres, out);
-    return 0;
-}
-
-// results in the finalize kernel's layout (3 + 5 U, internal order) -> the caller's arrays (snp_map / study order)
+// results in the finalize kernel's layout (3 + 5 U, internal order) -> the caller's arrays (snp_map / study order).  NULL
+// members are skipped; when every per-SNP member is NULL nothing past the three scalars is read (the evidence read's blocks).
 static void scatter_results(const pipsort_engine* e, const double* r, const pipsort_outputs* out) {
     const int U = e->U;
     if (out->total) *out->total = r[0];
@@ -1793,30 +1762,9 @@ static int grid_read_enqueue(pipsort_engine* e, int n_priors, const double* tab,
     CU(cudaMemcpyAsync(e->d_grid, e->h_grid, npri * sizeof(double), cudaMemcpyHostToDevice, e->stream));
     if ((rc = finalize_grid_launch(e, n_priors, e->d_grid, e->d_grid + npri, false, evidence))) return rc;
     CU(cudaMemcpyAsync(e->h_grid + npri, e->d_grid + npri, (need - npri) * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
-    e->grid_n = n_priors;
-    e->grid_evidence = evidence;
-    return 0;
-}
-
-// second half: wait for the engine's stream, check the error counters, scatter prior i into outs[i]
-static int grid_read_complete(pipsort_engine* e, const pipsort_outputs* outs, uint64_t* n_configs) {
-    CU(cudaStreamSynchronize(e->stream));
-    const size_t stride = e->grid_evidence ? 3 : 3 + (size_t)5 * e->U;
-    const double* res = e->h_grid + (size_t)e->grid_n * PRIOR_STRIDE;
-    const double* counters = res + (size_t)e->grid_n * stride;
-    int rc = flags_to_error(counters);
-    if (rc) return rc;
-    e->last_read_count = (uint64_t)counters[0];
-    if (n_configs) *n_configs = e->last_read_count;
-    for (int i = 0; i < e->grid_n; i++) {
-        const double* r = res + (size_t)i * stride;
-        if (e->grid_evidence) {     // nothing per SNP to scatter
-            if (outs[i].total) *outs[i].total = r[0];
-            if (outs[i].noCausal) { outs[i].noCausal[0] = r[1]; outs[i].noCausal[1] = r[2]; }
-        } else {
-            scatter_results(e, r, &outs[i]);
-        }
-    }
+    e->h_read = e->h_grid + npri;
+    e->read_n = n_priors;
+    e->read_stride = stride;
     return 0;
 }
 
@@ -1829,55 +1777,25 @@ int pipsort_read_prior_grid(pipsort_engine* e, int n_priors, const double* gamma
     std::vector<double> tab;
     int rc = grid_tables(n_priors, gamma, sharing_param, &tab);
     if (!rc) rc = grid_read_enqueue(e, n_priors, tab.data(), evidence_only(outs, n_priors));
-    if (!rc) rc = grid_read_complete(e, outs, n_configs);
+    if (!rc) rc = read_complete(e, outs);
+    if (!rc && n_configs) *n_configs = e->last_read_count;
     return rc;
 }
 
+// the one-call entry points are the batch of one locus; their own checks come first, so that a null or bad argument is
+// reported as pipsort_create and pipsort_read_prior_grid would report it
 int pipsort_posterior_exhaustive_grid(const pipsort_locus* locus, int device, uint32_t flags, int c, int n_priors, const double* gamma,
                                       const double* sharing_param, const pipsort_outputs* outs, uint64_t* n_configs) {
     if (!outs) return fail(PIPSORT_E_ARG, "null argument");
     if (n_priors < 1) return fail(PIPSORT_E_ARG, "n_priors=%d must be >= 1", n_priors);
-    pipsort_engine* e = nullptr;
-    int rc = pipsort_create(locus, device, flags | PIPSORT_PRIOR_CLASSES | PIPSORT_INTERNAL_NO_UPLOAD_WAIT |
-                                               (c >= 2 ? PIPSORT_INTERNAL_WITH_PAIRS : 0u), &e);
-    if (rc) return rc;
-    uint64_t total = 0;
-    rc = pipsort_total_ranks(e, c, &total);
-    if (!rc) rc = pipsort_run_exhaustive(e, c, 0, total);
-    if (!rc) rc = pipsort_read_prior_grid(e, n_priors, gamma, sharing_param, outs, n_configs);
-    std::string keep = g_err;
-    pipsort_destroy(e);
-    g_err = keep;
-    return rc;
+    if (!locus) return fail(PIPSORT_E_ARG, "null argument");
+    return pipsort_posterior_exhaustive_grid_batch(locus, 1, device, flags, c, n_priors, gamma, sharing_param, outs, n_configs);
 }
 
 int pipsort_posterior_exhaustive(const pipsort_locus* locus, int device, uint32_t flags, int c, const pipsort_outputs* out,
                                  uint64_t* n_configs) {
-    if (!out) return fail(PIPSORT_E_ARG, "null argument");
-    static const bool trace = getenv("PIPSORT_TRACE") != nullptr;
-    auto now = [] { return std::chrono::steady_clock::now(); };
-    const auto t0 = now();
-    pipsort_engine* e = nullptr;
-    // the caller's buffers stay valid until this function returns: no need to wait for the uploads inside create
-    int rc = pipsort_create(locus, device, flags | PIPSORT_INTERNAL_NO_UPLOAD_WAIT | (c >= 2 ? PIPSORT_INTERNAL_WITH_PAIRS : 0u), &e);
-    if (rc) return rc;
-    const auto t1 = now();
-    uint64_t total = 0;
-    rc = pipsort_total_ranks(e, c, &total);
-    if (!rc) rc = pipsort_run_exhaustive(e, c, 0, total);
-    const auto t2 = now();
-    if (!rc) rc = pipsort_read_accumulators(e, out);
-    const auto t3 = now();
-    if (!rc && n_configs) *n_configs = e->last_read_count;
-    std::string keep = g_err;
-    pipsort_destroy(e);
-    g_err = keep;
-    if (trace) {
-        auto us = [](auto a, auto b) { return std::chrono::duration<double, std::micro>(b - a).count(); };
-        fprintf(stderr, "[pipsort] create %.1f us, run (enqueue) %.1f us, read (incl. device time) %.1f us, destroy %.1f us\n", us(t0, t1),
-                us(t1, t2), us(t2, t3), us(t3, now()));
-    }
-    return rc;
+    if (!locus || !out) return fail(PIPSORT_E_ARG, "null argument");
+    return pipsort_posterior_exhaustive_batch(locus, 1, device, flags, c, out, n_configs);
 }
 
 // The grid read of a list of loci (pipsort_posterior_exhaustive_grid_batch): n priors whose tables are built once
@@ -1896,14 +1814,12 @@ static int batch_worker(const pipsort_locus* loci, int32_t n_loci, int first, in
     int idx_of[DEPTH] = {-1, -1, -1};
     int rc = 0;
     if (grid.n) flags |= PIPSORT_PRIOR_CLASSES;
-    auto finish = [&](int slot) -> int {       // results of the locus in pipeline slot `slot`
+    auto finish = [&](int slot) -> int {       // results of the locus in pipeline slot `slot`: its read_n output blocks
         pipsort_engine*& e = inflight[slot];
         const int i = idx_of[slot];
-        int r = grid.n ? grid_read_complete(e, &outs[(size_t)i * grid.n], nullptr) : read_complete(e, &outs[i]);
+        int r = read_complete(e, &outs[(size_t)i * e->read_n]);
         if (!r && n_configs) n_configs[i] = e->last_read_count;
-        std::string keep = g_err;
         pipsort_destroy(e);
-        g_err = keep;
         e = nullptr;
         return r;
     };
@@ -1927,7 +1843,7 @@ static int batch_worker(const pipsort_locus* loci, int32_t n_loci, int first, in
         const int slot = (k + d) % DEPTH;
         if (!inflight[slot]) continue;
         if (!rc && !stop->load(std::memory_order_relaxed)) rc = finish(slot);
-        else { std::string keep = g_err; pipsort_destroy(inflight[slot]); g_err = keep; inflight[slot] = nullptr; }
+        else { pipsort_destroy(inflight[slot]); inflight[slot] = nullptr; }
     }
     if (rc) { stop->store(1); *err = g_err; }
     return rc;
@@ -2116,24 +2032,9 @@ int pipsort_p2p_combine_finalize(pipsort_engine* e) {
         return rc ? rc : finalize_launch(e, true);
     }
     CU(cudaSetDevice(e->device));
-    const int U = e->U;
-    const double cy = -0.5 * e->K, cx = cy + U * std::log(1.0 - e->gamma);
-    static const bool no_pdl = getenv("PIPSORT_NO_PDL") != nullptr;
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof cfg);
-    cfg.gridDim = dim3((U + 3 + FIN_WARPS - 1) / FIN_WARPS);
-    cfg.blockDim = dim3(FIN_WARPS * 32);
-    cfg.stream = e->stream;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = no_pdl ? 0 : 1;
     double* errf = e->L.acc.counters + 1 + ERR_P2P_TIMEOUT;
-    CU(cudaLaunchKernelEx(&cfg, finalize_merge_kernel, e->L.acc, U, cx, cy, e->d_res, p2p_slots(q.mailbox),
-                          p2p_slot_len(e), e->bins_len, q.peers.ctrl[q.rank], q.peers, q.rank, q.d_done, errf));
-    e->launches++;
-    return 0;
+    return launch_pdl(e, finalize_merge_kernel, finalize_blocks(e), FIN_WARPS * 32, e->L.acc, e->U, e->L.cx, e->L.neg_half_K, e->d_res,
+                      p2p_slots(q.mailbox), p2p_slot_len(e), q.peers.ctrl[q.rank], q.peers, q.rank, q.d_done, errf);
 }
 
 static int p2p_reduce_impl(pipsort_engine* e, bool clear_sender) {
@@ -2144,26 +2045,11 @@ static int p2p_reduce_impl(pipsort_engine* e, bool clear_sender) {
     const size_t n = e->bins_len, slot = p2p_slot_len(e);
     const unsigned blocks = (unsigned)std::min<size_t>((n + 511) / 512, (size_t)e->sm_count * 2);
     double* errf = e->L.acc.counters + 1 + ERR_P2P_TIMEOUT;
-    static const bool no_pdl = getenv("PIPSORT_NO_PDL") != nullptr;
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof cfg);
-    cfg.gridDim = dim3(blocks);
-    cfg.blockDim = dim3(256);
-    cfg.stream = e->stream;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = no_pdl ? 0 : 1;
-    if (q.rank != q.root) {
-        CU(cudaLaunchKernelEx(&cfg, p2p_push_kernel, e->L.acc.bins, n, p2p_slots(q.peer_base[q.root]) + (size_t)q.rank * slot,
-                              q.peers.ctrl[q.rank], q.d_done, errf, clear_sender ? 1 : 0));
-    } else {
-        CU(cudaLaunchKernelEx(&cfg, p2p_merge_kernel, e->L.acc.bins, (const ulonglong2*)p2p_slots(q.mailbox), n, slot,
-                              q.peers.ctrl[q.rank], q.peers, q.rank, q.d_done, errf));
-    }
-    e->launches++;
-    return 0;
+    if (q.rank != q.root)
+        return launch_pdl(e, p2p_push_kernel, blocks, 256, e->L.acc.bins, n, p2p_slots(q.peer_base[q.root]) + (size_t)q.rank * slot,
+                          q.peers.ctrl[q.rank], q.d_done, errf, clear_sender ? 1 : 0);
+    return launch_pdl(e, p2p_merge_kernel, blocks, 256, e->L.acc.bins, (const ulonglong2*)p2p_slots(q.mailbox), n, slot,
+                      q.peers.ctrl[q.rank], q.peers, q.rank, q.d_done, errf);
 }
 
 int pipsort_shard_ranks(const pipsort_engine* e, int c, int parts, uint64_t* bounds) {

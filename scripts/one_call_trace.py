@@ -1,4 +1,5 @@
-"""Host-side phases of the one-locus call (PIPSORT_TRACE=1 PIPSORT_TRACE_CREATE=1): python scripts/one_call_trace.py"""
+"""Host-side phases of pipsort_create inside the one-locus call (PIPSORT_TRACE_CREATE=1): python scripts/one_call_trace.py.
+The create / run / read / destroy phases of a locus are timed through the engine API by scripts/e2e_breakdown.py."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
