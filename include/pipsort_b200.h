@@ -246,6 +246,51 @@ int pipsort_posterior_exhaustive_grid_batch(const pipsort_locus* loci, int32_t n
                                             int n_priors, const double* gamma, const double* sharing_param,
                                             const pipsort_outputs* outs, uint64_t* n_configs);
 
+/* Choosing the prior by marginal likelihood (DESIGN.md section 5f).  The log evidence totalLikeLihoodLOG of a locus
+ * (postcal.cpp:1144-1163) is a closed function of the prior:
+ *   total(gamma, p) = U log(1-gamma) + log sum_{J <= c, a <= J} pi'(J, a; gamma, p) exp(table[cls_T(J, a)]),
+ *   table[J (J+1)/2 + a] = -K/2 + log T[J][a],
+ * T[J][a] the unweighted sum of E_0 E_1 over the expanded configurations of J union SNPs of which a are causal in both
+ * studies, pi' log_prior's weight (postcal.cpp:19-59) without U log(1-gamma).  pipsort_read_class_evidence copies that
+ * table out of a class-resolved store: (c+1)(c+2)/2 doubles, NOT a PostCal array -- an empty class is -inf, and 0.0 is a
+ * value a class may have.  One finalize launch (warp 0 of the grid read's evidence mode), no prior uploaded.  Only for a
+ * PIPSORT_PRIOR_CLASSES engine (PIPSORT_E_ARG otherwise); 0 <= c <= the engine's class limit (its max_causal, at least 3);
+ * the store may be the sum of several engines' (pipsort_merge, an all-reduce of pipsort_accumulator_buffer,
+ * pipsort_p2p_reduce_to_root).  n_configs (optional) receives the configuration count; a singular block or a range overflow
+ * found by the pass is reported as the other reads report it.                                                          */
+int pipsort_read_class_evidence(pipsort_engine* e, int c, double* table, uint64_t* n_configs);
+
+/* The class tables of a list of loci: pipsort_create (flags | PIPSORT_PRIOR_CLASSES) + pipsort_run_exhaustive over the whole
+ * rank space + pipsort_read_class_evidence + pipsort_destroy per locus, pipelined as pipsort_posterior_exhaustive_batch
+ * pipelines the ordinary pass (same host threads, same depth).  Locus i goes to tables[i * (c+1)(c+2)/2 ..], n_configs[i]
+ * (optional) receives its configuration count.  Each locus's gamma / sharing_param is validated as pipsort_create does but
+ * not used.  n_loci == 0 returns 0.  Stops at the first error, as pipsort_posterior_exhaustive_batch does.            */
+int pipsort_class_evidence_batch(const pipsort_locus* loci, int32_t n_loci, int device, uint32_t flags, int c, double* tables,
+                                 uint64_t* n_configs);
+
+/* The prior (gamma, p) of largest joint log evidence sum_i total_i(gamma, p) over n_loci loci, from their class tables
+ * (tables[i * (c+1)(c+2)/2 ..] as pipsort_read_class_evidence writes them, union_count[i] = U of locus i).  Pure host code:
+ * needs no device.  fit is a bit mask: 1 fits gamma, 2 fits p; a parameter whose bit is clear keeps the value passed in, and
+ * fit == 0 only evaluates.  On return *gamma / *sharing_param hold the prior, *joint_log_evidence (optional) the joint log
+ * evidence there and log_evidence[n_loci] (optional) every locus's total there.  The weights pi' are the engine's own, so
+ * that p == 0 is the reference's separate prior (the sharing term is skipped, postcal.cpp:27) and not the limit p -> 0, and
+ * p == 1 gives classes with a < J the weight 0.  Loci are treated as independent.
+ * Search (deterministic): a grid, then a local search.  A sum of per-locus terms in p need not be concave.
+ *   gamma: 64 values uniform in log-odds over [1e-8, 1 - 1e-8];
+ *   p:     128 values uniform in log-odds over [1e-12, 1 - 1e-12], and p = 1;
+ *   every pair of the grid is evaluated; from the best pair with p < 1, and from the best gamma of the p = 1 column, the
+ *   fitted coordinates are refined one at a time by Brent's method within one grid step either side (log-odds), in rounds,
+ *   until a round gains less than 1e-9 nats (at most 100 rounds).  p = 1 is returned when it is strictly better than the
+ *   refined interior point.
+ *   A fit of p never returns p = 0: the skip rule gives every class weight (gamma/(1-gamma))^J, and any p in (0, 1] gives it
+ *   that times p^a ((1-p)/2)^(J-a) <= 1 -- the three sharing states of a SNP weigh 1 each instead of summing to 1 -- so its
+ *   evidence is at least that of every p on every locus, and strictly larger once a class with J >= 1 holds anything.
+ *   With p == 0 passed in and bit 2 clear, gamma is fitted (or the evidence evaluated) under the skip rule.
+ * PIPSORT_E_ARG: n_loci < 1, c outside [0, 8], fit > 3, gamma outside (0,1) or p outside [0,1] on input, union_count < 1,
+ * a NaN or +inf in a table, or a locus whose evidence is -inf at every candidate prior (the message names the locus).  */
+int pipsort_fit_prior(int32_t n_loci, int c, const double* tables, const int32_t* union_count, uint32_t fit, double* gamma,
+                      double* sharing_param, double* joint_log_evidence, double* log_evidence);
+
 /* The same count as it was when pipsort_read_accumulators last ran (it travels with the results: no extra device
  * round trip).                                                                                     */
 int pipsort_last_read_config_count(const pipsort_engine* e, uint64_t* out);

@@ -146,8 +146,9 @@ __device__ __forceinline__ XAcc bins_decode(int top, int bias, Bin bin) {
 __host__ __device__ constexpr int cls_slot(int J, int t, int ap) { return 3 * J * (J - 1) / 2 + t * J + ap; }
 __host__ __device__ constexpr int cls_nslot(int C) { return 3 * C * (C + 1) / 2; }
 __host__ __device__ constexpr int cls_T(int J, int a) { return J * (J + 1) / 2 + a; }
-__host__ __device__ constexpr int cls_N(int C, int s, int J) { return (C + 1) * (C + 2) / 2 + s * (C + 1) + J; }
-__host__ __device__ constexpr int cls_nscal(int C) { return (C + 1) * (C + 2) / 2 + 2 * (C + 1); }
+__host__ __device__ constexpr int cls_ntab(int C) { return (C + 1) * (C + 2) / 2; }   // classes (J, a) with J <= C
+__host__ __device__ constexpr int cls_N(int C, int s, int J) { return cls_ntab(C) + s * (C + 1) + J; }
+__host__ __device__ constexpr int cls_nscal(int C) { return cls_ntab(C) + 2 * (C + 1); }
 
 // scalar k of the class-resolved store += M * 2^N
 __device__ __forceinline__ void scal_add(const AccDev& a, int k, double M, int N) {

@@ -265,22 +265,28 @@ __device__ __forceinline__ void xadd_weighted(XAcc& acc, const XAcc& v, double w
 // pri[i * PRIOR_STRIDE ..] (PRIOR_STRIDE above) and its results go to res[i * (3 + 5 U) ..] in finalize_kernel's layout; the
 // counters follow the last prior (the same for every prior).  One warp per scalar output / union SNP: lane l reads the class
 // slots l, l + 32, .. once, then every prior costs one weighted warp sum per output.
-// evidence != 0 (launched with one block): the three scalars only, total | noCausal[0] | noCausal[1] at res[i * 3 ..], by the
+// GRID_EVIDENCE (launched with one block): the three scalars only, total | noCausal[0] | noCausal[1] at res[i * 3 ..], by the
 // same warps as the full read, so that their values are bit-identical to it.
+// GRID_TABLE (one block, no priors): the class table up to the class limit tab_c <= C -- res[cls_T(J, a)] = -K/2 + log T[J][a]
+// (cy = -K/2), unweighted, -inf for an empty class (0.0 is a value a class may have) -- then the counters.  Warp 0 decodes
+// the T[J][a] slots as the evidence read does, so that the table and the evidence read cannot disagree.
+enum GridMode : int { GRID_FULL = 0, GRID_EVIDENCE = 1, GRID_TABLE = 2 };
 constexpr int GRID_LANE_SLOTS = (cls_nslot(KMAX) + 31) / 32;
 __global__ void __launch_bounds__(FIN_WARPS * 32) finalize_grid_kernel(AccDev acc, int U, int n_priors, const double* __restrict__ pri,
-                                                                       double cy, double* __restrict__ res, int clear, int evidence) {
+                                                                       double cy, double* __restrict__ res, int clear, int mode,
+                                                                       int tab_c) {
     asm volatile("griddepcontrol.wait;" ::: "memory");
     const int lane = threadIdx.x & 31;
     const int w = blockIdx.x * FIN_WARPS + (threadIdx.x >> 5);
     const int C = acc.ccls;
-    const size_t stride = evidence ? 3 : 3 + (size_t)5 * U;
+    const size_t stride = mode == GRID_FULL ? 3 + (size_t)5 * U : 3;
     if (blockIdx.x == 0 && threadIdx.x < NCOUNTER) {
-        res[(size_t)n_priors * stride + threadIdx.x] = acc.counters[threadIdx.x];
+        res[(mode == GRID_TABLE ? (size_t)cls_ntab(tab_c) : (size_t)n_priors * stride) + threadIdx.x] = acc.counters[threadIdx.x];
         if (clear) acc.counters[threadIdx.x] = 0.0;
     }
     if (w < 3) {   // total: T[J][a], weight pi'(J,a);  noCausal[s]: N_s[J], weight pi'(J,0)
-        const int n = w == 0 ? (C + 1) * (C + 2) / 2 : C + 1;
+        if (mode == GRID_TABLE && w > 0) return;
+        const int n = w == 0 ? cls_ntab(C) : C + 1;
         XAcc v[2];
         int row[2];
         for (int q = 0; q < 2; q++) {
@@ -295,6 +301,13 @@ __global__ void __launch_bounds__(FIN_WARPS * 32) finalize_grid_kernel(AccDev ac
             v[q] = bins_read_lane(acc, cls_nslot(C) + idx / acc.Upad, idx % acc.Upad, clear != 0);
             row[q] = J * (KMAX + 1) + a;
         }
+        if (mode == GRID_TABLE) {
+            for (int q = 0; q < 2; q++) {
+                const int k = lane + 32 * q;   // = cls_T(J, a)
+                if (k < cls_ntab(tab_c)) res[k] = v[q].M > 0.0 ? xlog_or_zero(v[q], cy) : -INFINITY;
+            }
+            return;
+        }
         for (int i = 0; i < n_priors; i++) {
             const double* pi = pri + (size_t)i * PRIOR_STRIDE;
             XAcc s = xacc_empty();
@@ -306,7 +319,7 @@ __global__ void __launch_bounds__(FIN_WARPS * 32) finalize_grid_kernel(AccDev ac
         return;
     }
     const int g = w - 3;
-    if (evidence || g >= U) return;
+    if (mode != GRID_FULL || g >= U) return;
     XAcc v[GRID_LANE_SLOTS];
     int row[GRID_LANE_SLOTS], st[GRID_LANE_SLOTS];
     XAcc ys = xacc_empty(), yn = xacc_empty();      // likelihood-only sums: the same for every prior
@@ -464,11 +477,13 @@ struct pipsort_engine {
     double* d_grid = nullptr;       // grid read: priors | results | counters
     double* h_grid = nullptr;       // its host side, pinned (a slice of the staging buffer when it fits there, else grown)
     size_t cap_grid = 0, cap_h_grid = 0;
-    // where the read in flight lands on the host (read_back, grid_read_enqueue): read_n output blocks of read_stride doubles,
-    // each in finalize_kernel's layout, then the counters
+    // where the read in flight lands on the host (read_back, grid_read_enqueue, table_read_enqueue): read_n output blocks of
+    // read_stride doubles, each in finalize_kernel's layout (read_table: one class table of read_stride doubles), then the
+    // counters
     const double* h_read = nullptr;
     int read_n = 0;
     size_t read_stride = 0;
+    bool read_table = false;
 };
 
 namespace {
@@ -709,6 +724,48 @@ int launch_pdl(pipsort_engine* e, void (*kernel)(P...), unsigned blocks, unsigne
     e->launches++;
     return 0;
 }
+
+// The largest value of f on [a, b] by Brent's method (golden section with parabolic steps), x to within 1.5e-8 |x| + 1e-10;
+// *fx receives f there.  -inf values are handled as any value below the others.
+template <class F>
+double brent_max(F f, double a, double b, double* fx_out) {
+    const double CG = 0.3819660112501051;
+    double x = a + CG * (b - a), w = x, v = x, fx = -f(x), fw = fx, fv = fx, d = 0.0, e = 0.0;
+    for (int it = 0; it < 200; it++) {
+        const double m = 0.5 * (a + b), tol1 = 1.5e-8 * std::fabs(x) + 1e-10, tol2 = 2.0 * tol1;
+        if (std::fabs(x - m) <= tol2 - 0.5 * (b - a)) break;
+        bool golden = true;
+        if (std::fabs(e) > tol1) {
+            double r = (x - w) * (fx - fv), q = (x - v) * (fx - fw), pp = (x - v) * q - (x - w) * r;
+            q = 2.0 * (q - r);
+            if (q > 0.0) pp = -pp;
+            else q = -q;
+            const double etemp = e;
+            e = d;
+            if (std::fabs(pp) < std::fabs(0.5 * q * etemp) && pp > q * (a - x) && pp < q * (b - x)) {   // false for NaN
+                d = pp / q;
+                if ((x + d) - a < tol2 || b - (x + d) < tol2) d = x < m ? tol1 : -tol1;
+                golden = false;
+            }
+        }
+        if (golden) { e = (x >= m ? a : b) - x; d = CG * e; }
+        const double u = x + (std::fabs(d) >= tol1 ? d : (d > 0.0 ? tol1 : -tol1));
+        const double fu = -f(u);
+        if (fu <= fx) {
+            if (u >= x) a = x; else b = x;
+            v = w; fv = fw; w = x; fw = fx; x = u; fx = fu;
+        } else {
+            if (u < x) a = u; else b = u;
+            if (fu <= fw || w == x) { v = w; fv = fw; w = u; fw = fu; }
+            else if (fu <= fv || v == x || v == w) { v = u; fv = fu; }
+        }
+    }
+    *fx_out = -fx;
+    return x;
+}
+
+double logit(double x) { return std::log(x) - std::log1p(-x); }
+double expit(double u) { return 1.0 / (1.0 + std::exp(-u)); }
 
 // blocks of a finalize: one warp per scalar and per union SNP
 unsigned finalize_blocks(const pipsort_engine* e) { return (e->U + 3 + FIN_WARPS - 1) / FIN_WARPS; }
@@ -1627,11 +1684,12 @@ static int flags_to_error(const double* c) {
 }
 
 // the finalize of a class-resolved store for n_priors priors (device table `pri`, PRIOR_STRIDE doubles each) into `res`;
-// evidence: the three scalars per prior only (one block)
-static int finalize_grid_launch(pipsort_engine* e, int n_priors, const double* pri, double* res, bool clear, bool evidence = false) {
+// GRID_EVIDENCE: the three scalars per prior only (one block); GRID_TABLE: the class table up to tab_c (one block, no priors)
+static int finalize_grid_launch(pipsort_engine* e, int n_priors, const double* pri, double* res, bool clear, GridMode mode = GRID_FULL,
+                                int tab_c = 0) {
     CU(cudaSetDevice(e->device));
-    return launch_pdl(e, finalize_grid_kernel, evidence ? 1 : finalize_blocks(e), FIN_WARPS * 32, e->L.acc, e->U, n_priors, pri,
-                      e->L.neg_half_K, res, clear ? 1 : 0, evidence ? 1 : 0);
+    return launch_pdl(e, finalize_grid_kernel, mode == GRID_FULL ? finalize_blocks(e) : 1u, FIN_WARPS * 32, e->L.acc, e->U, n_priors,
+                      pri, e->L.neg_half_K, res, clear ? 1 : 0, (int)mode, tab_c);
 }
 
 static int finalize_launch(pipsort_engine* e, bool clear) {
@@ -1669,6 +1727,7 @@ static int read_back(pipsort_engine* e) {
     e->h_read = hres;
     e->read_n = 1;
     e->read_stride = 3 + (size_t)5 * e->U;
+    e->read_table = false;
     return 0;
 }
 
@@ -1681,15 +1740,16 @@ static int read_enqueue(pipsort_engine* e) {
 
 static void scatter_results(const pipsort_engine* e, const double* r, const pipsort_outputs* out);
 
-// second half of a read or a grid read: wait for the engine's stream, check the error counters, scatter output block i into
-// outs[i]
-static int read_complete(pipsort_engine* e, const pipsort_outputs* outs) {
+// second half of a read, a grid read or a table read: wait for the engine's stream, check the error counters, scatter output
+// block i into outs[i] (a table read: copy the table into `table`)
+static int read_complete(pipsort_engine* e, const pipsort_outputs* outs, double* table = nullptr) {
     CU(cudaStreamSynchronize(e->stream));
     const double* counters = e->h_read + (size_t)e->read_n * e->read_stride;
     int rc = flags_to_error(counters);
     if (rc) return rc;
     e->last_read_count = (uint64_t)counters[0];
-    for (int i = 0; i < e->read_n; i++) scatter_results(e, e->h_read + (size_t)i * e->read_stride, &outs[i]);
+    if (e->read_table) memcpy(table, e->h_read, e->read_stride * sizeof(double));
+    else for (int i = 0; i < e->read_n; i++) scatter_results(e, e->h_read + (size_t)i * e->read_stride, &outs[i]);
     return 0;
 }
 
@@ -1739,13 +1799,10 @@ static bool evidence_only(const pipsort_outputs* outs, int n) {
     return true;
 }
 
-// first half of a grid read (tables from grid_tables): the locus's prior tables and the results go through one pinned
-// buffer, priors | results | counters as d_grid, so that the upload, the finalize and the read-back are enqueued without
-// blocking.  The staging buffer serves it when it fits: a list of loci creates an engine per locus, and a pinned
-// allocation of its own would cost each locus a cudaMallocHost and a cudaFreeHost.
-static int grid_read_enqueue(pipsort_engine* e, int n_priors, const double* tab, bool evidence) {
-    const size_t stride = evidence ? 3 : 3 + (size_t)5 * e->U, npri = (size_t)n_priors * PRIOR_STRIDE;
-    const size_t need = npri + (size_t)n_priors * stride + NCOUNTER;
+// d_grid and its pinned host side h_grid, `need` doubles each: the pinned side is a slice of the staging buffer when it fits
+// there -- a list of loci creates an engine per locus, and a pinned allocation of its own would cost each locus a
+// cudaMallocHost and a cudaFreeHost.
+static int grid_buffers(pipsort_engine* e, size_t need) {
     CU(cudaSetDevice(e->device));
     int rc;
     if ((rc = grow(e, &e->d_grid, &e->cap_grid, need))) return rc;
@@ -1754,18 +1811,56 @@ static int grid_read_enqueue(pipsort_engine* e, int n_priors, const double* tab,
         if (s) { e->h_grid = reinterpret_cast<double*>(s); e->cap_h_grid = need; }
         else if ((rc = grow(e, &e->h_grid, &e->cap_h_grid, need, Mem::pinned))) return rc;
     }
+    return 0;
+}
+
+// first half of a grid read (tables from grid_tables): the locus's prior tables and the results go through one pinned
+// buffer, priors | results | counters as d_grid, so that the upload, the finalize and the read-back are enqueued without
+// blocking.
+static int grid_read_enqueue(pipsort_engine* e, int n_priors, const double* tab, bool evidence) {
+    const size_t stride = evidence ? 3 : 3 + (size_t)5 * e->U, npri = (size_t)n_priors * PRIOR_STRIDE;
+    const size_t need = npri + (size_t)n_priors * stride + NCOUNTER;
+    int rc;
+    if ((rc = grid_buffers(e, need))) return rc;
     memcpy(e->h_grid, tab, npri * sizeof(double));
     for (int i = 0; i < n_priors; i++) {
         double& cx = e->h_grid[(size_t)i * PRIOR_STRIDE + PRIOR_STRIDE - 1];
         cx = grid_cx(e, cx);
     }
     CU(cudaMemcpyAsync(e->d_grid, e->h_grid, npri * sizeof(double), cudaMemcpyHostToDevice, e->stream));
-    if ((rc = finalize_grid_launch(e, n_priors, e->d_grid, e->d_grid + npri, false, evidence))) return rc;
+    if ((rc = finalize_grid_launch(e, n_priors, e->d_grid, e->d_grid + npri, false, evidence ? GRID_EVIDENCE : GRID_FULL))) return rc;
     CU(cudaMemcpyAsync(e->h_grid + npri, e->d_grid + npri, (need - npri) * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
     e->h_read = e->h_grid + npri;
     e->read_n = n_priors;
     e->read_stride = stride;
+    e->read_table = false;
     return 0;
+}
+
+// first half of a table read (c <= the class limit): the table mode of the grid finalize, (c+1)(c+2)/2 + NCOUNTER doubles back
+// through the grid read's buffers, nothing uploaded
+static int table_read_enqueue(pipsort_engine* e, int c) {
+    const size_t ntab = cls_ntab(c), need = ntab + NCOUNTER;
+    int rc;
+    if ((rc = grid_buffers(e, need))) return rc;
+    if ((rc = finalize_grid_launch(e, 0, nullptr, e->d_grid, false, GRID_TABLE, c))) return rc;
+    CU(cudaMemcpyAsync(e->h_grid, e->d_grid, need * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+    e->h_read = e->h_grid;
+    e->read_n = 1;
+    e->read_stride = ntab;
+    e->read_table = true;
+    return 0;
+}
+
+int pipsort_read_class_evidence(pipsort_engine* e, int c, double* table, uint64_t* n_configs) {
+    if (!e) return fail(PIPSORT_E_ARG, "null engine");
+    if (!e->classes) return fail(PIPSORT_E_ARG, "the engine was not created with PIPSORT_PRIOR_CLASSES: its store has no prior classes");
+    if (c < 0 || c > e->kb) return fail(PIPSORT_E_ARG, "c=%d must be in [0, %d] (the engine's class limit)", c, e->kb);
+    if (!table) return fail(PIPSORT_E_ARG, "null table");
+    int rc = table_read_enqueue(e, c);
+    if (!rc) rc = read_complete(e, nullptr, table);
+    if (!rc && n_configs) *n_configs = e->last_read_count;
+    return rc;
 }
 
 int pipsort_read_prior_grid(pipsort_engine* e, int n_priors, const double* gamma, const double* sharing_param,
@@ -1799,8 +1894,9 @@ int pipsort_posterior_exhaustive(const pipsort_locus* locus, int device, uint32_
 }
 
 // The grid read of a list of loci (pipsort_posterior_exhaustive_grid_batch): n priors whose tables are built once
-// (grid_tables); locus i reports into outs[i * n ..].  n == 0: the ordinary read, locus i into outs[i].
-struct GridRead { int n; const double* tab; };
+// (grid_tables); locus i reports into outs[i * n ..].  n == 0: the ordinary read, locus i into outs[i].  table_c >= 0: the table
+// read (pipsort_class_evidence_batch), locus i into tables[i * cls_ntab(table_c) ..].
+struct GridRead { int n; const double* tab; int table_c = -1; double* tables = nullptr; };
 
 // loci first, first + stride, first + 2 stride, ... through a software pipeline over DEPTH engines, each on its own stream:
 // while locus i is being evaluated the uploads and the preparation launches of the next one are already queued, and the
@@ -1813,11 +1909,13 @@ static int batch_worker(const pipsort_locus* loci, int32_t n_loci, int first, in
     pipsort_engine* inflight[DEPTH] = {nullptr, nullptr, nullptr};
     int idx_of[DEPTH] = {-1, -1, -1};
     int rc = 0;
-    if (grid.n) flags |= PIPSORT_PRIOR_CLASSES;
-    auto finish = [&](int slot) -> int {       // results of the locus in pipeline slot `slot`: its read_n output blocks
+    const bool table = grid.table_c >= 0;
+    if (grid.n || table) flags |= PIPSORT_PRIOR_CLASSES;
+    auto finish = [&](int slot) -> int {       // results of the locus in pipeline slot `slot`: its read_n output blocks or its table
         pipsort_engine*& e = inflight[slot];
         const int i = idx_of[slot];
-        int r = read_complete(e, &outs[(size_t)i * e->read_n]);
+        int r = table ? read_complete(e, nullptr, grid.tables + (size_t)i * e->read_stride)
+                      : read_complete(e, &outs[(size_t)i * e->read_n]);
         if (!r && n_configs) n_configs[i] = e->last_read_count;
         pipsort_destroy(e);
         e = nullptr;
@@ -1836,7 +1934,9 @@ static int batch_worker(const pipsort_locus* loci, int32_t n_loci, int first, in
         uint64_t total = 0;
         rc = pipsort_total_ranks(e, c, &total);
         if (!rc) rc = pipsort_run_exhaustive(e, c, 0, total);
-        if (!rc) rc = grid.n ? grid_read_enqueue(e, grid.n, grid.tab, evidence_only(&outs[(size_t)i * grid.n], grid.n)) : read_enqueue(e);
+        if (!rc) rc = table    ? table_read_enqueue(e, grid.table_c)
+                      : grid.n ? grid_read_enqueue(e, grid.n, grid.tab, evidence_only(&outs[(size_t)i * grid.n], grid.n))
+                               : read_enqueue(e);
     }
     // drain in issue order (also after an error: every engine still in flight is destroyed)
     for (int d = 0; d < DEPTH; d++) {
@@ -1888,6 +1988,158 @@ int pipsort_posterior_exhaustive_grid_batch(const pipsort_locus* loci, int32_t n
     int rc = grid_tables(n_priors, gamma, sharing_param, &tab);
     if (rc || !n_loci) return rc;
     return batch_run(loci, n_loci, device, flags, c, GridRead{n_priors, tab.data()}, outs, n_configs);
+}
+
+int pipsort_class_evidence_batch(const pipsort_locus* loci, int32_t n_loci, int device, uint32_t flags, int c, double* tables,
+                                 uint64_t* n_configs) {
+    if (n_loci < 0 || (n_loci > 0 && (!loci || !tables))) return fail(PIPSORT_E_ARG, "bad argument");
+    if (c < 0 || c > KMAX) return fail(PIPSORT_E_ARG, "c=%d must be in [0, %d]", c, KMAX);
+    if (!n_loci) return 0;
+    return batch_run(loci, n_loci, device, flags, c, GridRead{0, nullptr, c, tables}, nullptr, n_configs);
+}
+
+// ---- choosing the prior from class tables (pipsort_fit_prior; host code, DESIGN.md section 5f) ------------------------------
+// sum_i total_i(gamma, p), total_i = U_i log(1-gamma) + log sum_k pi'_k exp(tab_ik) over the classes k = cls_T(J, a), with
+// pi' from prior_tables (the engine's own weights: p == 0 skips the sharing term, p == 1 gives a < J the weight 0).
+// A locus's classes are kept scaled once, exp(tab_ik - top_i) with top_i its largest class, so that an evaluation is a dot
+// product and one log per locus; a locus with a class more than 700 nats below its top (it would underflow), or whose
+// weighted sum comes out tiny (every class with a non-zero weight far below top_i), is summed in log space instead.
+struct ClassEvidence {
+    int n, ntab;
+    const double* tab;
+    const int32_t* U;
+    std::vector<double> scaled, top;
+    std::vector<char> scaled_ok;
+
+    ClassEvidence(int n_, int ntab_, const double* tab_, const int32_t* U_)
+        : n(n_), ntab(ntab_), tab(tab_), U(U_), scaled((size_t)n_ * ntab_), top(n_, -INFINITY), scaled_ok(n_, 1) {
+        for (int i = 0; i < n; i++) {
+            const double* t = tab + (size_t)i * ntab;
+            for (int k = 0; k < ntab; k++) top[i] = std::max(top[i], t[k]);
+            for (int k = 0; k < ntab; k++) {
+                scaled[(size_t)i * ntab + k] = std::exp(t[k] - top[i]);
+                if (t[k] > -INFINITY && !(t[k] - top[i] >= -700.0)) scaled_ok[i] = 0;
+            }
+            if (top[i] == -INFINITY) scaled_ok[i] = 0;
+        }
+    }
+
+    // the joint log evidence at (gam, p) (validated by the caller); out[i] (may be NULL) receives total_i
+    double operator()(double gam, double p, double* out) const {
+        double pi[KMAX + 1][KMAX + 1], w[cls_ntab(KMAX)], lw[cls_ntab(KMAX)];
+        prior_tables(gam, p, 0, 0, pi, nullptr, nullptr);
+        for (int J = 0, k = 0; k < ntab; J++)
+            for (int a = 0; a <= J; a++, k++) { w[k] = pi[J][a]; lw[k] = std::log(w[k]); }
+        const double l1m = std::log(1.0 - gam);
+        double sum = 0.0;
+        for (int i = 0; i < n; i++) {
+            const double* t = tab + (size_t)i * ntab;
+            double v = -INFINITY;
+            if (scaled_ok[i]) {
+                const double* s = scaled.data() + (size_t)i * ntab;
+                double acc = 0.0;
+                for (int k = 0; k < ntab; k++) acc += w[k] * s[k];
+                if (acc > 1e-290) v = top[i] + std::log(acc);
+            }
+            if (v == -INFINITY) {
+                double m = -INFINITY, acc = 0.0;
+                for (int k = 0; k < ntab; k++) m = std::max(m, lw[k] + t[k]);
+                if (m > -INFINITY) {
+                    for (int k = 0; k < ntab; k++) acc += std::exp(lw[k] + t[k] - m);
+                    v = m + std::log(acc);
+                }
+            }
+            v += U[i] * l1m;
+            if (out) out[i] = v;
+            sum += v;
+        }
+        return sum;
+    }
+};
+
+int pipsort_fit_prior(int32_t n_loci, int c, const double* tables, const int32_t* union_count, uint32_t fit, double* gamma,
+                      double* sharing_param, double* joint_log_evidence, double* log_evidence) {
+    if (n_loci < 1) return fail(PIPSORT_E_ARG, "n_loci=%d must be >= 1", n_loci);
+    if (c < 0 || c > KMAX) return fail(PIPSORT_E_ARG, "c=%d must be in [0, %d]", c, KMAX);
+    if (fit > 3) return fail(PIPSORT_E_ARG, "fit=%u must be <= 3 (1: gamma, 2: sharing_param)", fit);
+    if (!tables || !union_count || !gamma || !sharing_param) return fail(PIPSORT_E_ARG, "null argument");
+    if (!(*gamma > 0.0 && *gamma < 1.0)) return fail(PIPSORT_E_ARG, "gamma=%g must be in (0,1)", *gamma);
+    if (!(*sharing_param >= 0.0 && *sharing_param <= 1.0)) return fail(PIPSORT_E_ARG, "sharing_param=%g must be in [0,1]", *sharing_param);
+    const int ntab = cls_ntab(c);
+    for (int i = 0; i < n_loci; i++) {
+        if (union_count[i] < 1) return fail(PIPSORT_E_ARG, "union_count[%d]=%d must be >= 1", i, union_count[i]);
+        for (int k = 0; k < ntab; k++) {
+            const double t = tables[(size_t)i * ntab + k];
+            if (std::isnan(t) || t == INFINITY) return fail(PIPSORT_E_ARG, "tables[%d][%d]=%g: a class value is finite or -inf", i, k, t);
+        }
+    }
+    const ClassEvidence S(n_loci, ntab, tables, union_count);
+    const bool fit_g = fit & 1, fit_p = fit & 2;
+    // candidates: gamma in log-odds over [1e-8, 1 - 1e-8]; p in log-odds over [1e-12, 1 - 1e-12], and p = 1.  Not p = 0: the
+    // skip rule weighs every class at least as much as any p in (0, 1] does, so it would win on every locus with a class J >= 1
+    const double LG = logit(1.0 - 1e-8), LP = logit(1.0 - 1e-12);
+    const int NG = fit_g ? 64 : 1, NPI = 128;
+    const double dg = 2.0 * LG / 63, dp = 2.0 * LP / (NPI - 1);
+    std::vector<double> gs(NG), ps;
+    for (int k = 0; k < NG; k++) gs[k] = fit_g ? expit(-LG + k * dg) : *gamma;
+    if (fit_p) {
+        for (int k = 0; k < NPI; k++) ps.push_back(expit(-LP + k * dp));
+        ps.push_back(1.0);
+    } else {
+        ps.push_back(*sharing_param);
+    }
+    // the grid; best[j]: the best gamma of column j
+    struct Pt { double g, p, f; };
+    std::vector<Pt> best(ps.size(), Pt{0.0, 0.0, -INFINITY});
+    std::vector<double> per(n_loci);
+    std::vector<char> seen(n_loci, 0);
+    for (size_t j = 0; j < ps.size(); j++)
+        for (int k = 0; k < NG; k++) {
+            const double f = S(gs[k], ps[j], per.data());
+            for (int i = 0; i < n_loci; i++) seen[i] |= per[i] > -INFINITY;
+            if (k == 0 || f > best[j].f) best[j] = Pt{gs[k], ps[j], f};
+        }
+    for (int i = 0; i < n_loci; i++)
+        if (!seen[i]) return fail(PIPSORT_E_ARG, "locus %d: its log evidence is -inf at every candidate prior (no class with a non-zero weight)", i);
+    // one coordinate at a time, within one grid step of the current point either side (log-odds)
+    auto refine_g = [&](Pt x) {
+        const double u0 = logit(x.g);
+        double f;
+        const double u = brent_max([&](double t) { return S(expit(t), x.p, nullptr); }, std::max(-LG, u0 - dg), std::min(LG, u0 + dg), &f);
+        if (f > x.f) x = Pt{expit(u), x.p, f};
+        return x;
+    };
+    auto refine_p = [&](Pt x) {
+        const double u0 = logit(x.p);
+        double f;
+        const double u = brent_max([&](double t) { return S(x.g, expit(t), nullptr); }, std::max(-LP, u0 - dp), std::min(LP, u0 + dp), &f);
+        if (f > x.f) x = Pt{x.g, expit(u), f};
+        return x;
+    };
+    auto local = [&](Pt x, bool vary_p) {
+        for (int round = 0; round < 100 && (fit_g || vary_p); round++) {
+            const double before = x.f;
+            if (fit_g) x = refine_g(x);
+            if (vary_p) x = refine_p(x);
+            if (!(x.f - before >= 1e-9)) break;
+        }
+        return x;
+    };
+    Pt x;
+    if (fit_p) {
+        x = best[0];
+        for (int j = 1; j < NPI; j++) if (best[j].f > x.f) x = best[j];
+        x = local(x, true);
+        const Pt one = local(best[NPI], false);
+        if (one.f > x.f) x = one;
+    } else {
+        x = local(best[0], false);
+    }
+    *gamma = x.g;
+    *sharing_param = x.p;
+    const double joint = S(x.g, x.p, log_evidence);
+    if (joint_log_evidence) *joint_log_evidence = joint;
+    return 0;
 }
 
 int pipsort_last_read_config_count(const pipsort_engine* e, uint64_t* out) {

@@ -75,6 +75,11 @@ def lib():
         L.pipsort_posterior_exhaustive_grid_batch.argtypes = [C.POINTER(_LocusV), C.c_int32, i32, C.c_uint32, i32, i32,
                                                               C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(_OutputsV),
                                                               C.POINTER(u64)]
+        L.pipsort_read_class_evidence.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(u64)]
+        L.pipsort_class_evidence_batch.argtypes = [C.POINTER(_LocusV), C.c_int32, i32, C.c_uint32, i32, C.POINTER(C.c_double),
+                                                   C.POINTER(u64)]
+        L.pipsort_fit_prior.argtypes = [C.c_int32, i32, C.POINTER(C.c_double), C.POINTER(C.c_int32), C.c_uint32,
+                                        C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_double)]
         L.pipsort_destroy.argtypes = [vp]
         L.pipsort_destroy.restype = None
         L.pipsort_reset.argtypes = [vp]
@@ -322,6 +327,13 @@ class Engine:
         _check(lib().pipsort_read_prior_grid(self._h, len(gam), _dp(gam), _dp(p), outs, C.byref(cnt)))
         return res(int(cnt.value))
 
+    def read_class_evidence(self, c):
+        """The class table of the store (an engine created with prior_classes=True; pipsort_read_class_evidence): ndarray
+        [(c+1)(c+2)/2], entry J(J+1)/2 + a = -K/2 + log T[J][a], -inf for an empty class.  fit_prior takes it."""
+        tab = np.empty(_ntab(c))
+        _check(lib().pipsort_read_class_evidence(self._h, int(c), _dp(tab), None))
+        return tab
+
     def finalize(self, reset=False):
         """Bins -> log-space results on the device; reset=True also leaves the accumulators empty (no reset() needed before
         the next pass; fetch() then returns the results)."""
@@ -455,6 +467,11 @@ def posterior_exhaustive(num_snps, sigma, z, d, K, snp_map, c, gamma=0.01, shari
     return Results(float(total[0]), post, nc, sp, sl, nl, int(cnt.value))
 
 
+def _ntab(c):
+    """Entries of a class table up to class limit c (0 for a c the engine refuses)."""
+    return max(0, (int(c) + 1) * (int(c) + 2) // 2)
+
+
 def _prior_arrays(priors):
     pr = np.asarray(priors, dtype=np.float64).reshape(-1, 2) if len(priors) else np.zeros((0, 2))
     return np.ascontiguousarray(pr[:, 0]), np.ascontiguousarray(pr[:, 1])
@@ -536,11 +553,15 @@ class LocusBatch:
     optionally gamma, sharing_param); sigma / z flat float64 arrays (studies concatenated).
     priors: a list of (gamma, p) -- run() is then pipsort_posterior_exhaustive_grid_batch, one result block per locus and
     prior (results() gives a list of Results per locus); evidence_only=True leaves every per-SNP member NULL (the evidence
-    read) and the buffer holds (total, noCausal[0], noCausal[1]) per locus and prior, read with evidence()."""
+    read) and the buffer holds (total, noCausal[0], noCausal[1]) per locus and prior, read with evidence().
+    class_evidence=True: run() is pipsort_class_evidence_batch, the buffer holds every locus's class table
+    ((c+1)(c+2)/2 doubles, Engine.read_class_evidence's layout), read with tables()."""
 
-    def __init__(self, loci, c, device=0, raw_ld=False, priors=None, evidence_only=False):
+    def __init__(self, loci, c, device=0, raw_ld=False, priors=None, evidence_only=False, class_evidence=False):
         if evidence_only and priors is None:
             raise ValueError("evidence_only needs priors")
+        if class_evidence and priors is not None:
+            raise ValueError("class_evidence takes no priors")
         n = self.n = len(loci)
         self.c, self.device, self.flags = int(c), int(device), RAW_LD if raw_ld else 0
         f64, i32 = np.dtype(np.float64), np.dtype(np.int32)
@@ -564,8 +585,12 @@ class LocusBatch:
         la["max_causal"] = self.c
         self.priors = None if priors is None else _prior_arrays(priors)
         self.evidence_only = bool(evidence_only)
+        self.class_evidence = bool(class_evidence)
         k = self.k = 1 if priors is None else len(self.priors[0])      # result blocks per locus: locus i, prior j -> i * k + j
-        if evidence_only:
+        if class_evidence:
+            buf = self.buf = np.empty(n * _ntab(self.c))
+            oa = self.oa = np.zeros(0, dtype=_OUT_DT)
+        elif evidence_only:
             buf = self.buf = np.empty(n * k * 3)
             b0 = buf.ctypes.data + 24 * np.arange(n * k, dtype=np.int64)
             oa = self.oa = np.zeros(n * k, dtype=_OUT_DT)              # per-SNP members NULL
@@ -588,7 +613,9 @@ class LocusBatch:
         self.cnt = np.zeros(n, dtype=np.uint64)
         lp, op = C.cast(la.ctypes.data, C.POINTER(_LocusV)), C.cast(oa.ctypes.data, C.POINTER(_OutputsV))
         cp = C.cast(self.cnt.ctypes.data, C.POINTER(C.c_uint64))
-        if priors is None:
+        if class_evidence:
+            self._args = (lp, n, self.device, self.flags, self.c, _dp(buf), cp)
+        elif priors is None:
             self._args = (lp, n, self.device, self.flags, self.c, op, cp)
         else:
             gam, p = self.priors
@@ -597,7 +624,9 @@ class LocusBatch:
     def run(self):
         """pipsort_posterior_exhaustive_batch (pipsort_posterior_exhaustive_grid_batch with priors): host buffers in, host
         buffers out."""
-        if self.priors is not None:         # the priors are validated even for an empty list
+        if self.class_evidence:
+            _check(lib().pipsort_class_evidence_batch(*self._args))
+        elif self.priors is not None:       # the priors are validated even for an empty list
             _check(lib().pipsort_posterior_exhaustive_grid_batch(*self._args))
         elif self.n:
             _check(lib().pipsort_posterior_exhaustive_batch(*self._args))
@@ -605,8 +634,8 @@ class LocusBatch:
 
     def results(self):
         """A Results per locus; with priors, a list of Results (one per prior) per locus."""
-        if self.evidence_only:
-            raise ValueError("an evidence-only batch has no per-SNP results: use evidence()")
+        if self.evidence_only or self.class_evidence:
+            raise ValueError("an evidence-only or class-evidence batch has no per-SNP results: use evidence() / tables()")
         out, buf, k = [], self.buf, self.k
         offl, Nl, Sl, Ul, cl = self.off.tolist(), self.N.tolist(), self.S.tolist(), self.U.tolist(), self.cnt.tolist()
         for i in range(self.n):
@@ -630,6 +659,12 @@ class LocusBatch:
         nc = o + 1 + np.repeat(self.N, self.k)
         return np.stack([self.buf[o], self.buf[nc], self.buf[nc + 1]], axis=-1).reshape(self.n, self.k, 3)
 
+    def tables(self):
+        """ndarray [n_loci, (c+1)(c+2)/2] of class tables (a class_evidence batch)."""
+        if not self.class_evidence:
+            raise ValueError("tables() needs a class_evidence batch")
+        return self.buf.reshape(self.n, _ntab(self.c)).copy()
+
 
 def posterior_exhaustive_batch(loci, c, device=0, raw_ld=False):
     """A list of loci in one call (pipsort_posterior_exhaustive_batch): the engine pipelines them over three streams, so
@@ -644,6 +679,41 @@ def posterior_exhaustive_grid_batch(loci, c, priors, device=0, raw_ld=False, evi
     or with evidence_only=True the ndarray [n_loci, n_priors, 3] of (total, noCausal[0], noCausal[1])."""
     B = LocusBatch(loci, c, device, raw_ld, priors=priors, evidence_only=evidence_only).run()
     return B.evidence() if evidence_only else B.results()
+
+
+def class_evidence_batch(loci, c, device=0, raw_ld=False):
+    """The class table of every locus (pipsort_class_evidence_batch): one class-resolved pass per locus, pipelined as
+    posterior_exhaustive_batch.  loci as posterior_exhaustive_batch takes them; returns ndarray [n_loci, (c+1)(c+2)/2]."""
+    return LocusBatch(loci, c, device, raw_ld, class_evidence=True).run().tables()
+
+
+_FIT = {"gamma": 1, "p": 2, "gamma,p": 3}
+
+
+def fit_prior(tables, union_counts, fit="p", gamma=0.01, p=0.75):
+    """The prior of largest joint log evidence over the loci of `tables` ([n_loci, (c+1)(c+2)/2], from class_evidence_batch
+    or Engine.read_class_evidence; union_counts: U per locus) -- pipsort_fit_prior, host code, no device.  fit: "p",
+    "gamma", "gamma,p", or the bit mask itself (1 gamma, 2 p; 0 evaluates at (gamma, p) only); a parameter not fitted keeps
+    the value given.  Returns (gamma, p, joint_log_evidence, per_locus_log_evidence).  Then run posterior_exhaustive_batch at
+    that prior for the PIPs."""
+    if isinstance(fit, str) and fit not in _FIT:
+        raise ValueError(f"fit must be one of {sorted(_FIT)} or a bit mask")
+    bits = _FIT[fit] if isinstance(fit, str) else int(fit)
+    tab = np.ascontiguousarray(tables, dtype=np.float64)
+    if tab.ndim != 2:
+        raise ValueError("tables must be [n_loci, (c+1)(c+2)/2]")
+    n, w = tab.shape
+    c = next((k for k in range(KMAX + 1) if _ntab(k) == w), -1)
+    if c < 0:
+        raise ValueError(f"a class table has (c+1)(c+2)/2 entries for some c in [0, {KMAX}], not {w}")
+    U = np.ascontiguousarray(union_counts, dtype=np.int32).ravel()
+    if U.size != n:
+        raise ValueError("one union count per locus")
+    g, q, joint = C.c_double(gamma), C.c_double(p), C.c_double()
+    per = np.empty(n)
+    _check(lib().pipsort_fit_prior(n, c, _dp(tab), U.ctypes.data_as(C.POINTER(C.c_int32)), bits, C.byref(g), C.byref(q),
+                                   C.byref(joint), _dp(per)))
+    return g.value, q.value, joint.value, per
 
 
 def preprocess_study(ld, z, device=0):
