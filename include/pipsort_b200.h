@@ -48,6 +48,12 @@ extern "C" {
                                    report it.  Such an engine refuses pipsort_sss(_sharded), pipsort_score_union_configs*,
                                    pipsort_score_given_configs* and pipsort_p2p_combine_finalize (PIPSORT_E_ARG). */
 
+#define PIPSORT_CAUSAL_COUNTS 16u /* implies PIPSORT_PRIOR_CLASSES: the class-resolved store also keeps the count table
+                                    R[a][b0][b1] -- the total split by the numbers of SNPs causal in both studies (a), in study 0
+                                    only (b0) and in study 1 only (b1), C(C+3, 3) scalars for class limit C -- so that
+                                    pipsort_read_count_table gives the posterior of the causal counts under any prior.  Every
+                                    read of a class-resolved engine works unchanged; the calls it refuses are refused too. */
+
 typedef struct pipsort_engine pipsort_engine;
 
 /* Locus description = the PostCal constructor arguments the likelihood actually consumes
@@ -267,6 +273,33 @@ int pipsort_read_class_evidence(pipsort_engine* e, int c, double* table, uint64_
  * not used.  n_loci == 0 returns 0.  Stops at the first error, as pipsort_posterior_exhaustive_batch does.            */
 int pipsort_class_evidence_batch(const pipsort_locus* loci, int32_t n_loci, int device, uint32_t flags, int c, double* tables,
                                  uint64_t* n_configs);
+
+/* The count table of a PIPSORT_CAUSAL_COUNTS store (DESIGN.md section 5f, "Causal counts"):
+ *   table[cnt_idx(J, a, b0)] = -K/2 + log R[a][b0][b1],   cnt_idx(J, a, b0) = J(J+1)(J+2)/6 + a(2J+3-a)/2 + b0,
+ * for every J = a + b0 + b1 <= c: C(c+3, 3) doubles (20 at c = 3), the table at c the prefix of the one at any larger c.
+ * R[a][b0][b1] is the unweighted sum of E_0 E_1 over the expanded configurations with a SNPs causal in both studies, b0 in
+ * study 0 only and b1 in study 1 only (the null configuration adds e^-1 to R[0][0][0]); sum_{b0} R[a][b0][J-a-b0] = T[J][a]
+ * of pipsort_read_class_evidence.  An empty class is -inf.  One finalize launch, no prior uploaded.  Only for a
+ * PIPSORT_CAUSAL_COUNTS engine, 0 <= c <= its class limit (PIPSORT_E_ARG otherwise, naming why); the store may be the sum of
+ * several engines' as for pipsort_read_class_evidence.  n_configs (optional) receives the configuration count.         */
+int pipsort_read_count_table(pipsort_engine* e, int c, double* table, uint64_t* n_configs);
+
+/* The count tables of a list of loci: pipsort_create (flags | PIPSORT_CAUSAL_COUNTS) + pipsort_run_exhaustive over the whole
+ * rank space + pipsort_read_count_table + pipsort_destroy per locus, pipelined as pipsort_class_evidence_batch (same host
+ * threads, same depth).  Locus i goes to tables[i * C(c+3, 3) ..], n_configs[i] (optional) receives its configuration count.
+ * n_loci == 0 returns 0.  Stops at the first error, as pipsort_posterior_exhaustive_batch does.                        */
+int pipsort_count_table_batch(const pipsort_locus* loci, int32_t n_loci, int device, uint32_t flags, int c, double* tables,
+                              uint64_t* n_configs);
+
+/* The posterior of the causal counts under one prior (gamma, p), per locus, from count tables (tables[i * C(c+3, 3) ..] as
+ * pipsort_read_count_table writes them, union_count[i] = U of locus i).  Pure host code: needs no device.
+ *   post[i * C(c+3, 3) + cnt_idx(J, a, b0)] = pi'(J, a) exp(table) / sum over the classes of locus i,
+ *   log_evidence[i] (optional) = U log(1-gamma) + log sum_k pi'_k exp(table_k)  -- the total of the grid read at that prior.
+ * The weights pi' are the engine's own (prior_tables), so p == 0 and p == 1 follow the reference's rules as in
+ * pipsort_fit_prior.  PIPSORT_E_ARG: n_loci < 1, c outside [0, 8], gamma outside (0,1), p outside [0,1], union_count < 1, a
+ * NaN or +inf in a table, or a locus whose every class has weight 0 or is -inf (the message names the locus).          */
+int pipsort_count_posterior(int32_t n_loci, int c, const double* tables, const int32_t* union_count, double gamma,
+                            double sharing_param, double* post, double* log_evidence);
 
 /* The prior (gamma, p) of largest joint log evidence sum_i total_i(gamma, p) over n_loci loci, from their class tables
  * (tables[i * (c+1)(c+2)/2 ..] as pipsort_read_class_evidence writes them, union_count[i] = U of locus i).  Pure host code:

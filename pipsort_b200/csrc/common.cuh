@@ -150,6 +150,17 @@ __host__ __device__ constexpr int cls_ntab(int C) { return (C + 1) * (C + 2) / 2
 __host__ __device__ constexpr int cls_N(int C, int s, int J) { return cls_ntab(C) + s * (C + 1) + J; }
 __host__ __device__ constexpr int cls_nscal(int C) { return cls_ntab(C) + 2 * (C + 1); }
 
+// Count table (PIPSORT_CAUSAL_COUNTS, DESIGN.md section 5f): a class-resolved store that also keeps R[a][b0][b1], the total
+// split by a SNPs causal in both studies, b0 in study 0 only and b1 in study 1 only (J = a + b0 + b1 <= C), as the scalars
+// after cls_nscal(C).  Within size class J the classes follow a, then b0; the table at any c is the prefix of the one at C.
+__host__ __device__ constexpr int cnt_idx(int J, int a, int b0) { return J * (J + 1) * (J + 2) / 6 + a * (2 * J + 3 - a) / 2 + b0; }
+__host__ __device__ constexpr int cnt_ntab(int C) { return (C + 1) * (C + 2) * (C + 3) / 6; }   // classes (a, b0, b1) with J <= C
+__host__ __device__ constexpr int cls_R(int C, int J, int a, int b0) { return cls_nscal(C) + cnt_idx(J, a, b0); }
+
+// What the accumulator store holds, and so which instantiation of the exhaustive kernels an engine launches: the five-slot
+// store of one prior, the class-resolved store (PIPSORT_PRIOR_CLASSES), or that store with the count table (PIPSORT_CAUSAL_COUNTS)
+enum StoreKind : int { STORE_PLAIN = 0, STORE_CLASSES = 1, STORE_COUNTS = 2 };
+
 // scalar k of the class-resolved store += M * 2^N
 __device__ __forceinline__ void scal_add(const AccDev& a, int k, double M, int N) {
     bin_add(a, cls_nslot(a.ccls) + k / a.Upad, k % a.Upad, M, N);

@@ -270,19 +270,35 @@ __device__ __forceinline__ void xadd_weighted(XAcc& acc, const XAcc& v, double w
 // GRID_TABLE (one block, no priors): the class table up to the class limit tab_c <= C -- res[cls_T(J, a)] = -K/2 + log T[J][a]
 // (cy = -K/2), unweighted, -inf for an empty class (0.0 is a value a class may have) -- then the counters.  Warp 0 decodes
 // the T[J][a] slots as the evidence read does, so that the table and the evidence read cannot disagree.
-enum GridMode : int { GRID_FULL = 0, GRID_EVIDENCE = 1, GRID_TABLE = 2 };
+// GRID_COUNTS (one block, no priors, a store with the count table): the count table up to tab_c <= C -- res[cnt_idx(J, a, b0)] =
+// -K/2 + log R[a][b0][b1], -inf for an empty class -- then the counters; the lanes of warp 0 loop over the classes.
+// counts: the store keeps the count table (PIPSORT_CAUSAL_COUNTS): a read that clears the store clears that table too.
+enum GridMode : int { GRID_FULL = 0, GRID_EVIDENCE = 1, GRID_TABLE = 2, GRID_COUNTS = 3 };
 constexpr int GRID_LANE_SLOTS = (cls_nslot(KMAX) + 31) / 32;
 __global__ void __launch_bounds__(FIN_WARPS * 32) finalize_grid_kernel(AccDev acc, int U, int n_priors, const double* __restrict__ pri,
                                                                        double cy, double* __restrict__ res, int clear, int mode,
-                                                                       int tab_c) {
+                                                                       int tab_c, int counts) {
     asm volatile("griddepcontrol.wait;" ::: "memory");
     const int lane = threadIdx.x & 31;
     const int w = blockIdx.x * FIN_WARPS + (threadIdx.x >> 5);
     const int C = acc.ccls;
     const size_t stride = mode == GRID_FULL ? 3 + (size_t)5 * U : 3;
     if (blockIdx.x == 0 && threadIdx.x < NCOUNTER) {
-        res[(mode == GRID_TABLE ? (size_t)cls_ntab(tab_c) : (size_t)n_priors * stride) + threadIdx.x] = acc.counters[threadIdx.x];
+        const size_t at = mode == GRID_TABLE ? (size_t)cls_ntab(tab_c) : mode == GRID_COUNTS ? (size_t)cnt_ntab(tab_c) : (size_t)n_priors * stride;
+        res[at + threadIdx.x] = acc.counters[threadIdx.x];
         if (clear) acc.counters[threadIdx.x] = 0.0;
+    }
+    if (mode == GRID_COUNTS) {
+        if (w > 0) return;
+        for (int k = lane; k < cnt_ntab(tab_c); k += 32) {
+            const XAcc v = bins_read_lane(acc, cls_nslot(C) + (cls_nscal(C) + k) / acc.Upad, (cls_nscal(C) + k) % acc.Upad, false);
+            res[k] = v.M > 0.0 ? xlog_or_zero(v, cy) : -INFINITY;
+        }
+        return;
+    }
+    if (w == 0 && clear && counts) {   // the count table is not read here: leave it empty for the next pass
+        for (int k = cls_nscal(C) + lane; k < cls_nscal(C) + cnt_ntab(C); k += 32)
+            bins_read_lane(acc, cls_nslot(C) + k / acc.Upad, k % acc.Upad, true);
     }
     if (w < 3) {   // total: T[J][a], weight pi'(J,a);  noCausal[s]: N_s[J], weight pi'(J,0)
         if (mode == GRID_TABLE && w > 0) return;
@@ -630,8 +646,9 @@ int ensure_score_smem(pipsort_engine* e, int ws_kmax, size_t* bytes) {
     if (e->score_smem_set < ws_kmax) {
         size_t mx = SCORE_WARPS * warp_ws_bytes(KMAX);
         CU(cudaFuncSetAttribute(score_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mx));
-        CU(cudaFuncSetAttribute(exhaustive_generic_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mx));
-        CU(cudaFuncSetAttribute(exhaustive_generic_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mx));
+        CU(cudaFuncSetAttribute(exhaustive_generic_kernel<STORE_PLAIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mx));
+        CU(cudaFuncSetAttribute(exhaustive_generic_kernel<STORE_CLASSES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mx));
+        CU(cudaFuncSetAttribute(exhaustive_generic_kernel<STORE_COUNTS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mx));
         e->score_smem_set = KMAX;
     }
     return 0;
@@ -859,9 +876,10 @@ static int grid_tables(int n_priors, const double* gamma, const double* sharing_
 }
 
 // slot rows of the accumulator store: the five per-SNP slots + the scalars' slot, or (class-resolved) 3 c(c+1)/2 class slots
-// per SNP and as many rows as the scalars need (common.cuh)
-static size_t store_rows(bool classes, int kb, size_t upad) {
-    return classes ? (size_t)cls_nslot(kb) + (cls_nscal(kb) + upad - 1) / upad : (size_t)NSLOT;
+// per SNP and as many rows as the scalars need, the count table's among them (common.cuh)
+static size_t store_rows(StoreKind kind, int kb, size_t upad) {
+    const size_t nscal = cls_nscal(kb) + (kind == STORE_COUNTS ? cnt_ntab(kb) : 0);
+    return kind != STORE_PLAIN ? (size_t)cls_nslot(kb) + (nscal + upad - 1) / upad : (size_t)NSLOT;
 }
 
 static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pipsort_engine* e) {
@@ -904,7 +922,8 @@ static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pips
     e->U = U;
     e->K = lc->K; e->gamma = lc->gamma; e->p = lc->sharing_param;
     e->kb = std::min(KMAX, std::max(3, lc->max_causal));
-    e->classes = (flags & PIPSORT_PRIOR_CLASSES) != 0;
+    e->classes = (flags & (PIPSORT_PRIOR_CLASSES | PIPSORT_CAUSAL_COUNTS)) != 0;
+    e->exh.kind = (flags & PIPSORT_CAUSAL_COUNTS) ? STORE_COUNTS : e->classes ? STORE_CLASSES : STORE_PLAIN;
     e->use_reg_kernel = !(flags & PIPSORT_GENERIC_ONLY);
 
     TR(0);
@@ -944,7 +963,7 @@ static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pips
     {
         const size_t upad = (size_t)std::max((U + 3) & ~3, 4);
         size_t est = 64 * 256 + sizeof(LocusDev) + (size_t)(3 + 5 * U + NCOUNTER) * 8 + (size_t)(U + 2) * 8 +
-                     (store_rows(e->classes, e->kb, upad) * 16 * upad + NCOUNTER) * 8;
+                     (store_rows(e->exh.kind, e->kb, upad) * 16 * upad + NCOUNTER) * 8;
         est += ((size_t)e->sm_count * 12 + 256) * sizeof(int4) + 512;               // chunk descriptors of the exhaustive launch
         size_t nints = (size_t)6 * U + 2 * ((size_t)U / 32 + 8);
         for (int s = 0; s < S; s++) {
@@ -1151,7 +1170,7 @@ static int create_impl(const pipsort_locus* lc, int device, uint32_t flags, pips
     acc.NB = ((int)std::ceil(maxexp_bits) + acc.bias) / 512 + 2;
     acc.Upad = std::max((U + 3) & ~3, 4);
     acc.ccls = e->classes ? e->kb : 0;
-    e->bins_len = store_rows(e->classes, e->kb, acc.Upad) * acc.NB * acc.Upad + NCOUNTER;   // the counters ride in the tail of the store
+    e->bins_len = store_rows(e->exh.kind, e->kb, acc.Upad) * acc.NB * acc.Upad + NCOUNTER;   // the counters ride in the tail of the store
     if ((rc = dev_alloc(e, &acc.bins, e->bins_len))) return rc;
     acc.counters = acc.bins + (e->bins_len - NCOUNTER);
     if ((rc = dev_alloc(e, &e->d_res, 3 + (size_t)5 * U + NCOUNTER))) return rc;   // results | counters: one D2H per read
@@ -1360,8 +1379,10 @@ int pipsort_run_exhaustive(pipsort_engine* e, int c, uint64_t rank_begin, uint64
             const int chunk = (re - rb) >= (u64)e->sm_count * SCORE_WARPS * 64 ? 16 : 1;
             const u64 nchunks = (re - rb + chunk - 1) / chunk;
             const int blocks = (int)std::min<u64>((nchunks + SCORE_WARPS - 1) / SCORE_WARPS, (u64)e->sm_count * 8);
-            if (e->classes) exhaustive_generic_kernel<true><<<blocks, SCORE_WARPS * 32, smem, e->stream>>>(e->L, j, rb, re, chunk, wk);
-            else exhaustive_generic_kernel<false><<<blocks, SCORE_WARPS * 32, smem, e->stream>>>(e->L, j, rb, re, chunk, wk);
+            void (*kernel)(LocusDev, int, u64, u64, int, int) = e->exh.kind == STORE_PLAIN ? exhaustive_generic_kernel<STORE_PLAIN>
+                                                              : e->exh.kind == STORE_CLASSES ? exhaustive_generic_kernel<STORE_CLASSES>
+                                                                                             : exhaustive_generic_kernel<STORE_COUNTS>;
+            kernel<<<blocks, SCORE_WARPS * 32, smem, e->stream>>>(e->L, j, rb, re, chunk, wk);
             e->launches++;
             CU(cudaGetLastError());
             if (dominant && !e->capturing) { CU(cudaEventRecord(e->evk1, e->stream)); e->evk_valid = true; }
@@ -1689,7 +1710,7 @@ static int finalize_grid_launch(pipsort_engine* e, int n_priors, const double* p
                                 int tab_c = 0) {
     CU(cudaSetDevice(e->device));
     return launch_pdl(e, finalize_grid_kernel, mode == GRID_FULL ? finalize_blocks(e) : 1u, FIN_WARPS * 32, e->L.acc, e->U, n_priors,
-                      pri, e->L.neg_half_K, res, clear ? 1 : 0, (int)mode, tab_c);
+                      pri, e->L.neg_half_K, res, clear ? 1 : 0, (int)mode, tab_c, e->exh.kind == STORE_COUNTS ? 1 : 0);
 }
 
 static int finalize_launch(pipsort_engine* e, bool clear) {
@@ -1838,12 +1859,12 @@ static int grid_read_enqueue(pipsort_engine* e, int n_priors, const double* tab,
 }
 
 // first half of a table read (c <= the class limit): the table mode of the grid finalize, (c+1)(c+2)/2 + NCOUNTER doubles back
-// through the grid read's buffers, nothing uploaded
-static int table_read_enqueue(pipsort_engine* e, int c) {
-    const size_t ntab = cls_ntab(c), need = ntab + NCOUNTER;
+// through the grid read's buffers, nothing uploaded; counts: the count table, C(c+3, 3) + NCOUNTER doubles
+static int table_read_enqueue(pipsort_engine* e, int c, bool counts = false) {
+    const size_t ntab = counts ? cnt_ntab(c) : cls_ntab(c), need = ntab + NCOUNTER;
     int rc;
     if ((rc = grid_buffers(e, need))) return rc;
-    if ((rc = finalize_grid_launch(e, 0, nullptr, e->d_grid, false, GRID_TABLE, c))) return rc;
+    if ((rc = finalize_grid_launch(e, 0, nullptr, e->d_grid, false, counts ? GRID_COUNTS : GRID_TABLE, c))) return rc;
     CU(cudaMemcpyAsync(e->h_grid, e->d_grid, need * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
     e->h_read = e->h_grid;
     e->read_n = 1;
@@ -1858,6 +1879,18 @@ int pipsort_read_class_evidence(pipsort_engine* e, int c, double* table, uint64_
     if (c < 0 || c > e->kb) return fail(PIPSORT_E_ARG, "c=%d must be in [0, %d] (the engine's class limit)", c, e->kb);
     if (!table) return fail(PIPSORT_E_ARG, "null table");
     int rc = table_read_enqueue(e, c);
+    if (!rc) rc = read_complete(e, nullptr, table);
+    if (!rc && n_configs) *n_configs = e->last_read_count;
+    return rc;
+}
+
+int pipsort_read_count_table(pipsort_engine* e, int c, double* table, uint64_t* n_configs) {
+    if (!e) return fail(PIPSORT_E_ARG, "null engine");
+    if (e->exh.kind != STORE_COUNTS)
+        return fail(PIPSORT_E_ARG, "the engine was not created with PIPSORT_CAUSAL_COUNTS: its store has no count table");
+    if (c < 0 || c > e->kb) return fail(PIPSORT_E_ARG, "c=%d must be in [0, %d] (the engine's class limit)", c, e->kb);
+    if (!table) return fail(PIPSORT_E_ARG, "null table");
+    int rc = table_read_enqueue(e, c, true);
     if (!rc) rc = read_complete(e, nullptr, table);
     if (!rc && n_configs) *n_configs = e->last_read_count;
     return rc;
@@ -1895,8 +1928,9 @@ int pipsort_posterior_exhaustive(const pipsort_locus* locus, int device, uint32_
 
 // The grid read of a list of loci (pipsort_posterior_exhaustive_grid_batch): n priors whose tables are built once
 // (grid_tables); locus i reports into outs[i * n ..].  n == 0: the ordinary read, locus i into outs[i].  table_c >= 0: the table
-// read (pipsort_class_evidence_batch), locus i into tables[i * cls_ntab(table_c) ..].
-struct GridRead { int n; const double* tab; int table_c = -1; double* tables = nullptr; };
+// read (pipsort_class_evidence_batch), locus i into tables[i * cls_ntab(table_c) ..]; with counts, the count-table read
+// (pipsort_count_table_batch), locus i into tables[i * cnt_ntab(table_c) ..].
+struct GridRead { int n; const double* tab; int table_c = -1; double* tables = nullptr; bool counts = false; };
 
 // loci first, first + stride, first + 2 stride, ... through a software pipeline over DEPTH engines, each on its own stream:
 // while locus i is being evaluated the uploads and the preparation launches of the next one are already queued, and the
@@ -1911,6 +1945,7 @@ static int batch_worker(const pipsort_locus* loci, int32_t n_loci, int first, in
     int rc = 0;
     const bool table = grid.table_c >= 0;
     if (grid.n || table) flags |= PIPSORT_PRIOR_CLASSES;
+    if (grid.counts) flags |= PIPSORT_CAUSAL_COUNTS;
     auto finish = [&](int slot) -> int {       // results of the locus in pipeline slot `slot`: its read_n output blocks or its table
         pipsort_engine*& e = inflight[slot];
         const int i = idx_of[slot];
@@ -1934,7 +1969,7 @@ static int batch_worker(const pipsort_locus* loci, int32_t n_loci, int first, in
         uint64_t total = 0;
         rc = pipsort_total_ranks(e, c, &total);
         if (!rc) rc = pipsort_run_exhaustive(e, c, 0, total);
-        if (!rc) rc = table    ? table_read_enqueue(e, grid.table_c)
+        if (!rc) rc = table    ? table_read_enqueue(e, grid.table_c, grid.counts)
                       : grid.n ? grid_read_enqueue(e, grid.n, grid.tab, evidence_only(&outs[(size_t)i * grid.n], grid.n))
                                : read_enqueue(e);
     }
@@ -1996,6 +2031,52 @@ int pipsort_class_evidence_batch(const pipsort_locus* loci, int32_t n_loci, int 
     if (c < 0 || c > KMAX) return fail(PIPSORT_E_ARG, "c=%d must be in [0, %d]", c, KMAX);
     if (!n_loci) return 0;
     return batch_run(loci, n_loci, device, flags, c, GridRead{0, nullptr, c, tables}, nullptr, n_configs);
+}
+
+int pipsort_count_table_batch(const pipsort_locus* loci, int32_t n_loci, int device, uint32_t flags, int c, double* tables,
+                              uint64_t* n_configs) {
+    if (n_loci < 0 || (n_loci > 0 && (!loci || !tables))) return fail(PIPSORT_E_ARG, "bad argument");
+    if (c < 0 || c > KMAX) return fail(PIPSORT_E_ARG, "c=%d must be in [0, %d]", c, KMAX);
+    if (!n_loci) return 0;
+    return batch_run(loci, n_loci, device, flags, c, GridRead{0, nullptr, c, tables, true}, nullptr, n_configs);
+}
+
+// ---- the posterior of the causal counts (pipsort_count_posterior; host code, DESIGN.md section 5f) ------------------------------
+// class k = cnt_idx(J, a, b0) of locus i weighs pi'(J, a) exp(tab_ik); the posterior is that weight over the sum, computed from
+// the largest weighted class so that it neither overflows nor underflows, and total_i = U_i log(1-gamma) + log of the sum.
+int pipsort_count_posterior(int32_t n_loci, int c, const double* tables, const int32_t* union_count, double gamma,
+                            double sharing_param, double* post, double* log_evidence) {
+    if (n_loci < 1) return fail(PIPSORT_E_ARG, "n_loci=%d must be >= 1", n_loci);
+    if (c < 0 || c > KMAX) return fail(PIPSORT_E_ARG, "c=%d must be in [0, %d]", c, KMAX);
+    if (!tables || !union_count || !post) return fail(PIPSORT_E_ARG, "null argument");
+    if (!(gamma > 0.0 && gamma < 1.0)) return fail(PIPSORT_E_ARG, "gamma=%g must be in (0,1)", gamma);
+    if (!(sharing_param >= 0.0 && sharing_param <= 1.0)) return fail(PIPSORT_E_ARG, "sharing_param=%g must be in [0,1]", sharing_param);
+    const int ntab = cnt_ntab(c);
+    for (int i = 0; i < n_loci; i++) {
+        if (union_count[i] < 1) return fail(PIPSORT_E_ARG, "union_count[%d]=%d must be >= 1", i, union_count[i]);
+        for (int k = 0; k < ntab; k++) {
+            const double t = tables[(size_t)i * ntab + k];
+            if (std::isnan(t) || t == INFINITY) return fail(PIPSORT_E_ARG, "tables[%d][%d]=%g: a class value is finite or -inf", i, k, t);
+        }
+    }
+    double pi[KMAX + 1][KMAX + 1], lw[cnt_ntab(KMAX)];
+    prior_tables(gamma, sharing_param, 0, 0, pi, nullptr, nullptr);
+    for (int J = 0; J <= c; J++)
+        for (int a = 0; a <= J; a++)
+            for (int b0 = 0; a + b0 <= J; b0++) lw[cnt_idx(J, a, b0)] = std::log(pi[J][a]);
+    const double l1m = std::log(1.0 - gamma);
+    for (int i = 0; i < n_loci; i++) {
+        const double* t = tables + (size_t)i * ntab;
+        double* q = post + (size_t)i * ntab;
+        double m = -INFINITY, sum = 0.0;
+        for (int k = 0; k < ntab; k++) m = std::max(m, lw[k] + t[k]);
+        if (m == -INFINITY)
+            return fail(PIPSORT_E_ARG, "locus %d: every class has weight 0 or is empty under this prior: its posterior is undefined", i);
+        for (int k = 0; k < ntab; k++) sum += (q[k] = std::exp(lw[k] + t[k] - m));
+        for (int k = 0; k < ntab; k++) q[k] /= sum;
+        if (log_evidence) log_evidence[i] = union_count[i] * l1m + (m + std::log(sum));
+    }
+    return 0;
 }
 
 // ---- choosing the prior from class tables (pipsort_fit_prior; host code, DESIGN.md section 5f) ------------------------------

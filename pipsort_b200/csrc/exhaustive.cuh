@@ -18,6 +18,7 @@ struct ExhScratch {           // owned by the engine, reused across launches; th
     int4* d_chunks = nullptr;     // chunk descriptors of the plan on the device
     size_t cap_chunks = 0;
     unsigned* d_counter = nullptr;   // [0] work-queue head, [1] finished blocks (the kernel re-arms both)
+    StoreKind kind = STORE_PLAIN; // the engine's store: which instantiation of exhaustive_all_kernel runs
     int occ = 0;                  // resident blocks per SM of exhaustive_all_kernel
     char* pin_stage = nullptr;    // pinned staging slice for the FIRST descriptor upload (later ones may overlap an in-flight copy)
     size_t pin_stage_cap = 0;
@@ -29,6 +30,11 @@ struct ExhScratch {           // owned by the engine, reused across launches; th
     ExhAll plan;
     int plan_blocks = 0;
 };
+
+inline auto exh_kernel(StoreKind k) {
+    return k == STORE_PLAIN ? exhaustive_all_kernel<STORE_PLAIN> : k == STORE_CLASSES ? exhaustive_all_kernel<STORE_CLASSES>
+                                                                                      : exhaustive_all_kernel<STORE_COUNTS>;
+}
 
 inline u64 exh_binom(int n, int k) {
     if (k < 0 || k > n) return 0;
@@ -174,18 +180,18 @@ inline int exhaustive_plan(const LocusDev& L, int c, u64 rank_begin, u64 rank_en
                            const ExhCostModel* M) {
     const int U = L.U;
     cudaError_t err;
-    // the instantiation that matches the engine's store (class-resolved: PIPSORT_PRIOR_CLASSES)
-    const bool cr = L.acc.ccls > 0;
+    // the instantiation that matches the engine's store
+    const StoreKind k = sc->kind;
     if (!sc->occ) {
-        void (*kernel)(LocusDev, ExhAll, const LocusDev*) = cr ? exhaustive_all_kernel<true> : exhaustive_all_kernel<false>;
-        const size_t smem = cr ? EXH_SMEM_BYTES_CR : EXH_SMEM_BYTES;
+        void (*kernel)(LocusDev, ExhAll, const LocusDev*) = exh_kernel(k);
+        const size_t smem = exh_smem_bytes(k);
         // (the attribute is per device: set it for every engine, not once per process)
         if ((err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return (int)err;
-        static int occ_cache[2] = {0, 0};    // a property of the kernel and the device generation: query once per process
+        static int occ_cache[3] = {0, 0, 0};    // a property of the kernel and the device generation: query once per process
         static std::mutex occ_mutex;
         std::lock_guard<std::mutex> g(occ_mutex);
-        if (!occ_cache[cr] && (err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_cache[cr], kernel, EXH_WARPS * 32, smem)) != cudaSuccess) return (int)err;
-        sc->occ = occ_cache[cr];
+        if (!occ_cache[k] && (err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_cache[k], kernel, EXH_WARPS * 32, smem)) != cudaSuccess) return (int)err;
+        sc->occ = occ_cache[k];
     }
     const double forced = [] { const char* v = getenv("PIPSORT_EXH_CHUNK"); return v ? atof(v) : 0.0; }();   // experiments / tests
     if (sc->plan_valid && !(forced > 0.0) && sc->plan_c == c && sc->plan_rb == rank_begin && sc->plan_re == rank_end) return 0;
@@ -246,10 +252,8 @@ inline int exhaustive_launch(const LocusDev& L, const LocusDev* Lg, cudaStream_t
     }
     sc->plan_valid = true;
     if (sc->plan.n_total == 0) return 0;
-    const bool cr = L.acc.ccls > 0;
     if (ev0 && (err = cudaEventRecord(ev0, stream)) != cudaSuccess) return (int)err;
-    if (cr) exhaustive_all_kernel<true><<<sc->plan_blocks, EXH_WARPS * 32, EXH_SMEM_BYTES_CR, stream>>>(L, sc->plan, Lg);
-    else exhaustive_all_kernel<false><<<sc->plan_blocks, EXH_WARPS * 32, EXH_SMEM_BYTES, stream>>>(L, sc->plan, Lg);
+    exh_kernel(sc->kind)<<<sc->plan_blocks, EXH_WARPS * 32, exh_smem_bytes(sc->kind), stream>>>(L, sc->plan, Lg);
     if (ev1 && (err = cudaEventRecord(ev1, stream)) != cudaSuccess) return (int)err;
     (*launches)++;
     return (int)cudaGetLastError();

@@ -102,10 +102,12 @@ __device__ __forceinline__ int pow3(int k) {
 
 // Scores the configuration whose internal union indices are in ws.g[0..k).  Warp-collective.
 // Returns (on every lane) the expansion value l with the largest |l|, 0.0 if there is none.
-// CR: class-resolved store (PIPSORT_PRIOR_CLASSES, common.cuh): the cells are kept per a' = a - [t == 2] instead of being
-// weighted with L.pi[k][a], and go unweighted to their (k, t, a') slots; the total per a, the no-causal sums per class
-template <bool CR = false>
+// SK != STORE_PLAIN: class-resolved store (PIPSORT_PRIOR_CLASSES, common.cuh): the cells are kept per a' = a - [t == 2]
+// instead of being weighted with L.pi[k][a], and go unweighted to their (k, t, a') slots; the total per a, the no-causal sums
+// per class.  STORE_COUNTS: the total also per (a, b0), b0 = popcount(m0) - a, into the count table.
+template <StoreKind SK = STORE_PLAIN>
 __device__ inline double score_config(const LocusDev& L, const WarpWS& ws, int k, bool upd, int lane) {
+    constexpr bool CR = SK != STORE_PLAIN;
     const AccDev& acc = L.acc;
     if (k == 0) {  // postcal.cpp:793-822, sss_postcal.cpp:463-499
         if (upd && lane == 0) {
@@ -114,6 +116,7 @@ __device__ inline double score_config(const LocusDev& L, const WarpWS& ws, int k
                 scal_add(acc, cls_T(0, 0), einv, 0);
                 scal_add(acc, cls_N(acc.ccls, 0, 0), einv, 0);
                 scal_add(acc, cls_N(acc.ccls, 1, 0), einv, 0);
+                if (SK == STORE_COUNTS) scal_add(acc, cls_R(acc.ccls, 0, 0, 0), einv, 0);
             } else {
                 bin_add(acc, SCAL, S_TOTAL, einv, 0);
                 bin_add(acc, SCAL, S_NC0, einv, 0);
@@ -264,6 +267,25 @@ __device__ inline double score_config(const LocusDev& L, const WarpWS& ws, int k
                         if (i == 0) scal_add(acc, cls_T(k, q + (t == 2 ? 1 : 0)), v, nr);
                     }
                 }
+                if (SK == STORE_COUNTS && i == 0) {   // the same expansions by class (a, b0)
+                    // sr[a (2k + 3 - a) / 2 + b0]: the classes of size k, each with its own exponent (a class may lie far below
+                    // the cell's reference nr, where a plain sum relative to it would flush its terms)
+                    XAcc sr[cls_ntab(KMAX)];
+                    const int nl = cls_ntab(k);
+                    for (int q = 0; q < nl; q++) sr[q] = xacc_empty();
+                    for (int ep = lane; ep < n3m; ep += 32) {
+                        const int hi = ep / p3i, lo = ep - hi * p3i;
+                        const uint32_t pk = tab[(hi * 3 + t) * p3i + lo];
+                        const int m0 = pk & 255, m1 = (pk >> 8) & 255, a = pk >> 16;
+                        const double v0 = em0[m0], v1 = em1[m1];
+                        if (v0 == 0.0 || v1 == 0.0) continue;
+                        xadd(sr[a * (2 * k + 3 - a) / 2 + __popc(m0) - a], v0 * v1, en0[m0] + en1[m1]);
+                    }
+                    for (int q = 0; q < nl; q++) {
+                        const XAcc v = xwarp_sum(sr[q]);
+                        if (lane == 0) scal_add(acc, cls_R(acc.ccls, k, 0, 0) + q, v.M, v.N);
+                    }
+                }
                 continue;
             }
             double sx = 0.0, sy = 0.0;
@@ -342,8 +364,8 @@ score_batch_kernel(LocusDev L, const int* __restrict__ idx, long long n, int kma
 
 // Exhaustive enumeration of the j-subsets with in-class ranks [r_begin, r_end) (internal SNP order):
 // every warp takes chunks of `chunk` consecutive ranks, unranks the first and walks the rest.
-// CR: the class-resolved store (PIPSORT_PRIOR_CLASSES); the engine launches the instantiation that matches its store.
-template <bool CR>
+// SK: the engine's store (StoreKind, common.cuh); the engine launches the instantiation that matches it.
+template <StoreKind SK>
 __global__ void __launch_bounds__(SCORE_WARPS * 32)
 exhaustive_generic_kernel(LocusDev L, int j, u64 r_begin, u64 r_end, int chunk, int ws_kmax) {
     extern __shared__ __align__(16) unsigned char smem[];
@@ -357,7 +379,7 @@ exhaustive_generic_kernel(LocusDev L, int j, u64 r_begin, u64 r_end, int chunk, 
         if (lane == 0) unrank_subset(lo, L.U, j, ws.g);
         __syncwarp();
         for (u64 r = lo; r < hi; r++) {
-            score_config<CR>(L, ws, j, true, lane);
+            score_config<SK>(L, ws, j, true, lane);
             __syncwarp();
             if (lane == 0) next_subset(L.U, j, ws.g);
             __syncwarp();

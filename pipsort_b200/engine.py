@@ -21,6 +21,7 @@ KEEP_ORDER = 1
 GENERIC_ONLY = 2
 RAW_LD = 4
 PRIOR_CLASSES = 8
+CAUSAL_COUNTS = 16
 IPC_HANDLE_BYTES = 64
 KMAX = 8
 
@@ -78,6 +79,11 @@ def lib():
         L.pipsort_read_class_evidence.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(u64)]
         L.pipsort_class_evidence_batch.argtypes = [C.POINTER(_LocusV), C.c_int32, i32, C.c_uint32, i32, C.POINTER(C.c_double),
                                                    C.POINTER(u64)]
+        L.pipsort_read_count_table.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(u64)]
+        L.pipsort_count_table_batch.argtypes = [C.POINTER(_LocusV), C.c_int32, i32, C.c_uint32, i32, C.POINTER(C.c_double),
+                                                C.POINTER(u64)]
+        L.pipsort_count_posterior.argtypes = [C.c_int32, i32, C.POINTER(C.c_double), C.POINTER(C.c_int32), C.c_double,
+                                              C.c_double, C.POINTER(C.c_double), C.POINTER(C.c_double)]
         L.pipsort_fit_prior.argtypes = [C.c_int32, i32, C.POINTER(C.c_double), C.POINTER(C.c_int32), C.c_uint32,
                                         C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_double)]
         L.pipsort_destroy.argtypes = [vp]
@@ -173,7 +179,7 @@ class Engine:
     """Device-resident locus + accumulators (the hot-path half of the reference's PostCal)."""
 
     def __init__(self, num_snps, sigma, z, d, K, snp_map, gamma=0.01, sharing_param=0.75, max_causal=3, device=0,
-                 keep_order=False, generic_only=False, raw_ld=False, prior_classes=False):
+                 keep_order=False, generic_only=False, raw_ld=False, prior_classes=False, causal_counts=False):
         self.num_snps = np.ascontiguousarray(num_snps, dtype=np.int32)
         if isinstance(sigma, (list, tuple)):
             sigma = np.concatenate([np.asarray(s, dtype=np.float64).ravel() for s in sigma])
@@ -193,7 +199,8 @@ class Engine:
                      int(max_causal))
         self._h = C.c_void_p()
         _check(lib().pipsort_create(C.byref(loc), int(device), (KEEP_ORDER if keep_order else 0) | (GENERIC_ONLY if generic_only else 0) |
-                                    (RAW_LD if raw_ld else 0) | (PRIOR_CLASSES if prior_classes else 0), C.byref(self._h)))
+                                    (RAW_LD if raw_ld else 0) | (PRIOR_CLASSES if prior_classes else 0) |
+                                    (CAUSAL_COUNTS if causal_counts else 0), C.byref(self._h)))
         self.max_causal = int(max_causal)
         self.device = int(device)
 
@@ -334,6 +341,15 @@ class Engine:
         _check(lib().pipsort_read_class_evidence(self._h, int(c), _dp(tab), None))
         return tab
 
+    def read_count_table(self, c):
+        """The count table of the store (an engine created with causal_counts=True; pipsort_read_count_table): ndarray
+        [C(c+3, 3)], entry cnt_idx(J, a, b0) = J(J+1)(J+2)/6 + a(2J+3-a)/2 + b0 = -K/2 + log R[a][b0][b1] (a SNPs causal in
+        both studies, b0 in study 0 only, b1 = J - a - b0 in study 1 only), -inf for an empty class.  count_posterior takes
+        it; class_tables_from_counts turns it into read_class_evidence's table."""
+        tab = np.empty(_ncnt(c))
+        _check(lib().pipsort_read_count_table(self._h, int(c), _dp(tab), None))
+        return tab
+
     def finalize(self, reset=False):
         """Bins -> log-space results on the device; reset=True also leaves the accumulators empty (no reset() needed before
         the next pass; fetch() then returns the results)."""
@@ -472,6 +488,16 @@ def _ntab(c):
     return max(0, (int(c) + 1) * (int(c) + 2) // 2)
 
 
+def _ncnt(c):
+    """Entries of a count table up to class limit c: C(c+3, 3) (0 for a c the engine refuses)."""
+    return max(0, (int(c) + 1) * (int(c) + 2) * (int(c) + 3) // 6)
+
+
+def _cnt_classes(c):
+    """(J, a, b0, b1) of every entry of a count table up to c, in table order."""
+    return [(J, a, b0, J - a - b0) for J in range(c + 1) for a in range(J + 1) for b0 in range(J - a + 1)]
+
+
 def _prior_arrays(priors):
     pr = np.asarray(priors, dtype=np.float64).reshape(-1, 2) if len(priors) else np.zeros((0, 2))
     return np.ascontiguousarray(pr[:, 0]), np.ascontiguousarray(pr[:, 1])
@@ -555,13 +581,18 @@ class LocusBatch:
     prior (results() gives a list of Results per locus); evidence_only=True leaves every per-SNP member NULL (the evidence
     read) and the buffer holds (total, noCausal[0], noCausal[1]) per locus and prior, read with evidence().
     class_evidence=True: run() is pipsort_class_evidence_batch, the buffer holds every locus's class table
-    ((c+1)(c+2)/2 doubles, Engine.read_class_evidence's layout), read with tables()."""
+    ((c+1)(c+2)/2 doubles, Engine.read_class_evidence's layout), read with tables().
+    count_table=True: run() is pipsort_count_table_batch, the buffer holds every locus's count table (C(c+3, 3) doubles,
+    Engine.read_count_table's layout), read with tables()."""
 
-    def __init__(self, loci, c, device=0, raw_ld=False, priors=None, evidence_only=False, class_evidence=False):
+    def __init__(self, loci, c, device=0, raw_ld=False, priors=None, evidence_only=False, class_evidence=False,
+                 count_table=False):
         if evidence_only and priors is None:
             raise ValueError("evidence_only needs priors")
-        if class_evidence and priors is not None:
-            raise ValueError("class_evidence takes no priors")
+        if (class_evidence or count_table) and priors is not None:
+            raise ValueError("class_evidence and count_table take no priors")
+        if class_evidence and count_table:
+            raise ValueError("one table read per batch: class_evidence or count_table")
         n = self.n = len(loci)
         self.c, self.device, self.flags = int(c), int(device), RAW_LD if raw_ld else 0
         f64, i32 = np.dtype(np.float64), np.dtype(np.int32)
@@ -586,9 +617,11 @@ class LocusBatch:
         self.priors = None if priors is None else _prior_arrays(priors)
         self.evidence_only = bool(evidence_only)
         self.class_evidence = bool(class_evidence)
+        self.count_table = bool(count_table)
+        self.ntab = _ncnt(self.c) if count_table else _ntab(self.c)
         k = self.k = 1 if priors is None else len(self.priors[0])      # result blocks per locus: locus i, prior j -> i * k + j
-        if class_evidence:
-            buf = self.buf = np.empty(n * _ntab(self.c))
+        if class_evidence or count_table:
+            buf = self.buf = np.empty(n * self.ntab)
             oa = self.oa = np.zeros(0, dtype=_OUT_DT)
         elif evidence_only:
             buf = self.buf = np.empty(n * k * 3)
@@ -613,7 +646,7 @@ class LocusBatch:
         self.cnt = np.zeros(n, dtype=np.uint64)
         lp, op = C.cast(la.ctypes.data, C.POINTER(_LocusV)), C.cast(oa.ctypes.data, C.POINTER(_OutputsV))
         cp = C.cast(self.cnt.ctypes.data, C.POINTER(C.c_uint64))
-        if class_evidence:
+        if class_evidence or count_table:
             self._args = (lp, n, self.device, self.flags, self.c, _dp(buf), cp)
         elif priors is None:
             self._args = (lp, n, self.device, self.flags, self.c, op, cp)
@@ -626,6 +659,8 @@ class LocusBatch:
         buffers out."""
         if self.class_evidence:
             _check(lib().pipsort_class_evidence_batch(*self._args))
+        elif self.count_table:
+            _check(lib().pipsort_count_table_batch(*self._args))
         elif self.priors is not None:       # the priors are validated even for an empty list
             _check(lib().pipsort_posterior_exhaustive_grid_batch(*self._args))
         elif self.n:
@@ -634,8 +669,8 @@ class LocusBatch:
 
     def results(self):
         """A Results per locus; with priors, a list of Results (one per prior) per locus."""
-        if self.evidence_only or self.class_evidence:
-            raise ValueError("an evidence-only or class-evidence batch has no per-SNP results: use evidence() / tables()")
+        if self.evidence_only or self.class_evidence or self.count_table:
+            raise ValueError("an evidence-only or table batch has no per-SNP results: use evidence() / tables()")
         out, buf, k = [], self.buf, self.k
         offl, Nl, Sl, Ul, cl = self.off.tolist(), self.N.tolist(), self.S.tolist(), self.U.tolist(), self.cnt.tolist()
         for i in range(self.n):
@@ -660,10 +695,11 @@ class LocusBatch:
         return np.stack([self.buf[o], self.buf[nc], self.buf[nc + 1]], axis=-1).reshape(self.n, self.k, 3)
 
     def tables(self):
-        """ndarray [n_loci, (c+1)(c+2)/2] of class tables (a class_evidence batch)."""
-        if not self.class_evidence:
-            raise ValueError("tables() needs a class_evidence batch")
-        return self.buf.reshape(self.n, _ntab(self.c)).copy()
+        """ndarray [n_loci, (c+1)(c+2)/2] of class tables (a class_evidence batch) or [n_loci, C(c+3, 3)] of count tables
+        (a count_table batch)."""
+        if not (self.class_evidence or self.count_table):
+            raise ValueError("tables() needs a class_evidence or count_table batch")
+        return self.buf.reshape(self.n, self.ntab).copy()
 
 
 def posterior_exhaustive_batch(loci, c, device=0, raw_ld=False):
@@ -685,6 +721,70 @@ def class_evidence_batch(loci, c, device=0, raw_ld=False):
     """The class table of every locus (pipsort_class_evidence_batch): one class-resolved pass per locus, pipelined as
     posterior_exhaustive_batch.  loci as posterior_exhaustive_batch takes them; returns ndarray [n_loci, (c+1)(c+2)/2]."""
     return LocusBatch(loci, c, device, raw_ld, class_evidence=True).run().tables()
+
+
+def count_table_batch(loci, c, device=0, raw_ld=False):
+    """The count table of every locus (pipsort_count_table_batch): one pass per locus on a store with the count table,
+    pipelined as posterior_exhaustive_batch.  loci as posterior_exhaustive_batch takes them; returns ndarray
+    [n_loci, C(c+3, 3)] (Engine.read_count_table's layout)."""
+    return LocusBatch(loci, c, device, raw_ld, count_table=True).run().tables()
+
+
+def _count_c(w):
+    c = next((k for k in range(KMAX + 1) if _ncnt(k) == w), -1)
+    if c < 0:
+        raise ValueError(f"a count table has C(c+3, 3) entries for some c in [0, {KMAX}], not {w}")
+    return c
+
+
+def count_posterior(tables, union_counts, gamma, p):
+    """The posterior of the numbers of causal SNPs under the prior (gamma, p), per locus (pipsort_count_posterior, host
+    code, no device).  tables: [n_loci, C(c+3, 3)] from count_table_batch or Engine.read_count_table; union_counts: U per
+    locus.  Returns (post, log_evidence): post[i, a, b0, b1] is the posterior probability that locus i has a SNPs causal in
+    both studies, b0 in study 0 only and b1 in study 1 only (zero outside a + b0 + b1 <= c), an ndarray of shape
+    (n, c+1, c+1, c+1); log_evidence[i] is the locus's log evidence at that prior (the grid read's total).  The marginals:
+      P(a >= 1)  = 1 - post[i, 0].sum()                     -- at least one causal SNP shared by the two studies;
+      P(k0 = n)  = sum over a + b0 = n of post[i, a, b0, :]  -- n causal SNPs in study 0 (k0 = a + b0);
+      P(k1 = n)  = sum over a + b1 = n of post[i, a, :, b1]  -- the same for study 1 (k1 = a + b1)."""
+    tab = np.ascontiguousarray(tables, dtype=np.float64)
+    if tab.ndim != 2:
+        raise ValueError("tables must be [n_loci, C(c+3, 3)]")
+    n, w = tab.shape
+    c = _count_c(w)
+    U = np.ascontiguousarray(union_counts, dtype=np.int32).ravel()
+    if U.size != n:
+        raise ValueError("one union count per locus")
+    flat, ev = np.empty((n, w)), np.empty(n)
+    _check(lib().pipsort_count_posterior(n, c, _dp(tab), U.ctypes.data_as(C.POINTER(C.c_int32)), float(gamma), float(p),
+                                         _dp(flat), _dp(ev)))
+    post = np.zeros((n, c + 1, c + 1, c + 1))
+    cls = np.array(_cnt_classes(c))
+    post[:, cls[:, 1], cls[:, 2], cls[:, 3]] = flat
+    return post, ev
+
+
+def class_tables_from_counts(tables, c=None):
+    """Class tables ([n_loci, (c+1)(c+2)/2], Engine.read_class_evidence's layout) from count tables ([n_loci, C(c+3, 3)]): a
+    log-sum-exp over b0 per class (J, a), so that one count_table_batch also feeds fit_prior.  c (optional) must match the
+    tables' width."""
+    tab = np.asarray(tables, dtype=np.float64)
+    one = tab.ndim == 1
+    tab = tab.reshape(1, -1) if one else tab
+    cw = _count_c(tab.shape[1])
+    if c is not None and int(c) != cw:
+        raise ValueError(f"count tables of width {tab.shape[1]} are for c={cw}, not {c}")
+    out = np.empty((tab.shape[0], _ntab(cw)))
+    k = 0
+    for J in range(cw + 1):
+        for a in range(J + 1):
+            part = tab[:, k:k + J - a + 1]
+            m = part.max(axis=1)
+            safe = np.where(np.isneginf(m), 0.0, m)
+            with np.errstate(divide="ignore"):
+                out[:, J * (J + 1) // 2 + a] = np.where(np.isneginf(m), -np.inf,
+                                                        safe + np.log(np.exp(part - safe[:, None]).sum(axis=1)))
+            k += J - a + 1
+    return out[0] if one else out
 
 
 _FIT = {"gamma": 1, "p": 2, "gamma,p": 3}

@@ -2,7 +2,8 @@
 finds the innermost loops that hold the MUFU.RSQ64H of the bordered step and prints, per loop, the instruction count, the
 sum of the stall counts the compiler encoded (= issue cycles of ONE warp running alone, scoreboard waits excluded), the
 opcode mix and the local-memory traffic (spills).   python scripts/sass_loop.py [-DEXH_...=...] [--dump file] [--classes]
-(--classes: the instantiation for the class-resolved store of PIPSORT_PRIOR_CLASSES instead of the default one)"""
+(--classes: the instantiation for the class-resolved store of PIPSORT_PRIOR_CLASSES instead of the default one; --counts: the one
+for the store with the count table of PIPSORT_CAUSAL_COUNTS)"""
 import os, re, subprocess, sys, tempfile
 from collections import Counter
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -56,8 +57,8 @@ def main():
         print(l.strip())
     fns = parse(out)
     os.unlink(out)
-    tag = "ILb1E" if "--classes" in sys.argv else "ILb0E"
-    name = [k for k in fns if "exhaustive_all_kernel" in k and tag in k][0]
+    kind = 2 if "--counts" in sys.argv else (1 if "--classes" in sys.argv else 0)   # StoreKind (common.cuh)
+    name = [k for k in fns if "exhaustive_all_kernel" in k and re.search(r"StoreKindE%dE" % kind, k)][0]
     ins = fns[name]
     print("kernel instructions:", len(ins))
     loops = []
