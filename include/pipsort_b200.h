@@ -180,6 +180,22 @@ int pipsort_sss_sharded(pipsort_engine* e, int max_causal, int max_iterations, i
 /* Forget the explored configurations (pipsort_sss does this itself when it starts). */
 int pipsort_sss_reset(pipsort_engine* e);
 
+/* The shotgun search for a list of loci (the -q 1 loop of a fine-mapping run): for every locus what pipsort_create +
+ * pipsort_sss + pipsort_read_accumulators + pipsort_destroy do -- the same trajectory, draws and results.  Locus i goes to
+ * outs[i]; iterations[i], stop_reasons[i] (as pipsort_sss reports them) and n_configs[i] (the configuration count) are
+ * optional.  Each locus's engine is created from loci[i] as given (its max_causal must admit max_causal, as for pipsort_sss).
+ * Host threads as pipsort_posterior_exhaustive_batch (PIPSORT_BATCH_THREADS, default 3; lists of fewer than 8 loci: one),
+ * loci dealt round robin; each thread keeps up to 2 searches in flight, each on its own engine and stream, and advances
+ * them in turn: it waits for one search's round, draws its next state and enqueues its next round, then moves to the next
+ * search.  A search is mostly host work and latency between short launches, so the searches overlap one another's waits.
+ * Refused before any device work: PIPSORT_E_ARG for a null loci / outs with n_loci > 0, n_loci < 0, max_causal outside
+ * [0, 8], max_iterations < 0, flags with PIPSORT_PRIOR_CLASSES or PIPSORT_CAUSAL_COUNTS; a locus at sharing_param = 1 with
+ * max_causal > 0 (PIPSORT_E_ARG) or with more union SNPs than the search state holds (PIPSORT_E_RANGE), the message naming
+ * the locus ("locus 17: ...").  n_loci == 0 returns 0.  An error found during a search (a singular block, a range overflow)
+ * stops the call as pipsort_posterior_exhaustive_batch does: every engine in flight is released.                      */
+int pipsort_sss_batch(const pipsort_locus* loci, int32_t n_loci, int device, uint32_t flags, int max_causal, int max_iterations,
+                      const pipsort_outputs* outs, int32_t* iterations, int32_t* stop_reasons, uint64_t* n_configs);
+
 /* Reads the accumulators into PostCal's result arrays (any member of `out` may be NULL).  Replaces the
  * reads of totalLikeLihoodLOG / postValues / noCausal / sharedPips / sharedLL / notSharedLL by
  * findOptimalSetGreedy (postcal.cpp:1144-1163) and printPost2File (postcal.h:288-336).            */

@@ -10,6 +10,7 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <functional>
 #include <mutex>
 #include <numeric>
 #include <random>
@@ -429,6 +430,7 @@ struct pipsort_engine {
     cudaStream_t stream = nullptr, own_stream = nullptr;
     char* l2_scratch = nullptr;
     size_t cap_l2 = 0;
+    // ev_up: the end of pipsort_create's uploads, later the end of each round of the shotgun search (sss_round_enqueue)
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, evk0 = nullptr, evk1 = nullptr, ev_up = nullptr;
     bool evk_valid = false;
     LocusDev L, L_host_copy;
@@ -470,7 +472,8 @@ struct pipsort_engine {
         u64 count = 0;              // entries in the table
         double* d_out_l = nullptr; int* d_batch = nullptr; unsigned char* d_upd = nullptr; int* d_counter = nullptr;
         double* d_scored = nullptr; unsigned char* d_state = nullptr; int* d_pos_of = nullptr; double* d_total = nullptr;
-        double* h_out_l = nullptr;  // pinned: [n_max] neighbour values, [n_max + 1] the running total
+        // pinned: [n_max] neighbour values, [n_max + 1] the running total, [n_max + 2] the round's two int counters
+        double* h_out_l = nullptr;
         size_t cap_out_l = 0, cap_batch = 0, cap_upd = 0, cap_counter = 0, cap_scored = 0, cap_state = 0, cap_pos_of = 0,
                cap_total = 0, cap_h_out_l = 0;
     } sss;
@@ -1529,120 +1532,178 @@ int pipsort_sss_reset(pipsort_engine* e) {
     return 0;
 }
 
+// What a locus must satisfy for the search at max_causal c, known before any engine exists (pipsort_sss_batch checks every
+// locus of a list with it before its first engine).
+static int sss_locus_check(int U, double p, int c) {
+    if (U > SSS_MAX_U) return fail(PIPSORT_E_RANGE, "the search state packs union indices into 15 bits: U=%d > %d", U, SSS_MAX_U);
+    // at p = 1 every non-empty configuration has an expansion of prior 0, so its largest-|l| value is -inf: the draws
+    // would weigh a group by nan (the reference then reads past its neighbourhood list)
+    if (c > 0 && p == 1.0)
+        return fail(PIPSORT_E_ARG, "the shotgun search is undefined at sharing_param = 1 (every neighbour scores -inf)");
+    return 0;
+}
+
+// One search in flight: what sss_postcal.cpp:102-380 keeps across rounds.  A search is sss_begin, then rounds of
+// sss_round_enqueue (kernels and read-back copies on the engine's stream, does not block) and sss_round_complete (waits for
+// them, stopping rules, draws, next state) until `more` is false.  pipsort_sss runs one search so; pipsort_sss_batch keeps
+// several in flight on one host thread, so that one search's host work overlaps the other searches' kernels.
+struct SssRun {
+    std::mt19937 gen{12345};                                             // sss_postcal.cpp:138
+    SssCur cur;                                                          // causal_locs starts empty (:115)
+    int c = 0, max_iterations = 0, conv_from = 99, world = 1, rank = 0;
+    long long n_max = 0;
+    long long nz = 0, nm = 0, n = 0;                                     // this round's group bounds and neighbourhood size
+    double old_sum_lkl = 0, sss_sum_lkl = 0;
+    int iter = 0, why = 0;
+    bool more = false;                                                   // another round is to be enqueued
+    std::vector<double> probs;
+};
+
 // The search on this engine alone (sharded = false) or in lockstep with the ranks of its p2p group, each scoring its share
-// of every round's unseen neighbours (sss.cuh).  With one rank no mailbox is touched.
-static int sss_run(pipsort_engine* e, int c, int max_iterations, int32_t* iterations, int32_t* stop_reason, bool sharded) {
+// of every round's unseen neighbours (sss.cuh).  With one rank no mailbox is touched.  Validates, sizes the per-round
+// buffers, forgets the explored configurations and sets up r for round 0.
+static int sss_begin(pipsort_engine* e, int c, int max_iterations, bool sharded, SssRun* r) {
     if (!e) return fail(PIPSORT_E_ARG, "null engine");
     if (e->classes) return fail(PIPSORT_E_ARG, "%s", CLASSES_NO_SSS);
     pipsort_engine::P2P& pp = e->p2p;
     if (sharded && !pp.connected) return fail(PIPSORT_E_ARG, "pipsort_p2p_connect has not been called");
-    const int U = e->U, world = sharded ? pp.world : 1, rank = sharded ? pp.rank : 0;
+    const int U = e->U, world = sharded ? pp.world : 1;
     if (c < 0 || c > e->kb) return fail(PIPSORT_E_ARG, "max_causal=%d outside [0,%d] (max_causal given at create)", c, e->kb);
-    if (U > SSS_MAX_U) return fail(PIPSORT_E_RANGE, "the search state packs union indices into 15 bits: U=%d > %d", U, SSS_MAX_U);
+    int rc = sss_locus_check(U, e->p, c);
+    if (rc) return rc;
     if (max_iterations < 0) return fail(PIPSORT_E_ARG, "negative iteration count");
-    // at p = 1 every non-empty configuration has an expansion of prior 0, so its largest-|l| value is -inf: the draws
-    // would weigh a group by nan (the reference then reads past its neighbourhood list)
-    if (c > 0 && e->p == 1.0)
-        return fail(PIPSORT_E_ARG, "the shotgun search is undefined at sharing_param = 1 (every neighbour scores -inf)");
     CU(cudaSetDevice(e->device));
     pipsort_engine::Sss& q = e->sss;
     const int kmax = std::max(c, 1);
     const long long n_max = (long long)U * std::max(c, 1) + c + U + 1;
     const size_t m = (size_t)n_max + 1;
-    int rc;
     if ((rc = grow(e, &q.d_out_l, &q.cap_out_l, m)) || (rc = grow(e, &q.d_batch, &q.cap_batch, m * kmax)) ||
         (rc = grow(e, &q.d_upd, &q.cap_upd, m)) || (rc = grow(e, &q.d_counter, &q.cap_counter, 2)) ||
         (rc = grow(e, &q.d_scored, &q.cap_scored, m)) || (rc = grow(e, &q.d_state, &q.cap_state, m)) ||
         (rc = grow(e, &q.d_pos_of, &q.cap_pos_of, m)) || (rc = grow(e, &q.d_total, &q.cap_total, 1)) ||
-        (rc = grow(e, &q.h_out_l, &q.cap_h_out_l, m + 1, Mem::pinned)) || (rc = pipsort_sss_reset(e)))
+        (rc = grow(e, &q.h_out_l, &q.cap_h_out_l, m + 2, Mem::pinned)) || (rc = pipsort_sss_reset(e)))
         return rc;
-    const size_t acc_len = p2p_acc_len(e), half = p2p_sss_half(e), stride = p2p_slot_len(e);
-    if (world > 1 && (size_t)n_max + (size_t)e->L.acc.NB > half) return fail(PIPSORT_E_ARG, "mailbox too small for this max_causal");
+    if (world > 1 && (size_t)n_max + (size_t)e->L.acc.NB > p2p_sss_half(e)) return fail(PIPSORT_E_ARG, "mailbox too small for this max_causal");
+    memset(&r->cur, 0, sizeof r->cur);
+    r->c = c; r->max_iterations = max_iterations; r->conv_from = sss_conv_from();
+    r->world = world; r->rank = sharded ? pp.rank : 0;
+    r->n_max = n_max;
+    r->more = max_iterations > 0;
+    return 0;
+}
+
+// where a round's counters land on the host (pinned, so that their copy does not block the host as a pageable one would)
+static int* sss_host_counters(pipsort_engine* e, const SssRun* r) { return reinterpret_cast<int*>(e->sss.h_out_l + r->n_max + 2); }
+
+// Round r->iter: lookup, scoring, exchange, insert and running total on the engine's stream, then the asynchronous copies of
+// the counters, the neighbours' values and the running total into pinned memory, then the round's event.  Does not block.
+static int sss_round_enqueue(pipsort_engine* e, SssRun* r) {
+    pipsort_engine::Sss& q = e->sss;
+    pipsort_engine::P2P& pp = e->p2p;
+    const int U = e->U, c = r->c, kmax = std::max(c, 1), world = r->world, rank = r->rank;
+    const long long n_max = r->n_max;
+    long long np;
+    sss_nbd_sizes(U, r->cur.k, c, r->nz, r->nm, np);
+    const long long n = r->n = r->nz + r->nm + np;
+    int rc;
+    if ((rc = sss_table_reserve(e, q.count + (u64)n))) return rc;
     double* errf = e->L.acc.counters + 1 + ERR_P2P_TIMEOUT;
-
-    const int conv_from = sss_conv_from();
-    std::mt19937 gen(12345);                                             // sss_postcal.cpp:138
-    SssCur cur;
-    memset(&cur, 0, sizeof cur);                                         // causal_locs starts empty (:115)
-    double old_sum_lkl = 0, sss_sum_lkl = 0;
-    int iter = 0, why = 0;
-    std::vector<double> probs;
-    for (iter = 0; iter < max_iterations; iter++) {
-        long long nz, nm, np;
-        sss_nbd_sizes(U, cur.k, c, nz, nm, np);
-        const long long n = nz + nm + np;
-        if ((rc = sss_table_reserve(e, q.count + (u64)n))) return rc;
-        SssShard sh;
-        memset(&sh, 0, sizeof sh);
-        sh.world = world; sh.rank = rank;
-        if (world > 1) {                                                 // this round's exchange: epoch flag + the half of the slots it uses
-            const u64 epoch = ++*pp.sss_epoch;
-            sh.flag = (unsigned)(epoch & 0x7fffffffu) + 1u;
-            const size_t hoff = acc_len + (size_t)(epoch & 1) * half;
-            for (int p = 0; p < world; p++) {
-                if (p == rank) continue;
-                sh.peer_slot[p] = p2p_slots(pp.peer_base[p]) + (size_t)rank * stride + hoff;
-                sh.my_slot[p] = p2p_slots(pp.mailbox) + (size_t)p * stride + hoff;
-            }
+    SssShard sh;
+    memset(&sh, 0, sizeof sh);
+    sh.world = world; sh.rank = rank;
+    if (world > 1) {                                                     // this round's exchange: epoch flag + the half of the slots it uses
+        const size_t acc_len = p2p_acc_len(e), half = p2p_sss_half(e), stride = p2p_slot_len(e);
+        const u64 epoch = ++*pp.sss_epoch;
+        sh.flag = (unsigned)(epoch & 0x7fffffffu) + 1u;
+        const size_t hoff = acc_len + (size_t)(epoch & 1) * half;
+        for (int p = 0; p < world; p++) {
+            if (p == rank) continue;
+            sh.peer_slot[p] = p2p_slots(pp.peer_base[p]) + (size_t)rank * stride + hoff;
+            sh.my_slot[p] = p2p_slots(pp.mailbox) + (size_t)p * stride + hoff;
         }
-        CU(cudaMemsetAsync(q.d_counter, 0, 2 * sizeof(int), e->stream));
-        sss_lookup_kernel<<<(unsigned)((n + 1 + 255) / 256), 256, 0, e->stream>>>(q.tab, cur, U, c, n, kmax, world, rank, q.d_out_l,
-                                                                                 q.d_batch, q.d_upd, q.d_pos_of, q.d_state, q.d_counter);
-        e->launches++;
-        // one launch scores the current configuration + this rank's unseen neighbours (the batch length is read on the device)
-        if ((rc = launch_score_batch(e, q.d_batch, 1, (n + world - 1) / world + 1, kmax, q.d_upd, q.d_scored, q.d_counter))) return rc;
-        if (n > 0) {
-            if (world > 1) {
-                sss_push_kernel<<<(unsigned)((n + 255) / 256), 256, 0, e->stream>>>(sh, n, q.d_state, q.d_pos_of, q.d_scored);
-                e->launches++;
-            }
-            sss_insert_kernel<<<(unsigned)((n + 255) / 256), 256, 0, e->stream>>>(q.tab, cur, U, c, n, sh, q.d_state, q.d_pos_of,
-                                                                                 q.d_scored, q.d_out_l, errf);
-            e->launches++;
-        }
-        if (iter >= conv_from) {                                         // the running sum is only consulted from here on
-            // total = log(sum) + cx, as the finalize
-            sss_total_kernel<<<1, 32, 0, e->stream>>>(e->L.acc, sh, (long long)n_max, e->L.cx, q.d_total, errf);
-            e->launches++;
-        }
-        CU(cudaGetLastError());
-        int cnt[2] = {0, 0};
-        CU(cudaMemcpyAsync(cnt, q.d_counter, sizeof cnt, cudaMemcpyDeviceToHost, e->stream));
-        if (n > 0) CU(cudaMemcpyAsync(q.h_out_l, q.d_out_l, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
-        if (iter >= conv_from) CU(cudaMemcpyAsync(q.h_out_l + n_max + 1, q.d_total, sizeof(double), cudaMemcpyDeviceToHost, e->stream));
-        CU(cudaStreamSynchronize(e->stream));
-        const int n_new = cnt[1];                                        // unseen neighbours of all ranks
-        if (n_new == 0) { why = 1; break; }                              // "hit break condition", :260-263
-        // (the reference inserts the new values after this check and the next one; the table already holds them, which
-        //  is unobservable: both exits leave the loop)
-        q.count += (u64)n_new;
-        if (iter >= conv_from) sss_sum_lkl = q.h_out_l[n_max + 1];
-        if (iter >= conv_from + 1 && (1 - std::exp(old_sum_lkl - sss_sum_lkl)) <= 0.001) { why = 2; break; }   // :265-270
-
-        // sampling, sss_postcal.cpp:289-343: one draw inside each group, then one across the groups
-        const double* ll = q.h_out_l;
-        double weight[3] = {0.0, 0.0, 0.0};
-        long long sample[3] = {n, n, n};
-        const long long lo[3] = {0, nz, nz + nm}, hi[3] = {nz, nz + nm, n};
-        for (int g = 0; g < 3; g++) {
-            if (lo[g] == hi[g]) continue;
-            const double max_log = *std::max_element(ll + lo[g], ll + hi[g]);
-            probs.clear();
-            for (long long ii = lo[g]; ii < hi[g]; ii++) probs.push_back(std::exp(ll[ii] - max_log));
-            std::discrete_distribution<size_t> dist(probs.begin(), probs.end());
-            sample[g] = (long long)dist(gen);
-            weight[g] = std::accumulate(probs.begin(), probs.end(), 0.0);
-        }
-        std::discrete_distribution<size_t> dist({weight[0], weight[1], weight[2]});
-        const size_t grp = dist(gen);
-        SssCur nxt;
-        memset(&nxt, 0, sizeof nxt);
-        nxt.k = sss_neighbour(cur, U, c, sample[grp] + lo[grp], nxt.g);  // :354
-        cur = nxt;
-        old_sum_lkl = sss_sum_lkl;
     }
-    if (iterations) *iterations = iter;
-    if (stop_reason) *stop_reason = why;
+    CU(cudaMemsetAsync(q.d_counter, 0, 2 * sizeof(int), e->stream));
+    sss_lookup_kernel<<<(unsigned)((n + 1 + 255) / 256), 256, 0, e->stream>>>(q.tab, r->cur, U, c, n, kmax, world, rank, q.d_out_l,
+                                                                             q.d_batch, q.d_upd, q.d_pos_of, q.d_state, q.d_counter);
+    e->launches++;
+    // one launch scores the current configuration + this rank's unseen neighbours (the batch length is read on the device)
+    if ((rc = launch_score_batch(e, q.d_batch, 1, (n + world - 1) / world + 1, kmax, q.d_upd, q.d_scored, q.d_counter))) return rc;
+    if (n > 0) {
+        if (world > 1) {
+            sss_push_kernel<<<(unsigned)((n + 255) / 256), 256, 0, e->stream>>>(sh, n, q.d_state, q.d_pos_of, q.d_scored);
+            e->launches++;
+        }
+        sss_insert_kernel<<<(unsigned)((n + 255) / 256), 256, 0, e->stream>>>(q.tab, r->cur, U, c, n, sh, q.d_state, q.d_pos_of,
+                                                                             q.d_scored, q.d_out_l, errf);
+        e->launches++;
+    }
+    const bool conv = r->iter >= r->conv_from;                           // the running sum is only consulted from here on
+    if (conv) {
+        // total = log(sum) + cx, as the finalize
+        sss_total_kernel<<<1, 32, 0, e->stream>>>(e->L.acc, sh, n_max, e->L.cx, q.d_total, errf);
+        e->launches++;
+    }
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(sss_host_counters(e, r), q.d_counter, 2 * sizeof(int), cudaMemcpyDeviceToHost, e->stream));
+    if (n > 0) CU(cudaMemcpyAsync(q.h_out_l, q.d_out_l, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+    if (conv) CU(cudaMemcpyAsync(q.h_out_l + n_max + 1, q.d_total, sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaEventRecord(e->ev_up, e->stream));
+    return 0;
+}
+
+// Waits for the round sss_round_enqueue issued, applies the break and convergence rules and, when the search goes on, draws
+// the next state.  Clears r->more when the search has stopped.
+static int sss_round_complete(pipsort_engine* e, SssRun* r) {
+    pipsort_engine::Sss& q = e->sss;
+    CU(cudaEventSynchronize(e->ev_up));
+    const int n_new = sss_host_counters(e, r)[1];                        // unseen neighbours of all ranks
+    if (n_new == 0) { r->why = 1; r->more = false; return 0; }           // "hit break condition", :260-263
+    // (the reference inserts the new values after this check and the next one; the table already holds them, which
+    //  is unobservable: both exits leave the loop)
+    q.count += (u64)n_new;
+    const int iter = r->iter;
+    if (iter >= r->conv_from) r->sss_sum_lkl = q.h_out_l[r->n_max + 1];
+    if (iter >= r->conv_from + 1 && (1 - std::exp(r->old_sum_lkl - r->sss_sum_lkl)) <= 0.001) {   // :265-270
+        r->why = 2; r->more = false; return 0;
+    }
+
+    // sampling, sss_postcal.cpp:289-343: one draw inside each group, then one across the groups
+    const long long n = r->n, nz = r->nz, nm = r->nm;
+    const double* ll = q.h_out_l;
+    double weight[3] = {0.0, 0.0, 0.0};
+    long long sample[3] = {n, n, n};
+    const long long lo[3] = {0, nz, nz + nm}, hi[3] = {nz, nz + nm, n};
+    std::vector<double>& probs = r->probs;
+    for (int g = 0; g < 3; g++) {
+        if (lo[g] == hi[g]) continue;
+        const double max_log = *std::max_element(ll + lo[g], ll + hi[g]);
+        probs.clear();
+        for (long long ii = lo[g]; ii < hi[g]; ii++) probs.push_back(std::exp(ll[ii] - max_log));
+        std::discrete_distribution<size_t> dist(probs.begin(), probs.end());
+        sample[g] = (long long)dist(r->gen);
+        weight[g] = std::accumulate(probs.begin(), probs.end(), 0.0);
+    }
+    std::discrete_distribution<size_t> dist({weight[0], weight[1], weight[2]});
+    const size_t grp = dist(r->gen);
+    SssCur nxt;
+    memset(&nxt, 0, sizeof nxt);
+    nxt.k = sss_neighbour(r->cur, e->U, r->c, sample[grp] + lo[grp], nxt.g);   // :354
+    r->cur = nxt;
+    r->old_sum_lkl = r->sss_sum_lkl;
+    r->more = ++r->iter < r->max_iterations;
+    return 0;
+}
+
+static int sss_run(pipsort_engine* e, int c, int max_iterations, int32_t* iterations, int32_t* stop_reason, bool sharded) {
+    SssRun r;
+    int rc = sss_begin(e, c, max_iterations, sharded, &r);
+    while (!rc && r.more) {
+        rc = sss_round_enqueue(e, &r);
+        if (!rc) rc = sss_round_complete(e, &r);
+    }
+    if (rc) return rc;
+    if (iterations) *iterations = r.iter;
+    if (stop_reason) *stop_reason = r.why;
     return check_flags(e);
 }
 
@@ -1984,9 +2045,9 @@ static int batch_worker(const pipsort_locus* loci, int32_t n_loci, int first, in
     return rc;
 }
 
-// the host threads of a batch (PIPSORT_BATCH_THREADS), each running batch_worker over its share of the loci
-static int batch_run(const pipsort_locus* loci, int32_t n_loci, int device, uint32_t flags, int c, const GridRead& grid,
-                     const pipsort_outputs* outs, uint64_t* n_configs) {
+// the host threads of a batch (PIPSORT_BATCH_THREADS), each running worker(first, stride, &stop, &err) over its share of the
+// loci; the first error of any thread is the call's
+static int batch_threads(int32_t n_loci, const std::function<int(int, int, std::atomic<int>*, std::string*)>& worker) {
     // The host side of a small locus (a dozen runtime calls, ~60 us) costs as much as its evaluation on the device: long lists
     // are issued by several host threads (PIPSORT_BATCH_THREADS, default 3), each with its own pipeline over its own engines
     // and streams, loci dealt round robin.  The kernels of different loci then also overlap on the device -- a 150-SNP
@@ -1998,13 +2059,90 @@ static int batch_run(const pipsort_locus* loci, int32_t n_loci, int device, uint
     std::vector<std::string> errs(T);
     std::vector<int> rcs(T, 0);
     std::vector<std::thread> th;
-    for (int t = 1; t < T; t++)
-        th.emplace_back([&, t] { rcs[t] = batch_worker(loci, n_loci, t, T, device, flags, c, grid, outs, n_configs, &stop, &errs[t]); });
-    rcs[0] = batch_worker(loci, n_loci, 0, T, device, flags, c, grid, outs, n_configs, &stop, &errs[0]);
+    for (int t = 1; t < T; t++) th.emplace_back([&, t] { rcs[t] = worker(t, T, &stop, &errs[t]); });
+    rcs[0] = worker(0, T, &stop, &errs[0]);
     for (auto& x : th) x.join();
     for (int t = 0; t < T; t++)
         if (rcs[t]) { g_err = errs[t]; return rcs[t]; }
     return 0;
+}
+
+static int batch_run(const pipsort_locus* loci, int32_t n_loci, int device, uint32_t flags, int c, const GridRead& grid,
+                     const pipsort_outputs* outs, uint64_t* n_configs) {
+    return batch_threads(n_loci, [&](int first, int stride, std::atomic<int>* stop, std::string* err) {
+        return batch_worker(loci, n_loci, first, stride, device, flags, c, grid, outs, n_configs, stop, err);
+    });
+}
+
+// Searches in flight per host thread of pipsort_sss_batch (DESIGN.md section 5a has the measurement behind the default;
+// PIPSORT_SSS_DEPTH, read at every call, overrides it for such measurements).
+static int sss_depth() {
+    const char* v = getenv("PIPSORT_SSS_DEPTH");
+    return v ? std::max(1, std::min(16, atoi(v))) : 2;
+}
+
+// The shotgun searches of loci first, first + stride, ... with up to `depth` of them in flight, each on its own engine and
+// stream, advanced round robin: complete search A's round and draw A's next state, enqueue A's next round, move on to B.
+// One search's host work -- the wait, the draws over up to 30k exponentials -- then overlaps the other searches' kernels and
+// copies.  A search that stops has its read enqueued; at the slot's next visit the read completes, the engine is destroyed
+// and the slot takes this worker's next locus.  `stop` is raised by the first worker that fails; every engine still in
+// flight is then destroyed.
+static int sss_batch_worker(const pipsort_locus* loci, int32_t n_loci, int first, int stride, int device, uint32_t flags, int c,
+                            int max_iterations, int depth, const pipsort_outputs* outs, int32_t* iterations, int32_t* stop_reasons,
+                            uint64_t* n_configs, std::atomic<int>* stop, std::string* err) {
+    struct Slot { pipsort_engine* e = nullptr; int i = -1; bool reading = false; SssRun r; };
+    std::vector<Slot> slots(depth);
+    int next = first;
+    // the search's next round, or its read once it has stopped
+    auto enqueue = [](Slot& s) -> int {
+        if (s.r.more) return sss_round_enqueue(s.e, &s.r);
+        s.reading = true;
+        return read_enqueue(s.e);
+    };
+    auto start = [&](Slot& s) -> int {          // this worker's next locus into the empty slot s (none left: s stays empty)
+        if (next >= n_loci) return 0;
+        s.i = next;
+        next += stride;
+        s.r = SssRun();
+        s.reading = false;
+        int r = pipsort_create(&loci[s.i], device, flags | PIPSORT_INTERNAL_NO_UPLOAD_WAIT, &s.e);
+        if (!r && (r = sss_begin(s.e, c, max_iterations, false, &s.r))) {
+            const std::string why = g_err;
+            r = fail(r, "locus %d: %s", s.i, why.c_str());
+        }
+        return r ? r : enqueue(s);
+    };
+    auto advance = [&](Slot& s) -> int {
+        if (!s.reading) {
+            int r = sss_round_complete(s.e, &s.r);
+            return r ? r : enqueue(s);
+        }
+        int r = read_complete(s.e, &outs[s.i]);
+        if (!r) {
+            if (iterations) iterations[s.i] = s.r.iter;
+            if (stop_reasons) stop_reasons[s.i] = s.r.why;
+            if (n_configs) n_configs[s.i] = s.e->last_read_count;
+        }
+        pipsort_destroy(s.e);
+        s.e = nullptr;
+        return r ? r : start(s);
+    };
+    int rc = 0;
+    for (Slot& s : slots)
+        if (!rc) rc = start(s);
+    for (bool busy = true; busy && !rc;) {
+        busy = false;
+        for (Slot& s : slots) {
+            if (!s.e) continue;
+            if (stop->load(std::memory_order_relaxed)) break;
+            busy = true;
+            if ((rc = advance(s))) break;
+        }
+        if (stop->load(std::memory_order_relaxed)) break;
+    }
+    for (Slot& s : slots) pipsort_destroy(s.e);      // after an error or a stop raised by another worker
+    if (rc) { stop->store(1); *err = g_err; }
+    return rc;
 }
 
 int pipsort_posterior_exhaustive_batch(const pipsort_locus* loci, int32_t n_loci, int device, uint32_t flags, int c,
@@ -2039,6 +2177,27 @@ int pipsort_count_table_batch(const pipsort_locus* loci, int32_t n_loci, int dev
     if (c < 0 || c > KMAX) return fail(PIPSORT_E_ARG, "c=%d must be in [0, %d]", c, KMAX);
     if (!n_loci) return 0;
     return batch_run(loci, n_loci, device, flags, c, GridRead{0, nullptr, c, tables, true}, nullptr, n_configs);
+}
+
+int pipsort_sss_batch(const pipsort_locus* loci, int32_t n_loci, int device, uint32_t flags, int max_causal, int max_iterations,
+                      const pipsort_outputs* outs, int32_t* iterations, int32_t* stop_reasons, uint64_t* n_configs) {
+    if (n_loci < 0 || (n_loci > 0 && (!loci || !outs))) return fail(PIPSORT_E_ARG, "bad argument");
+    if (max_causal < 0 || max_causal > KMAX) return fail(PIPSORT_E_ARG, "max_causal=%d must be in [0, %d]", max_causal, KMAX);
+    if (max_iterations < 0) return fail(PIPSORT_E_ARG, "negative iteration count");
+    if (flags & (PIPSORT_PRIOR_CLASSES | PIPSORT_CAUSAL_COUNTS)) return fail(PIPSORT_E_ARG, "%s", CLASSES_NO_SSS);
+    for (int i = 0; i < n_loci; i++) {
+        const int rc = sss_locus_check(loci[i].union_count, loci[i].sharing_param, max_causal);
+        if (rc) {
+            const std::string why = g_err;
+            return fail(rc, "locus %d: %s", i, why.c_str());
+        }
+    }
+    if (!n_loci) return 0;
+    const int depth = sss_depth();
+    return batch_threads(n_loci, [&](int first, int stride, std::atomic<int>* stop, std::string* err) {
+        return sss_batch_worker(loci, n_loci, first, stride, device, flags, max_causal, max_iterations, depth, outs, iterations,
+                                stop_reasons, n_configs, stop, err);
+    });
 }
 
 // ---- the posterior of the causal counts (pipsort_count_posterior; host code, DESIGN.md section 5f) ------------------------------

@@ -99,6 +99,8 @@ def lib():
         L.pipsort_sss.argtypes = [vp, i32, i32, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
         L.pipsort_sss_reset.argtypes = [vp]
         L.pipsort_sss_sharded.argtypes = [vp, i32, i32, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
+        L.pipsort_sss_batch.argtypes = [C.POINTER(_LocusV), C.c_int32, i32, C.c_uint32, i32, i32, C.POINTER(_OutputsV),
+                                        C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(u64)]
         L.pipsort_read_accumulators.argtypes = [vp, C.POINTER(_Outputs)]
         L.pipsort_read_prior_grid.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(_OutputsV),
                                               C.POINTER(u64)]
@@ -583,16 +585,21 @@ class LocusBatch:
     class_evidence=True: run() is pipsort_class_evidence_batch, the buffer holds every locus's class table
     ((c+1)(c+2)/2 doubles, Engine.read_class_evidence's layout), read with tables().
     count_table=True: run() is pipsort_count_table_batch, the buffer holds every locus's count table (C(c+3, 3) doubles,
-    Engine.read_count_table's layout), read with tables()."""
+    Engine.read_count_table's layout), read with tables().
+    search=True: run() is pipsort_sss_batch, the shotgun search of every locus at max_causal c with at most max_iterations
+    rounds; results() as for the ordinary batch, and the arrays `iterations` and `stop_reasons` hold what Engine.sss returns
+    with them."""
 
     def __init__(self, loci, c, device=0, raw_ld=False, priors=None, evidence_only=False, class_evidence=False,
-                 count_table=False):
+                 count_table=False, search=False, max_iterations=1000):
         if evidence_only and priors is None:
             raise ValueError("evidence_only needs priors")
         if (class_evidence or count_table) and priors is not None:
             raise ValueError("class_evidence and count_table take no priors")
         if class_evidence and count_table:
             raise ValueError("one table read per batch: class_evidence or count_table")
+        if search and (priors is not None or class_evidence or count_table):
+            raise ValueError("a search batch takes no priors and reads no tables")
         n = self.n = len(loci)
         self.c, self.device, self.flags = int(c), int(device), RAW_LD if raw_ld else 0
         f64, i32 = np.dtype(np.float64), np.dtype(np.int32)
@@ -618,6 +625,7 @@ class LocusBatch:
         self.evidence_only = bool(evidence_only)
         self.class_evidence = bool(class_evidence)
         self.count_table = bool(count_table)
+        self.search = bool(search)
         self.ntab = _ncnt(self.c) if count_table else _ntab(self.c)
         k = self.k = 1 if priors is None else len(self.priors[0])      # result blocks per locus: locus i, prior j -> i * k + j
         if class_evidence or count_table:
@@ -646,7 +654,13 @@ class LocusBatch:
         self.cnt = np.zeros(n, dtype=np.uint64)
         lp, op = C.cast(la.ctypes.data, C.POINTER(_LocusV)), C.cast(oa.ctypes.data, C.POINTER(_OutputsV))
         cp = C.cast(self.cnt.ctypes.data, C.POINTER(C.c_uint64))
-        if class_evidence or count_table:
+        if search:
+            self.iterations = np.zeros(n, dtype=np.int32)
+            self.stop_reasons = np.zeros(n, dtype=np.int32)
+            i32p = C.POINTER(C.c_int32)
+            self._args = (lp, n, self.device, self.flags, self.c, int(max_iterations), op,
+                          C.cast(self.iterations.ctypes.data, i32p), C.cast(self.stop_reasons.ctypes.data, i32p), cp)
+        elif class_evidence or count_table:
             self._args = (lp, n, self.device, self.flags, self.c, _dp(buf), cp)
         elif priors is None:
             self._args = (lp, n, self.device, self.flags, self.c, op, cp)
@@ -657,7 +671,9 @@ class LocusBatch:
     def run(self):
         """pipsort_posterior_exhaustive_batch (pipsort_posterior_exhaustive_grid_batch with priors): host buffers in, host
         buffers out."""
-        if self.class_evidence:
+        if self.search:                     # the arguments are checked even for an empty list
+            _check(lib().pipsort_sss_batch(*self._args))
+        elif self.class_evidence:
             _check(lib().pipsort_class_evidence_batch(*self._args))
         elif self.count_table:
             _check(lib().pipsort_count_table_batch(*self._args))
@@ -728,6 +744,15 @@ def count_table_batch(loci, c, device=0, raw_ld=False):
     pipelined as posterior_exhaustive_batch.  loci as posterior_exhaustive_batch takes them; returns ndarray
     [n_loci, C(c+3, 3)] (Engine.read_count_table's layout)."""
     return LocusBatch(loci, c, device, raw_ld, count_table=True).run().tables()
+
+
+def sss_batch(loci, c, max_iterations=1000, device=0, raw_ld=False):
+    """The shotgun search of every locus (pipsort_sss_batch): what Engine.sss(c, max_iterations) returns on a fresh engine
+    per locus, with several searches in flight per host thread.  loci as posterior_exhaustive_batch takes them.  Returns
+    (a list of Results, iterations, stop_reasons), the last two int32 ndarrays with one entry per locus (stop reason 0 =
+    iteration cap, 1 = no new configuration, 2 = convergence)."""
+    B = LocusBatch(loci, c, device, raw_ld, search=True, max_iterations=max_iterations).run()
+    return B.results(), B.iterations.copy(), B.stop_reasons.copy()
 
 
 def _count_c(w):
